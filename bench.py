@@ -15,15 +15,22 @@ basis, 4 option slots, 2 preset active logistic initiation classifiers (the cont
 warm-up) - weak scaling: each rank owns its own 65,536-env slice.  Synthetic data: random free-space start
 states, random-init weights.
 
-Prints ONE JSON line (rank 0).  The timed region is R consecutive blocks of exactly K steps (CUDA events at the
-block boundaries, max over ranks per block); `value` = env-steps of one block over all ranks / the median block
-time, state resident in HBM; `e2e` = the same blocks through SkillChainAgent.step_host (host buffers, H2D and D2H
-inside the timed region) with a per-step breakdown; `roofline` = the window trace-sweep kernel's algorithmic bytes /
-its CUDA-event time against the measured HBM copy peak; `cpu_baseline` = the NumPy oracle timed on this box;
+Prints ONE JSON line (rank 0).  The timed region is exactly K = --steps agent steps, cut into blocks of one sync
+interval each (CUDA events at the block boundaries, max over ranks per block); `value` = env-steps of the full blocks
+over all ranks / their summed time, state resident in HBM; `e2e` = K steps through SkillChainAgent.step_host
+(host buffers, H2D and D2H inside the timed region) in the same blocks, with a per-step breakdown; `roofline` = the
+window trace-sweep kernel's algorithmic bytes / its CUDA-event time against the measured HBM copy peak;
+`cpu_baseline` = the NumPy oracle timed on this box;
 `north_star_config` = the configs[2] per-GPU shape (hard map, order 5, 8 options, 131,072 envs) measured in the same
 process; `sync` (N > 1) = microseconds per weight exchange, peer-memory kernel vs NCCL.
 --impl reference times the stand-in reference (the NumPy oracle: the reference repository has no
 code) on all host cores for the same metric.
+
+--dump-outputs DIR writes what the timed path left after its last step (rank 0's envs) as DIR/<name>.npy, so that two
+builds can be compared output for output: the same arguments give the same inputs on every run.  The weight-delta sum
+uses floating-point atomics, so weights differ between runs in the last bits and an env whose arg-max is a near-tie can
+take another action.  Over a short run this touches a few envs (2 of 65,536 at --steps 20 --warmup 3 on a B200); over
+thousands of steps learning amplifies it and most env states differ, so compare builds on short runs.
 """
 import argparse
 import json
@@ -253,15 +260,20 @@ def make_agent(scg, torch, args, rank, world):
     return ag
 
 
-def timed_blocks(torch, ag, steps, n_blocks, barrier, t_done):
-    """`n_blocks` consecutive blocks of exactly `steps` agent steps each, device-resident, CUDA events at the block
-    boundaries (windows, syncs and the controller's cadence run on across blocks: a block is a slice of the steady
-    state, whatever `steps` is).  Returns per-block milliseconds and the global step counter."""
-    ev = [torch.cuda.Event(enable_timing=True) for _ in range(n_blocks + 1)]
-    barrier()
+def block_sizes(steps, per_block):
+    """`steps` steps as consecutive blocks of `per_block` steps; the last block holds the remainder."""
+    return [per_block] * (steps // per_block) + ([steps % per_block] if steps % per_block else [])
+
+
+def timed_blocks(torch, ag, sizes, barrier):
+    """Exactly sum(sizes) agent steps, device-resident, as consecutive blocks of the given sizes with CUDA events at the
+    block boundaries (windows, syncs and the controller's 64-step cadence run on across blocks), queued behind the work
+    already on the stream.  Returns per-block milliseconds."""
+    ev = [torch.cuda.Event(enable_timing=True) for _ in range(len(sizes) + 1)]
     ev[0].record()
-    for i in range(n_blocks):
-        left = steps
+    t_done = 0
+    for i, n in enumerate(sizes):
+        left = n
         while left > 0:                                         # full skill chaining: steps + the controller
             k = min(left, MANAGE_EVERY - t_done % MANAGE_EVERY)
             ag.run(k)
@@ -269,11 +281,41 @@ def timed_blocks(torch, ag, steps, n_blocks, barrier, t_done):
             left -= k
             if t_done % MANAGE_EVERY == 0:
                 ag.manage()
-        if i == n_blocks - 1:
+        if i == len(sizes) - 1:
             ag.flush()                                          # a partial last window is swept inside the timed region
         ev[i + 1].record()
     barrier()
-    return [ev[i].elapsed_time(ev[i + 1]) for i in range(n_blocks)], t_done
+    return [ev[i].elapsed_time(ev[i + 1]) for i in range(len(sizes))]
+
+
+def ms_per_step(blocks, sizes, per_block):
+    """Time per step of the full blocks, or of all blocks if none is full (a last, partial block carries the sweep of
+    a whole window for fewer steps)."""
+    full = [b for b, n in zip(blocks, sizes) if n == per_block]
+    return sum(full) / (len(full) * per_block) if full else sum(blocks) / sum(sizes)
+
+
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def last_step_outputs(ag, max_bytes=DUMP_MAX_BYTES):
+    """What a caller of SkillChainAgent.run holds after its last step, as float32 / float64 arrays: per env the state,
+    reward, termination flags (bit fields, exact in float64), next action, option and TD error, and the option weights.
+    If the per-env arrays would pass `max_bytes`, a fixed seeded sample of the envs is kept and `env_index` names them."""
+    per_env = dict(state=ag.state.cpu().numpy(), reward=ag.reward.cpu().numpy(),
+                   flags=ag.flags.cpu().numpy().view(np.uint32).astype(np.float64),
+                   action=ag.action.cpu().numpy().astype(np.float32), option=ag.option.cpu().numpy().astype(np.float32),
+                   td_error=ag.delta.cpu().numpy())
+    out = dict(weights=ag.options.W.cpu().numpy())
+    B = len(per_env["reward"])
+    bytes_per_env = sum(a.nbytes for a in per_env.values()) // max(B, 1) + 8      # + 8: its env_index entry
+    n = min(B, (max_bytes - out["weights"].nbytes) // bytes_per_env)
+    if n < B:
+        idx = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        out["env_index"] = idx.astype(np.float64)
+        per_env = {k: v[idx] for k, v in per_env.items()}
+    out.update(per_env)
+    return out
 
 
 def stage_pass(torch, ag, T, n_windows=8):
@@ -324,53 +366,68 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return [float(v) for v in t]
 
-    def measure(a, steps, n_blocks, n_warm, live_kind=True):
-        """Warm up, then time n_blocks blocks of `steps` steps -> dict of per-rank-max block times and kernel timings."""
+    def measure(a, steps, n_warm, live_kind=True, dump=False):
+        """Warm up, then time exactly `steps` steps in blocks of one sync interval -> dict of per-rank-max block times
+        and kernel timings (and, with dump=True, the outputs of the last timed step)."""
         ag = make_agent(scg, torch, a, rank, world)
         backend = a.sync_backend
         if world > 1 and a.sync_backend == "p2p" and ag._xchg is None:
             backend = "nccl"                                   # the agent fell back (it said why on stderr): report what ran
         B, T = a.batch, ag.win_cap
         ag.warm_up_controller()
-        t_done = 0
+        if live_kind:                                           # create the profiling events before the queue is filled
+            ag.profile_begin(steps + 64, kinds=(1,))
+            ag.profile_end()
         for lo in range(0, n_warm, MANAGE_EVERY):
-            k = min(MANAGE_EVERY, n_warm - lo)
-            ag.run(k)
-            t_done += k
-        t_done = 0                                              # the controller's cadence counts from the timed region
+            ag.run(min(MANAGE_EVERY, n_warm - lo))
         ag.manage()                                             # the preset gestating option qualifies within the warm-up
         barrier()
+        # the controller period after that promotion runs ~5 % slower than the steady state, so it ends the warm-up; it is
+        # queued after the barrier so that the GPU is still busy with it when the timed region starts (the first block
+        # then carries no launch latency)
+        ag.run(MANAGE_EVERY)
+        ag.manage()
         launches0 = lib.scg_launch_count()
         if live_kind:
-            ag.profile_begin(n_blocks * steps + 64, kinds=(1,))    # events around the dominant kernel only, live
-        blocks, t_done = timed_blocks(torch, ag, steps, n_blocks, barrier, t_done)
+            ag.profile_begin(steps + 64, kinds=(1,))               # events around the dominant kernel only, live
+        sizes = block_sizes(steps, a.sync_interval)
+        t0 = ag.t
+        blocks = timed_blocks(torch, ag, sizes, barrier)
+        steps_run = ag.t - t0                                   # the library's own step counter
         live_ms, live_n = ag.profile_end() if live_kind else ([0.0] * 6, [0] * 6)
         launches = lib.scg_launch_count() - launches0
+        outputs = last_step_outputs(ag) if dump else None
         blocks = reduce_max(blocks)                             # per block: the slowest rank
         side_ms, side_n, n_side = stage_pass(torch, ag, T)
         if ag.peer_sync_timed_out():
             raise scg.ScgError("a cross-GPU weight exchange timed out during the bench: no valid number")
-        med = float(np.median(blocks))
+        per_step = ms_per_step(blocks, sizes, a.sync_interval)
         k3_ms = live_ms[1] / live_n[1] if live_n[1] else side_ms[1]
-        return dict(ag=ag, backend=backend, blocks=blocks, ms_block=med, ms_per_step=med / steps, k3_ms=k3_ms,
+        return dict(ag=ag, backend=backend, blocks=blocks, sizes=sizes, steps_run=steps_run, ms_per_step=per_step, k3_ms=k3_ms,
                     k3_launches=live_n[1], side_ms=side_ms, side_n=side_n, n_side=n_side, launches=launches,
-                    ctl=ag.controller_state(sync=True))
+                    ctl=ag.controller_state(sync=True), outputs=outputs)
 
     n_warm = max(args.warmup, 16)          # at least two windows, so the preset gestating option has qualified by the end
-    n_blocks = args.blocks or max(5, -(-1024 // max(args.steps, 1)))
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    m = measure(args, args.steps, n_blocks, n_warm)
+    m = measure(args, args.steps, n_warm, dump=bool(args.dump_outputs))
     ag, B, T = m["ag"], args.batch, m["ag"].win_cap
     args.sync_backend = m["backend"]
-    # ---- e2e: the same K-step blocks through the host-buffer API ----
-    def e2e_blocks(step_fn, n_b):
+    dumped = None
+    if m["outputs"] is not None and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in m["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
+        dumped = {"dir": args.dump_outputs, "bytes": sum(arr.nbytes for arr in m["outputs"].values()),
+                  "envs": len(m["outputs"]["reward"]), "arrays": sorted(m["outputs"])}
+    # ---- e2e: K steps through the host-buffer API, in the same blocks ----
+    def e2e_blocks(step_fns):
         out = []
-        for _ in range(n_b):
+        for fn in step_fns:
             barrier()
             t0 = time.perf_counter()
-            step_fn()
+            fn()
             torch.cuda.synchronize()
             out.append((time.perf_counter() - t0) * 1e3)
         return reduce_max(out)
@@ -379,8 +436,8 @@ def run_ours(args):
     ha = ag.action.cpu().numpy().copy()
     host = dict(s=hs, a=ha, i=0)
 
-    def host_steps():
-        for _ in range(args.steps):
+    def host_steps(n):
+        for _ in range(n):
             s2, r, f, a2, d = ag.step_host(host["s"], host["a"])
             host["s"], host["a"] = s2, a2                       # views of the pinned result buffers, fed straight back
             host["i"] += 1
@@ -389,9 +446,8 @@ def run_ours(args):
 
     for _ in range(3):
         host["s"], r, f, host["a"], d = ag.step_host(host["s"], host["a"])
-    n_e2e = max(3, min(n_blocks, -(-256 // max(args.steps, 1))))
-    e2e = e2e_blocks(host_steps, n_e2e)
-    e2e_ms = float(np.median(e2e))
+    e2e = e2e_blocks([lambda n=n: host_steps(n) for n in m["sizes"]])
+    e2e_ms = ms_per_step(e2e, m["sizes"], args.sync_interval) * args.steps
 
     # where an end-to-end step goes: the pieces timed one by one with CUDA events (pinned host buffers, this stream)
     def ev_time(fn, reps=20):
@@ -439,12 +495,11 @@ def run_ours(args):
     hw = dict(s=ag.s.cpu().numpy().copy(), a=ag.action.cpu().numpy().copy())
     n_calls = max(args.steps // Ts, 1)
 
-    def host_windows():
-        for _ in range(n_calls):
-            hw["s"], hw["a"], r, f, d = ag.run_host(hw["s"], hw["a"], Ts)
+    def host_window():
+        hw["s"], hw["a"], r, f, d = ag.run_host(hw["s"], hw["a"], Ts)
 
-    host_windows()
-    e2e_win_ms = float(np.median(e2e_blocks(host_windows, 3)))
+    host_window()
+    e2e_win_ms = float(np.median(e2e_blocks([host_window] * n_calls)))
     clocks = sampler.stop() if rank == 0 else None
     # ---- cross-GPU sync: the peer-memory kernel against two NCCL all-reduces + apply on the same payload ----
     sync_cmp = None
@@ -472,11 +527,12 @@ def run_ours(args):
         torch.cuda.empty_cache()
         na = argparse.Namespace(**vars(args))
         na.map, na.order, na.options, na.batch, na.window = "hard", 5, 8, 131072, 0
-        nm = measure(na, 64, 5, 16)
+        nm = measure(na, 320, 16)
         F5 = 6 ** 4
         nb = 8 * 5 * F5 + 32 * nm["ag"].win_cap
-        north = {"workload": config_json(na, world)["workload"], "value": na.batch * world * 64 / (nm["ms_block"] * 1e-3),
-                 "unit": UNIT, "ms_per_step": nm["ms_per_step"], "steps_per_block": 64, "blocks_ms": nm["blocks"],
+        north = {"workload": config_json(na, world)["workload"], "value": na.batch * world / (nm["ms_per_step"] * 1e-3),
+                 "unit": UNIT, "ms_per_step": nm["ms_per_step"], "steps": 320, "steps_per_block": na.sync_interval,
+                 "blocks_ms": nm["blocks"],
                  "n_active_end": nm["ctl"]["n_active"],
                  "k_window": {"avg_launch_ms": nm["k3_ms"], "achieved_gbs": na.batch * nb / (nm["k3_ms"] * 1e-3) / 1e9 if nm["k3_ms"] else None,
                               "algorithmic_bytes_per_launch": na.batch * nb},
@@ -487,7 +543,7 @@ def run_ours(args):
     if rank == 0:
         F = (args.order + 1) ** 4
         total_env_steps = B * world * args.steps
-        value = total_env_steps / (m["ms_block"] * 1e-3)
+        value = B * world / (m["ms_per_step"] * 1e-3)
         peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
         if os.path.exists(peaks_path):
             peak, which = float(json.load(open(peaks_path))["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
@@ -507,12 +563,15 @@ def run_ours(args):
             "warmup": args.warmup, "ms_per_step": m["ms_per_step"], "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": config_json(args, world),
-            "timed_region": {"blocks": len(m["blocks"]), "steps_per_block": args.steps, "block_ms_median": m["ms_block"],
+            "timed_region": {"steps": args.steps, "steps_run": m["steps_run"], "total_ms": sum(m["blocks"]),
+                             "blocks": len(m["blocks"]), "steps_per_block": args.sync_interval,
                              "block_ms_min": min(m["blocks"]), "block_ms_max": max(m["blocks"]), "blocks_ms": m["blocks"],
-                             "warmup_steps_run": n_warm,
-                             "note": "value = steps of one block / median block time; blocks are consecutive slices of the "
-                                     "steady state (windows, syncs and the controller cadence run on across them), each "
-                                     "bracketed by CUDA events, max over ranks per block"},
+                             "warmup_steps_run": n_warm + MANAGE_EVERY,
+                             "note": "exactly `steps` steps, in blocks of one sync interval (its fused steps, trace sweeps "
+                                     "and weight apply; the last block takes the remainder and the sweep of a partial "
+                                     "window), each bracketed by CUDA events, max over ranks per block; value = steps of "
+                                     "the full blocks / their summed time (of all blocks if none is full); the controller "
+                                     "runs every 64 steps inside the timed region"},
             "roofline": {"kernel": "k_window (K3 Sarsa(lambda) trace sweep, forward-view window form)", "bound": "hbm",
                          "achieved": achieved, "peak": peak, "unit": "GB/s", "frac": achieved / peak,
                          "traffic": k3_traffic(args.order, B, T),
@@ -537,12 +596,12 @@ def run_ours(args):
                     "d2h_bytes_per_step": B * scg.SkillChainAgent.HOST_D2H_BYTES_PER_ENV,
                     "blocks_ms": e2e, "breakdown_per_step": brk,
                     "api": "SkillChainAgent.step_host -> scg_agent_step_host (pinned host buffers)"},
-            "e2e_per_sync_interval": {"value": B * world * n_calls * Ts / (e2e_win_ms * 1e-3), "unit": UNIT,
+            "e2e_per_sync_interval": {"value": B * world * Ts / (e2e_win_ms * 1e-3), "unit": UNIT, "calls": n_calls,
                                       "h2d_bytes_per_call": B * 20, "d2h_bytes_per_call": B * 32, "steps_per_call": Ts,
                                       "api": "SkillChainAgent.run_host: host state in / out once per sync interval "
                                              "(informational; `e2e` above copies every step)"},
             "controller_state_end": m["ctl"], "sync": sync_cmp, "north_star_config": north,
-            "gpu_launches": int(m["launches"]), "clocks": clocks,
+            "gpu_launches": int(m["launches"]), "clocks": clocks, "dump_outputs": dumped,
         }
         if world == 1 and not args.no_cpu:
             cores = max(1, len(os.sched_getaffinity(0)))
@@ -560,7 +619,7 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000, help="timed agent steps")
     ap.add_argument("--warmup", type=int, default=16)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--map", default="easy")
@@ -573,12 +632,17 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--sync-backend", default="p2p", choices=["p2p", "nccl"])
     ap.add_argument("--window", type=int, default=0, help="steps per trace sweep (0 = min(sync interval, 8))")
-    ap.add_argument("--blocks", type=int, default=0, help="timed blocks of --steps steps (0 = enough for ~1024 steps, at least 5)")
     ap.add_argument("--pin-cores", type=int, default=0, help="N > 1: pin each rank to its own slice of the host cores")
     ap.add_argument("--no-north-star", action="store_true", help="skip the extra configs[2]-shape measurement")
     ap.add_argument("--graph", action="store_true", help="option-graph variant (configs[4]): an option's targets are the "
                     "initiation sets of ALL earlier options and the goal, so chains merge")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0's envs) to DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1 or args.sync_interval < 1:
+        ap.error("--steps and --sync-interval must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
