@@ -282,8 +282,8 @@ int scg_xchg_sync_top(scg_xchg_t *x, int order, int K, int K_opt, float *W, floa
  * host (NumPy) arrays, as with the oracle's SkillChainAgent.  Copies state [4][B] and action [B]
  * host->device, runs the fused step, copies next state, reward, flags, next action and TD error
  * device->host and waits for them.  Traces and weights stay resident on the device.  When the SoA blocks are
- * back to back on both sides the step is pipelined over parts of the batch (copy in / step / copy out on three
- * streams; environment SCG_HOST_PARTS, default 2, 1 = one part); results are identical. */
+ * back to back on both sides and B >= 128 the step is pipelined over two halves of the batch (copy in / step / copy out
+ * on three streams); results are identical. */
 int scg_agent_step_host(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag,
                         const float *h_state_soa, const int *h_action, float *h_state2_soa,
                         float *h_reward, int *h_flags, int *h_action2, float *h_delta, void *stream);
@@ -298,7 +298,8 @@ int scg_agent_run_host(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, co
 /* Per-kernel device timing of the agent pipeline with CUDA events on the launch stream.
  * scg_profile_begin arms it (up to max_events kernel launches of the kinds in kind_mask are recorded);
  * scg_profile_end waits for the recorded events and returns, per kind, the summed milliseconds and the
- * launch count: kind 0 fused step kernel, 1 window trace sweep, 2 dW reduction, 3 weight apply / exchange.
+ * launch count: kind 0 fused step kernel, 1 window trace sweep, 2 dW reduction, 3 weight apply / exchange
+ * (scg_sarsa_update on the same context runs the same sweep and reduction, and is recorded as kinds 1 and 2).
  * (Events around the step kernels - bit 0 - keep consecutive step kernels from overlapping their prologues.) */
 #define SCG_PROF_KINDS 6   /* 0 fused step, 1 window sweep, 2 dW reduction, 3 apply / exchange, 4 example-ring pass, 5 controller */
 int scg_profile_begin(scg_ctx_t *ctx, int max_events, int kind_mask);

@@ -485,10 +485,8 @@ static int agent_steps(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, in
     args.b_begin = b_begin;
     args.b_end = b_end;
     // weights go to shared memory when two CTAs per SM still fit next to the map, or one big CTA
-    static int big = -1;
-    if (big < 0) { const char *e = getenv("SCG_STEP_BIG_CTA"); big = e ? atoi(e) : 1; }
     const size_t need = (size_t)args.w_bytes + args.blob_bytes + 256;
-    const int mode = need <= 100 * 1024 ? 1 : ((big && need <= 220 * 1024) ? 2 : 0);
+    const int mode = need <= 100 * 1024 ? 1 : (need <= 220 * 1024 ? 2 : 0);
     const bool pair = !ag->carry_valid;
     // a step kernel directly behind another step kernel of the same window may stage the weights early
     args.wait_first = !(ag->carry_valid && ag->win_len > 0 && !(ctx->prof_on && (ctx->prof_mask & 1)));
@@ -522,13 +520,10 @@ extern "C" int scg_agent_run(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *
     int rc = check_agent(map, ctx, ag);
     if (rc) return rc;
     if (ag->B == 0) return 0;
-    static int fuse = -1;   // SCG_STEPS_PER_LAUNCH=1 falls back to one launch per step (tuning / debugging)
-    if (fuse < 0) { const char *e = getenv("SCG_STEPS_PER_LAUNCH"); fuse = e ? atoi(e) : SCG_WIN_MAX; if (fuse < 1) fuse = 1; }
     for (int done = 0; done < n_steps;) {
         // as many steps as fit before the window is full, the sync is due, or the request ends
         int n = std::min(n_steps - done, ag->win_cap - ag->win_len);
         if (sync_interval > 0) n = std::min(n, std::max(1, sync_interval - ag->window_steps));
-        n = std::min(n, fuse);
         if ((rc = agent_steps(map, ctx, ag, n, stream))) return rc;
         done += n;
         if (sync_interval > 0 && ag->window_steps >= sync_interval) {
@@ -563,7 +558,8 @@ static int copy_rows(void *const *dst, const void *const *src, int rows, size_t 
 // for any one env but not across envs, so the batch is cut into parts (multiples of 32 envs) and pipelined: part p+1
 // is copied in while part p is stepped and part p-1 is copied out (PCIe is full duplex; copies in and copies out have
 // a stream each, the kernels stay on the caller's stream, events order the three).  Rows of the SoA blocks are moved
-// with one pitched copy per block.  SCG_HOST_PARTS (default 2; 1 = the plain sequence).
+// with one pitched copy per block.  Two parts measured fastest (DESIGN.md section 6); small batches, buffers that are not
+// back to back and profiled step kernels take the plain sequence.
 extern "C" int scg_agent_step_host(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, const float *h_state_soa,
                                    const int *h_action, float *h_state2_soa, float *h_reward, int *h_flags,
                                    int *h_action2, float *h_delta, void *stream) {
@@ -575,15 +571,13 @@ extern "C" int scg_agent_step_host(const scg_map_t *map, scg_ctx_t *ctx, scg_age
     const size_t n = (size_t)B * sizeof(float);
     int rc;
     if ((rc = check_agent(map, ctx, ag))) return rc;
-    static int parts_env = -1;
-    if (parts_env < 0) { const char *e = getenv("SCG_HOST_PARTS"); parts_env = e ? atoi(e) : 2; }
     // pitched copies need the SoA blocks back to back on both sides (they are in the Python layer: [4][B] tensors)
     auto rows4 = [&](const void *a, const void *b, const void *c, const void *d) {
         return (const char *)b == (const char *)a + n && (const char *)c == (const char *)a + 2 * n && (const char *)d == (const char *)a + 3 * n;
     };
     const bool blocks = rows4(ag->x, ag->y, ag->vx, ag->vy) && rows4(ag->x2, ag->y2, ag->vx2, ag->vy2) &&
                         rows4(ag->reward, ag->flags, ag->action, ag->delta) && rows4(h_reward, h_flags, h_action2, h_delta);
-    int parts = std::max(1, std::min(parts_env, SCG_HOST_PARTS_MAX));
+    int parts = SCG_HOST_PARTS_MAX;
     if (!blocks || B < 64 * parts || (ctx->prof_on && (ctx->prof_mask & 1))) parts = 1;
     if (parts == 1) {
         {

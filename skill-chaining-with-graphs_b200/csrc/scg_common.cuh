@@ -6,14 +6,10 @@
 #include "../../include/scg_b200.h"
 
 #define SCG_A SCG_N_ACTIONS
-#define SCG_REC_FLOATS 12
 #define SCG_WREC_FLOATS 8
 #define SCG_NUM_SMS 148
 
-// dense-sweep update record (scg_sarsa_update), 48 bytes per env:
-//   [0..7]  cos/sin(pi * s_hat_j), j = 0..3 of the state the update is for
-//   [8]     delta        [9] meta bits        [10],[11] unused
-// window step record (agent pipeline), 32 bytes per env-step:
+// window step record (agent pipeline and scg_sarsa_update), 32 bytes per env-step:
 //   [0..3]  x, y, vx, vy of the state the update is for     [4] delta     [5] meta bits     [6],[7] unused
 // meta bits: action (bits 0-2), option (bits 8-15), ZERO_AFTER (trace reset after the update), ACTIVE
 #define SCG_META_ACTIVE (1u << 31)
@@ -102,17 +98,16 @@ struct scg_map {
     size_t stage_cap;
 };
 
-#define SCG_HOST_PARTS_MAX 4
+#define SCG_HOST_PARTS_MAX 2
 struct scg_ctx {
     int order, K, F;
-    int n_partials;      // CTAs of the trace kernel
+    int n_partials;      // CTAs of the window sweep
     float *d_partial;    // [n_partials][K][A*F]
     float *d_red;        // [SCG_RED_SLICES][K][A*F] second-stage scratch of the slab reduction
     unsigned int *d_tickets;   // one "blocks done" counter per 256-element column of the reduction
     int deterministic;         // 1: fixed-order slab reduction (scg_ctx_set_deterministic)
     float *d_rec;        // records for the standalone scg_sarsa_update, grown on demand
     int rec_capacity;
-    int win_grid;        // CTAs of the window kernel (0 = not configured yet)
     cudaEvent_t host_ev; // "results copied" marker of scg_agent_step_host
     // scg_agent_step_host pipelines a step over parts of the batch: copies in on host_st[0], copies out on host_st[1]
     cudaStream_t host_st[2];

@@ -1,19 +1,13 @@
-// scg_sarsa.cu - K3, the Sarsa(lambda) eligibility-trace sweep and weight-delta accumulation (sm_100a).
+// scg_sarsa.cu - K3, the Sarsa(lambda) eligibility traces and weight deltas (sm_100a).
 //
-// Mirrors oracle/option.py OptionSet.update (trace part) and OptionSet.apply; the reference has
-// no code (/root/reference/README.md:1-2).  Per env b executing option o with action a:
+// Mirrors oracle/option.py OptionSet.flush, OptionSet.update (trace part) and OptionSet.apply.  Three kernels:
+//   k_window  the forward-view sweep over a window of T recorded steps: every env's dense trace (A*F fp32, HBM-bound) is
+//             read and written once per window, and each CTA accumulates its envs' dW contribution in shared memory
+//   k_reduce  folds the per-CTA dW slabs into dW
+//   k_apply   W += scaled dW, refreshes the packed copy Wt, zeroes dW and cnt
+// The agent pipeline sweeps the windows its step kernel recorded.  The dense per-step operator scg_sarsa_update is the
+// same sweep over a window of one step (k_make_rec writes that step's records): with T = 1 the forward view is
 //     e_b <- gamma*lambda e_b ;  e_b[a] += phi(s_b) ;  dW[o] += delta_b e_b ;  e_b <- 0 if done_b
-//
-// This is the HBM-bound kernel of the pipeline: the dense trace is A*F fp32 per env, read and
-// written once per env-step => 8*A*F (+48 record) algorithmic bytes per env-step.
-//
-// Design: one CTA sweeps one env at a time; thread t owns the same 16-byte chunk(s) of every env's
-// trace, i.e. a fixed set of (action, feature) entries.  Because ownership is exclusive, the CTA's
-// dW accumulator (shared memory, [K][A*F]) is updated with plain read-modify-write - no atomics, no
-// barriers inside the env loop.  phi(s_b) is rebuilt in registers from the four phasors the
-// record carries (only by the threads that own row a), so the only HBM traffic is the trace itself
-// plus a 48-byte record per env.  Two envs are in flight per CTA for memory-level parallelism.
-// At the end each CTA writes its accumulator to a scratch slab; k_reduce folds the slabs into dW.
 #include <stdlib.h>
 
 #include <algorithm>
@@ -33,134 +27,6 @@ __device__ __forceinline__ float4 vfma(float s, float4 a, float4 c) {
 }
 __device__ __forceinline__ float vfma(float s, float a, float c) { return fmaf(s, a, c); }
 __device__ __forceinline__ float4 vzero4() { return make_float4(0.f, 0.f, 0.f, 0.f); }
-
-// z^c for 0 <= c < 8 from (z, z^2, z^4) with selects (no dynamic register indexing)
-__device__ __forceinline__ float2 cpow_sel(float2 z1, float2 z2, float2 z4, int c) {
-    float2 r = (c & 1) ? z1 : make_float2(1.f, 0.f);
-    if (c & 2) r = scg_cmul(r, z2);
-    if (c & 4) r = scg_cmul(r, z4);
-    return r;
-}
-
-struct Phasors {
-    float2 z1[4], z2[4], z4[4];
-};
-__device__ __forceinline__ Phasors make_phasors(float4 r0, float4 r1) {
-    Phasors p;
-    p.z1[0] = make_float2(r0.x, r0.y); p.z1[1] = make_float2(r0.z, r0.w);
-    p.z1[2] = make_float2(r1.x, r1.y); p.z1[3] = make_float2(r1.z, r1.w);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        p.z2[j] = scg_cmul(p.z1[j], p.z1[j]);
-        p.z4[j] = scg_cmul(p.z2[j], p.z2[j]);
-    }
-    return p;
-}
-// phi for the feature whose base-N1 digits are packed 4 bits each (c0 lowest nibble)
-__device__ __forceinline__ float phi_digits(const Phasors &p, uint32_t d) {
-    float2 a = cpow_sel(p.z1[0], p.z2[0], p.z4[0], d & 15);
-    float2 b = cpow_sel(p.z1[1], p.z2[1], p.z4[1], (d >> 4) & 15);
-    float2 c = cpow_sel(p.z1[2], p.z2[2], p.z4[2], (d >> 8) & 15);
-    float2 e = cpow_sel(p.z1[3], p.z2[3], p.z4[3], (d >> 12) & 15);
-    float2 ab = scg_cmul(a, b), ce = scg_cmul(c, e);
-    return fmaf(ab.x, ce.x, -ab.y * ce.y);
-}
-template <int N1>
-__device__ __forceinline__ uint32_t pack_digits(int f) {
-    int c3 = f % N1; f /= N1;
-    int c2 = f % N1; f /= N1;
-    int c1 = f % N1; f /= N1;
-    return (uint32_t)f | ((uint32_t)c1 << 4) | ((uint32_t)c2 << 8) | ((uint32_t)c3 << 12);
-}
-
-__device__ __forceinline__ float4 add_phi(float4 e, const Phasors &p, const uint32_t d[4]) {
-    e.x += phi_digits(p, d[0]); e.y += phi_digits(p, d[1]);
-    e.z += phi_digits(p, d[2]); e.w += phi_digits(p, d[3]);
-    return e;
-}
-__device__ __forceinline__ float add_phi(float e, const Phasors &p, const uint32_t d[1]) { return e + phi_digits(p, d[0]); }
-
-template <int N1, int VEC, int CPT, int NT, int U>
-__global__ void __launch_bounds__(NT) k_trace(int B, int K, const float4 *__restrict__ rec, float *trace,
-                                              float *__restrict__ partial, float gl) {
-    using V = typename VecT<VEC>::type;
-    constexpr int F = N1 * N1 * N1 * N1;
-    constexpr int AF = SCG_A * F;
-    constexpr int NCH = AF / VEC;
-    static_assert(AF % VEC == 0, "vector width must divide the trace");
-    static_assert(VEC == 1 || F % VEC == 0, "a vector must not straddle action rows");
-    static_assert(NT * CPT >= NCH, "not enough threads");
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    V *acc = reinterpret_cast<V *>(smem_raw);  // [K][NCH]
-
-    // per-thread constants: which (row, features) each owned chunk covers
-    int row[CPT];
-    uint32_t dig[CPT][VEC];
-    bool own[CPT];
-#pragma unroll
-    for (int i = 0; i < CPT; ++i) {
-        int c = threadIdx.x + i * NT;
-        own[i] = c < NCH;
-        int e0 = (own[i] ? c : 0) * VEC;
-        row[i] = e0 / F;
-#pragma unroll
-        for (int v = 0; v < VEC; ++v) dig[i][v] = pack_digits<N1>((e0 + v) % F);
-    }
-    for (int i = threadIdx.x; i < K * NCH; i += NT) {
-        if constexpr (VEC == 4) acc[i] = vzero4(); else acc[i] = 0.f;
-    }
-    __syncthreads();
-
-    const int stride = gridDim.x;
-    for (int b0 = blockIdx.x; b0 < B; b0 += U * stride) {
-        // issue every load of the U envs in flight before touching any of them
-        float2 dm[U];          // (delta, meta) of each env: the third 16-byte piece of its record
-        V e[U][CPT];
-        bool live[U];
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            int b = b0 + u * stride;
-            live[u] = b < B;
-            if (live[u]) {
-                dm[u] = __ldg(reinterpret_cast<const float2 *>(rec + (size_t)b * 3 + 2));
-                const V *tp = reinterpret_cast<const V *>(trace + (size_t)b * AF);
-#pragma unroll
-                for (int i = 0; i < CPT; ++i)
-                    if (own[i]) e[u][i] = tp[threadIdx.x + i * NT];
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < U; ++u) {
-            if (!live[u]) continue;
-            int b = b0 + u * stride;
-            uint32_t meta = __float_as_uint(dm[u].y);
-            if (!(meta & SCG_META_ACTIVE)) continue;
-            float delta = dm[u].x;
-            int a = meta & 7, o = (meta >> 8) & 0xFF;
-            bool zero_after = (meta & SCG_META_ZERO_AFTER) != 0;
-            V *tp = reinterpret_cast<V *>(trace + (size_t)b * AF);
-            V *ap = acc + (size_t)o * NCH;
-#pragma unroll
-            for (int i = 0; i < CPT; ++i) {
-                if (!own[i]) continue;
-                int c = threadIdx.x + i * NT;
-                V v = vscale(e[u][i], gl);
-                if (row[i] == a) {   // only the owners of row a rebuild phi(s_b), from the record's phasors
-                    Phasors ph = make_phasors(__ldg(rec + (size_t)b * 3), __ldg(rec + (size_t)b * 3 + 1));
-                    v = add_phi(v, ph, dig[i]);
-                }
-                ap[c] = vfma(delta, v, ap[c]);
-                if (zero_after) {
-                    if constexpr (VEC == 4) v = vzero4(); else v = 0.f;
-                }
-                tp[c] = v;
-            }
-        }
-    }
-    __syncthreads();
-    V *out = reinterpret_cast<V *>(partial + (size_t)blockIdx.x * K * AF);
-    for (int i = threadIdx.x; i < K * NCH; i += NT) out[i] = acc[i];
-}
 
 // ---- windowed (forward-view) sweep: the agent pipeline's K3 --------------------------------------
 // Mirrors oracle/option.py OptionSet.flush.  The fused step kernel left, for each of the T steps of the
@@ -183,9 +49,6 @@ __global__ void __launch_bounds__(NT) k_trace(int B, int K, const float4 *__rest
 // env (orders 4, 5) an extra warp does nothing but the scan (CTRL).  A feature costs two 8-byte shared loads and two
 // FP32 ops to form, and the dense trace crosses HBM once per window: 8*A*F/T + 32 algorithmic bytes per env-step.
 #define SCG_WIN_TB 8   // steps per table block
-#ifndef SCG_WIN_PF
-#define SCG_WIN_PF 1
-#endif
 
 struct WinItem {   // a work item of the sweep: block `blk` of 8 steps of env `b`
     int b, blk;
@@ -615,22 +478,15 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
                 if (lo == (int)((rr.y >> 8) & 0xFF)) continue;         // no contributing step in this segment
                 const uint32_t so = cb.seg_o[sgm];
                 if (so != o_cur) change_option(so);
-#if SCG_WIN_PF
                 float4 en = cb.ent[lo];                  // the list is contiguous across the actions: always one ahead
-#endif
 #pragma unroll
                 for (int r = 0; r < SCG_A; ++r) {        // static register rows: no dynamic indexing, no switch
                     const int hi = r < 3 ? (rr.x >> (8 * (r + 1))) & 0xFF : (rr.y >> (8 * (r - 3))) & 0xFF;
 #pragma unroll 1
                     for (int i = lo; i < hi; ++i) {      // (two steps per trip, to spare the copy: measured equal)
-#if SCG_WIN_PF
                         const float4 nx = cb.ent[i + 1];
                         step_row(tbase + __float_as_int(en.z), en.x, en.y, d, e, r);
                         en = nx;
-#else
-                        const float4 en = cb.ent[i];
-                        step_row(tbase + __float_as_int(en.z), en.x, en.y, d, e, r);
-#endif
                     }
                     lo = hi;
                 }
@@ -763,6 +619,7 @@ static int reduce_slabs(scg_ctx *ctx, int n_slabs, int n, float *dW, cudaStream_
     return 0;
 }
 
+// the window records ([1][B][2] float4) of one step of the dense operator scg_sarsa_update, and its cnt increments
 __global__ void k_make_rec(int B, const float *__restrict__ x, const float *__restrict__ y,
                            const float *__restrict__ vx, const float *__restrict__ vy, const int *__restrict__ a,
                            const int *__restrict__ option, const float *__restrict__ delta,
@@ -770,14 +627,11 @@ __global__ void k_make_rec(int B, const float *__restrict__ x, const float *__re
                            float4 *__restrict__ rec, int *__restrict__ cnt) {
     for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
         bool act = !mask || mask[b];
-        float2 z[4];
-        scg_phasors(x[b], y[b], vx[b], vy[b], z);
         int o = min(max(option[b], 0), K - 1);
         uint32_t meta = (uint32_t)(a[b] & 7) | ((uint32_t)o << 8) | (done[b] ? SCG_META_ZERO_AFTER : 0u) |
                         (act ? SCG_META_ACTIVE : 0u);
-        rec[(size_t)b * 3 + 0] = make_float4(z[0].x, z[0].y, z[1].x, z[1].y);
-        rec[(size_t)b * 3 + 1] = make_float4(z[2].x, z[2].y, z[3].x, z[3].y);
-        rec[(size_t)b * 3 + 2] = make_float4(delta[b], __uint_as_float(meta), 0.f, 0.f);
+        rec[(size_t)b * 2 + 0] = make_float4(x[b], y[b], vx[b], vy[b]);
+        rec[(size_t)b * 2 + 1] = make_float4(delta[b], __uint_as_float(meta), 0.f, 0.f);
         if (act) atomicAdd(cnt + o, 1);
     }
 }
@@ -818,52 +672,6 @@ __global__ void k_apply(int K, int K_opt, float *__restrict__ W, float *__restri
 }
 
 // ---- launch plumbing ----------------------------------------------------------------------------
-static int ensure_partials(scg_ctx *ctx, int n);
-template <int N1, int VEC, int CPT, int NT, int U>
-static int launch_trace_t(scg_ctx *ctx, int B, const float4 *rec, float *trace, float gl, cudaStream_t st) {
-    size_t smem = (size_t)ctx->K * SCG_A * ctx->F * sizeof(float);
-    if (smem > 227 * 1024) return SCG_ELIMIT;   // the CTA accumulator must fit in shared memory
-    auto kern = k_trace<N1, VEC, CPT, NT, U>;
-    static ScgKernelCfg cfgc = {};
-    int per_sm = 0;
-    int rcc = scg_configure(cfgc, kern, NT, smem, &per_sm);
-    if (rcc) return rcc;
-    if (per_sm < 1) return SCG_ELIMIT;
-    int grid = std::max(std::min(B, SCG_NUM_SMS * per_sm), 1);
-    int rc = ensure_partials(ctx, grid);
-    if (rc) return rc;
-    kern<<<grid, NT, smem, st>>>(B, ctx->K, rec, trace, ctx->d_partial, gl);
-    SCG_LAUNCH_CHECK();
-    return grid;
-}
-
-int scg_launch_trace(scg_ctx *ctx, int B, const float *rec, float *trace, float gl, float *dW, cudaStream_t st) {
-    int grid = 0;
-    const float4 *r4 = reinterpret_cast<const float4 *>(rec);
-    static int u3 = -1;
-    if (u3 < 0) {   // SCG_TRACE_U: envs in flight per CTA for the order-3 sweep (tuning knob; default 4)
-        const char *ev = getenv("SCG_TRACE_U");
-        u3 = ev ? atoi(ev) : 4;
-    }
-    // (A bulk-TMA ring variant of this sweep - cp.async.bulk loads into a shared-memory ring, in-place update, bulk
-    // stores - was measured slower on B200: 0.165 vs 0.129 ms at order 3, B = 65,536; with 5 KiB blocks the mbarrier
-    // round trips cost more than register-held loads save.  Removed.)
-    switch (ctx->order) {
-        case 1: grid = launch_trace_t<2, 4, 1, 32, 4>(ctx, B, r4, trace, gl, st); break;
-        case 2: grid = launch_trace_t<3, 1, 2, 224, 2>(ctx, B, r4, trace, gl, st); break;
-        case 3:
-            if (u3 == 2) grid = launch_trace_t<4, 4, 1, 320, 2>(ctx, B, r4, trace, gl, st);
-            else if (u3 == 8) grid = launch_trace_t<4, 4, 1, 320, 8>(ctx, B, r4, trace, gl, st);
-            else grid = launch_trace_t<4, 4, 1, 320, 4>(ctx, B, r4, trace, gl, st);
-            break;
-        case 4: grid = launch_trace_t<5, 1, 4, 800, 2>(ctx, B, r4, trace, gl, st); break;
-        case 5: grid = launch_trace_t<6, 4, 2, 832, 2>(ctx, B, r4, trace, gl, st); break;
-        default: return SCG_ELIMIT;
-    }
-    if (grid <= 0) return grid == 0 ? SCG_EINVAL : grid;
-    return reduce_slabs(ctx, grid, ctx->K * SCG_A * ctx->F, dW, st);
-}
-
 static int ensure_partials(scg_ctx *ctx, int n) {
     if (n <= ctx->n_partials && ctx->d_partial) return 0;
     if (ctx->d_partial) cudaFree(ctx->d_partial);
@@ -889,6 +697,7 @@ template <int N1, int VEC, int NT, int CH, bool MULTI, int MINB, bool CTRL, bool
 static int launch_window_tm(scg_ctx *ctx, int B, int T, int k_used, const float4 *rec, float *trace, float gl,
                             float *dW, cudaStream_t st) {
     const size_t smem = window_smem<N1>(ctx, k_used, MULTI, LISTP);
+    if (smem > 227 * 1024) return SCG_ELIMIT;   // the CTA accumulator must fit in shared memory
     auto kern = k_window<N1, VEC, NT, CH, MULTI, MINB, CTRL, LISTP, L2PF, SPLITP>;
     constexpr int NTT = NT + (CTRL ? 32 : 0);
     static ScgKernelCfg cfgc = {};
@@ -896,10 +705,7 @@ static int launch_window_tm(scg_ctx *ctx, int B, int T, int k_used, const float4
     int rcc = scg_configure(cfgc, kern, NTT, smem, &per_sm);
     if (rcc) return rcc;
     if (per_sm < 1) return SCG_ELIMIT;
-    static int cap = -1;
-    if (cap < 0) { const char *e = getenv("SCG_WIN_CTAS_PER_SM"); cap = e ? atoi(e) : 0; }
-    int occ = cap > 0 ? std::min(cap, per_sm) : per_sm;
-    int grid = std::max(1, std::min(B, SCG_NUM_SMS * occ));
+    int grid = std::max(1, std::min(B, SCG_NUM_SMS * per_sm));
     int rc = ensure_partials(ctx, grid);
     if (rc) return rc;
     kern<<<grid, NTT, smem, st>>>(B, k_used, T, rec, trace, ctx->d_partial, gl, dW, ctx->K);
@@ -923,10 +729,6 @@ int scg_launch_window(scg_ctx *ctx, int B, int T, int k_used, const float *rec, 
     if (T < 1 || T > SCG_WIN_MAX || k_used < 1 || k_used > ctx->K) return SCG_EINVAL;
     const float4 *r4 = reinterpret_cast<const float4 *>(rec);
     int grid = 0, rc;
-    // tuning knobs (defaults = the measured best, see DESIGN.md section 3)
-    static int mode3 = -1, list5 = -1;
-    if (mode3 < 0) { const char *e = getenv("SCG_WIN_MODE3"); mode3 = e ? atoi(e) : 3; }
-    if (list5 < 0) { const char *e = getenv("SCG_WIN_LIST5"); list5 = e ? atoi(e) : 0; }
     if ((rc = scg_prof_push(ctx, 1, st, false))) return rc;
     switch (ctx->order) {
         // <N1, floats per chunk, threads, chunks per thread, min CTAs per SM, scan warp, step lists, L2 prefetch>
@@ -934,20 +736,17 @@ int scg_launch_window(scg_ctx *ctx, int B, int T, int k_used, const float *rec, 
         case 2: grid = launch_window_t<3, 1, 96, 1>(ctx, B, T, k_used, r4, trace, gl, dW, st); break;
         case 3:
             // two warps per env.  With the next trace prefetched into L2 instead of registers the sweep needs 140
-            // registers (7 CTAs per SM) and loses nothing when squeezed to 128 (8 CTAs, while 8 accumulators fit)
-            if (mode3 == 3 && 8 * (window_smem<4>(ctx, k_used, T > SCG_WIN_TB) + 1024) <= 227 * 1024)
+            // registers (7 CTAs per SM) and loses nothing when squeezed to 128 (8 CTAs, while 8 accumulators fit);
+            // with more option slots in use (larger accumulators) the same sweep without the split warps or the squeeze
+            if (8 * (window_smem<4>(ctx, k_used, T > SCG_WIN_TB) + 1024) <= 227 * 1024)
                 grid = launch_window_t<4, 4, 64, 1, 8, false, true, true, true>(ctx, B, T, k_used, r4, trace, gl, dW, st);
-            else if (mode3 >= 2 && 8 * (window_smem<4>(ctx, k_used, T > SCG_WIN_TB) + 1024) <= 227 * 1024)
-                grid = launch_window_t<4, 4, 64, 1, 8, false, true, true>(ctx, B, T, k_used, r4, trace, gl, dW, st);
-            else if (mode3 >= 1) grid = launch_window_t<4, 4, 64, 1, 1, false, true, true>(ctx, B, T, k_used, r4, trace, gl, dW, st);
-            else grid = launch_window_t<4, 4, 64, 1>(ctx, B, T, k_used, r4, trace, gl, dW, st);
+            else grid = launch_window_t<4, 4, 64, 1, 1, false, true, true>(ctx, B, T, k_used, r4, trace, gl, dW, st);
             break;
         case 4: grid = launch_window_t<5, 1, 640, 1>(ctx, B, T, k_used, r4, trace, gl, dW, st); break;
         case 5:
             // one CTA per SM: 11 work warps + a warp that only runs the per-env scan; next trace prefetched in registers
             // (L2 prefetch: 1.98 vs 1.75 ms - one CTA cannot cover the L2 latency); bit-mask loop (step lists: 1.74 vs 1.70 ms)
-            if (list5) grid = launch_window_t<6, 4, 352, 1, 1, true, true>(ctx, B, T, k_used, r4, trace, gl, dW, st);
-            else grid = launch_window_t<6, 4, 352, 1, 1, true, false>(ctx, B, T, k_used, r4, trace, gl, dW, st);
+            grid = launch_window_t<6, 4, 352, 1, 1, true, false>(ctx, B, T, k_used, r4, trace, gl, dW, st);
             break;
         default: return SCG_ELIMIT;
     }
@@ -1010,14 +809,17 @@ extern "C" int scg_sarsa_update(scg_ctx_t *ctx, int B, const float *x, const flo
     if (B > ctx->rec_capacity) {
         if (ctx->d_rec) cudaFree(ctx->d_rec);
         ctx->d_rec = nullptr; ctx->rec_capacity = 0;
-        SCG_CUDA_OK(cudaMalloc((void **)&ctx->d_rec, (size_t)B * SCG_REC_FLOATS * sizeof(float)));
+        SCG_CUDA_OK(cudaMalloc((void **)&ctx->d_rec, (size_t)B * SCG_WREC_FLOATS * sizeof(float)));
         ctx->rec_capacity = B;
     }
     int grid = std::max(1, std::min((B + 255) / 256, SCG_NUM_SMS * 8));
     k_make_rec<<<grid, 256, 0, st>>>(B, x, y, vx, vy, a, option, delta, done, mask, ctx->K,
                                      reinterpret_cast<float4 *>(ctx->d_rec), cnt);
     SCG_LAUNCH_CHECK();
-    return scg_launch_trace(ctx, B, ctx->d_rec, trace, gamma_lambda, dW, st);
+    // the dense update is the forward-view sweep over a window of one step
+    const int n = scg_launch_window(ctx, B, 1, ctx->K, ctx->d_rec, trace, gamma_lambda, dW, st);
+    if (n <= 0) return n == 0 ? SCG_EINVAL : n;
+    return scg_reduce_window(ctx, n, ctx->K, dW, st, false);
 }
 
 extern "C" int scg_apply(int order, int K, float *W, float *Wt, float *dW, int *cnt, float alpha, int window_steps,

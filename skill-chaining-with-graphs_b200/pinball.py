@@ -55,10 +55,9 @@ class PinballMap:
         offs[1:] = np.cumsum([len(p) for p in self.polygons])
         self._handle = C.c_void_p()
         lib = _lib.load()
-        grid_n = int(grid_n) or int(os.environ.get("SCG_GRID_N", "0"))      # 0: the library default (64)
         check(lib.scg_map_create(ptr(verts), ptr(offs), len(self.polygons), self.ball_r, self.target[0],
                                  self.target[1], self.target[2], ptr(self.starts), len(self.starts),
-                                 int(grid_n), C.byref(self._handle)))
+                                 int(grid_n), C.byref(self._handle)))     # grid_n 0: the library default (64)
         self.n_edges = lib.scg_map_num_edges(self._handle)
         self.n_candidates = lib.scg_map_num_candidates(self._handle)
 

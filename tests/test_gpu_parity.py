@@ -249,7 +249,7 @@ def test_q_select_td_match_oracle(scg, torch, order, K):
 
 
 # ---- K3 ------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("order,K", [(3, 4), (1, 2), (2, 2), (4, 2), (5, 8)])
+@pytest.mark.parametrize("order,K", [(3, 4), (3, 8), (1, 2), (2, 2), (4, 2), (5, 8)])
 def test_sarsa_updates_match_oracle(scg, torch, order, K):
     """N updates on a fixed seeded transition batch with a sync every 2 steps: Q values, TD errors,
     traces, dW and weights all within 1e-4 relative of the oracle."""

@@ -38,7 +38,7 @@ def launches(path, out):
     print(open(out).read())
 
 
-def full(rep, out, k3_json=None, k3_pattern="k_trace"):
+def full(rep, out, k3_json=None, k3_pattern="k_window"):
     raw = subprocess.run(["ncu", "-i", rep, "--page", "raw", "--csv"], capture_output=True, text=True).stdout
     rows = list(csv.reader(raw.splitlines()))
     hdr, units = rows[0], rows[1]
