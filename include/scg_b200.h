@@ -157,7 +157,7 @@ typedef struct scg_ctl {
     uint32_t active_mask;          /* bit k set <=> option k is active */
     int32_t n_promotions;          /* promotions decided on the device so far */
     uint32_t last_promotion_step;  /* agent step at which the last one was decided */
-    uint32_t manage_calls;         /* scg_agent_manage launches completed (sequence number of the host mirror) */
+    uint32_t manage_calls;         /* scg_agent_manage launches completed */
     uint32_t reserved[3];
     uint32_t parents[SCG_MAX_OPTIONS]; /* bit j: the initiation set of option j is a target of option k; bit 31: the goal */
 } scg_ctl_t;
@@ -238,7 +238,9 @@ int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
  * host-mapped mirror (scg_agent_poll).  xchg: NULL for a single rank.  Every rank must call it at the same steps. */
 int scg_agent_manage(scg_ctx_t *ctx, scg_agent_t *ag, scg_xchg_t *xchg, void *stream);
 /* Host copy of the controller state as of the last completed scg_agent_manage / scg_agent_set_ctl, without
- * synchronising the device (the values only ever grow, so a stale copy is a valid lower bound). */
+ * synchronising the device.  The copy is always one consistent state: a read that overlaps a write of the mirror is
+ * retried, for up to 1 ms, and then the last consistent copy is returned (the values only ever grow, so a stale copy is
+ * a valid lower bound). */
 int scg_agent_poll(scg_ctx_t *ctx, scg_ctl_t *out /* HOST */);
 /* Overwrite the controller state from the host (tests, checkpoints): device copy on `stream` + the mirror. */
 int scg_agent_set_ctl(scg_ctx_t *ctx, scg_agent_t *ag, const scg_ctl_t *in /* HOST */, void *stream);

@@ -27,7 +27,7 @@
 
 int scg_launch_window(scg_ctx *ctx, int B, int T, int k_used, const float *rec, float *trace, float gl, float *dW,
                       cudaStream_t st);
-int scg_reduce_window(scg_ctx *ctx, int n_slabs, int k_used, float *dW, cudaStream_t st, bool overlap_prev);
+int scg_reduce_window(scg_ctx *ctx, int n_slabs, int k_used, float *dW, cudaStream_t st);
 int scg_prof_push(scg_ctx *ctx, int kind, cudaStream_t st, bool end);
 int scg_launch_top(scg_ctx *ctx, const scg_agent_t *ag, cudaStream_t st);
 
@@ -453,7 +453,7 @@ extern "C" int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
     const int n_slabs = scg_launch_window(ctx, ag->B, ag->win_len, k_used, ag->win_rec, ag->trace, ag->gamma * ag->lambda,
                                           ag->dW, (cudaStream_t)stream);
     if (n_slabs <= 0) return n_slabs == 0 ? SCG_EINVAL : n_slabs;
-    if ((rc = scg_reduce_window(ctx, n_slabs, k_used, ag->dW, (cudaStream_t)stream, false))) return rc;
+    if ((rc = scg_reduce_window(ctx, n_slabs, k_used, ag->dW, (cudaStream_t)stream))) return rc;
     ag->win_len = 0;
     // the event history must have room for the next full window: when it has not, bring the rings up to date now
     if (ag->ev_len + ag->win_cap > ag->ev_cap && (rc = scg_agent_ring(ctx, ag, stream))) return rc;
@@ -469,7 +469,7 @@ static int agent_steps(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, in
     if (b_end < 0) b_end = ag->B;
     cudaStream_t st = (cudaStream_t)stream;
     // promotions happen on the device (scg_agent_manage); the host learns of them from the mirror, without waiting
-    if (ctx->h_ctl) ag->n_active = std::max(ag->n_active, std::min((int)ctx->h_ctl->n_active, ag->K - 1));
+    if (ctx->h_mirror) ag->n_active = std::max(ag->n_active, std::min((int)ctx->h_mirror->ctl.n_active, ag->K - 1));
     StepArgs args;
     args.ag = *ag;
     args.map_blob = map->d_blob;

@@ -98,6 +98,13 @@ struct scg_map {
     size_t stage_cap;
 };
 
+// host-mapped mirror of the device controller state (scg_agent_poll): the block and a sequence word that is odd while
+// a writer (k_manage's tail, scg_agent_set_ctl) stores the block
+struct scg_mirror {
+    scg_ctl_t ctl;
+    uint32_t seq;
+};
+
 #define SCG_HOST_PARTS_MAX 2
 struct scg_ctx {
     int order, K, F;
@@ -113,10 +120,11 @@ struct scg_ctx {
     cudaStream_t host_st[2];
     cudaEvent_t host_evs[2 * SCG_HOST_PARTS_MAX + 1];   // [part] copied in, [MAX + part] stepped, [2 MAX] entry marker
     // controller (scg_ctl.cu)
-    scg_ctl_t *h_ctl;          // host-mapped mirror of the device controller state (scg_agent_poll), allocated on first use
-    scg_ctl_t *d_hctl;         // its device alias
-    unsigned int *d_ring;      // scratch of the example-ring pass: per-CTA option counts, barrier and "done" tickets
-    unsigned int ring_gen;     // launches of the ring pass so far (generation of its grid barrier)
+    scg_mirror *h_mirror;      // host-mapped mirror of the device controller state, allocated on first use
+    scg_mirror *d_mirror;      // its device alias
+    uint32_t mirror_seq;       // the even sequence word the last queued write of the mirror leaves behind
+    scg_ctl_t ctl_snap;        // the last consistent copy of the mirror scg_agent_poll read
+    unsigned int *d_ring;      // scratch of the example-ring pass: per-CTA option counts and the "done" ticket
     // optional per-kernel timing of the agent pipeline (scg_profile_begin / scg_profile_end)
     cudaEvent_t *prof_ev;  // [prof_cap][2] start/stop pairs
     int *prof_kind;        // [prof_cap]
@@ -443,13 +451,19 @@ __device__ __forceinline__ void scg_q_pair(const float2 za[4], const float2 zb[4
 // initiation bits (oracle/agent.py initiation_bits): bit k iff active and z_k >= 0 (sigmoid(z) >= 0.5  <=>  z >= 0), with
 // z_k = theta_k . psi(x, y) formed exactly as oracle/option.py initiation_logit does - fp32, one rounding per operation,
 // the same order - so that the decision is bit-identical to the oracle's, also for states on a classifier's boundary.
-__device__ __forceinline__ float scg_init_logit(const float *__restrict__ t, float x, float y, float xx, float xy, float yy) {
-    float z = __fadd_rn(__ldg(t), __fmul_rn(__ldg(t + 1), x));
-    z = __fadd_rn(z, __fmul_rn(__ldg(t + 2), y));
-    z = __fadd_rn(z, __fmul_rn(__ldg(t + 3), xx));
-    z = __fadd_rn(z, __fmul_rn(__ldg(t + 4), xy));
-    z = __fadd_rn(z, __fmul_rn(__ldg(t + 5), yy));
+// th(j) yields theta_j; it is called where theta_j is used, so a loading th interleaves its loads with the arithmetic.
+template <typename Th>
+__device__ __forceinline__ float scg_init_logit_of(Th th, float x, float y, float xx, float xy, float yy) {
+    float z = __fadd_rn(th(0), __fmul_rn(th(1), x));
+    z = __fadd_rn(z, __fmul_rn(th(2), y));
+    z = __fadd_rn(z, __fmul_rn(th(3), xx));
+    z = __fadd_rn(z, __fmul_rn(th(4), xy));
+    z = __fadd_rn(z, __fmul_rn(th(5), yy));
     return z;
+}
+// the same for a classifier in global memory that no thread of the kernel writes (read-only path)
+__device__ __forceinline__ float scg_init_logit(const float *__restrict__ t, float x, float y, float xx, float xy, float yy) {
+    return scg_init_logit_of([t](int j) { return __ldg(t + j); }, x, y, xx, xy, yy);
 }
 __device__ __forceinline__ uint32_t scg_init_bits(const float *__restrict__ theta, int K, uint32_t active_mask,
                                                   float x, float y) {
@@ -466,5 +480,17 @@ __device__ __forceinline__ float scg_warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
+}
+
+// one example's term of the logistic loss gradient: g += (sigmoid(theta . psi) - label) * psi (classifier fits of
+// scg_q.cu and scg_ctl.cu)
+__device__ __forceinline__ void scg_clf_accum(float px, float py, float lab, const float th[SCG_N_PSI], float g[SCG_N_PSI]) {
+    const float psi[SCG_N_PSI] = {1.f, px, py, px * px, px * py, py * py};
+    float z = 0.f;
+#pragma unroll
+    for (int j = 0; j < SCG_N_PSI; ++j) z = fmaf(th[j], psi[j], z);
+    const float d = 1.0f / (1.0f + expf(-z)) - lab;
+#pragma unroll
+    for (int j = 0; j < SCG_N_PSI; ++j) g[j] = fmaf(d, psi[j], g[j]);
 }
 #endif  // __CUDACC__

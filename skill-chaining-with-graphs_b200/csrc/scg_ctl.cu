@@ -4,12 +4,14 @@
 // Mirrors oracle/agent.py SkillChainAgent.step item 6 (example ring append) and SkillChainAgent.manage (the reference
 // has no code: /root/reference/README.md:1-2).
 //
-// k_ring   The step kernel leaves one event byte per env-step (option terminated? hit? which option) and the option's
-//          start position in the step record.  k_ring turns the events of the steps not yet processed into ring
+// k_ring_count, k_ring_place
+//          The step kernel leaves one event byte per env-step (option terminated? hit? which option) and the option's
+//          start position in the step record.  The ring pass turns the events of the steps not yet processed into ring
 //          appends in exactly the oracle's order - steps in order, envs in order within a step - so the ring contents
 //          (including which examples survive once a ring wraps) do not depend on launch geometry or atomic timing:
-//          per-CTA per-option counts -> grid barrier -> exclusive prefix -> slot = (ex_count + rank) % capacity, and
-//          only the last `capacity` new examples of an option are written (no two writers per slot).
+//          per-CTA per-option counts (k_ring_count) -> exclusive prefix -> slot = (ex_count + rank) % capacity
+//          (k_ring_place, launched after it on the same stream), and only the last `capacity` new examples of an option
+//          are written (no two writers per slot).
 // k_manage One CTA.  Reads the gestating option's success count, and if it qualifies fits its logistic initiation
 //          classifier on its ring by batch gradient descent from theta = 0, flips the option to active and wires the
 //          next gestating slot's parents - all in device memory, so the agent loop never waits for the host.  Across
@@ -20,6 +22,9 @@
 #include <string.h>
 
 #include <algorithm>
+#include <atomic>
+#include <chrono>
+#include <mutex>
 
 #include "scg_common.cuh"
 #include "scg_xchg.cuh"
@@ -30,9 +35,8 @@ int scg_prof_push(scg_ctx *ctx, int kind, cudaStream_t st, bool end);
 #define RING_NT 1024
 #define RING_TILE (RING_NT * 4)      // bytes per tile: one 32-bit word per thread, coalesced
 
-// scratch layout (unsigned int): [RING_CTAS][16] per-CTA option counts | barrier counter | done ticket
-#define RING_BAR (RING_CTAS * SCG_MAX_OPTIONS)
-#define RING_DONE (RING_BAR + 1)
+// scratch layout (unsigned int): [RING_CTAS][16] per-CTA option counts | done ticket
+#define RING_DONE (RING_CTAS * SCG_MAX_OPTIONS)
 #define RING_WORDS (RING_DONE + 1)
 
 // exclusive prefix of one value per thread over the CTA (1024 threads); *total receives the sum
@@ -61,34 +65,30 @@ __device__ __forceinline__ uint32_t ring_block_scan(uint32_t v, uint32_t *warp_s
     return warp_sums[warp] + inc - v;
 }
 
-// CTA c owns the contiguous tiles [c * tiles_per_cta, ...) of the flat [step][env] event-byte array (n bytes, n % 4 == 0
-// after padding by the caller's layout: the array is read as aligned 32-bit words, `mis` leading bytes are skipped).
-__global__ void __launch_bounds__(RING_NT) k_ring(int n, int K, const uint8_t *__restrict__ ev, const float2 *__restrict__ pos,
-                                                  float *ex_xy, uint8_t *ex_label, long long *ex_count, uint32_t cap,
-                                                  unsigned int *scratch, unsigned int target, int tiles_per_cta) {
-    __shared__ uint32_t lst[RING_TILE];                 // this tile's events in flat order: option | hit << 4 | byte index << 8
-    __shared__ uint32_t rk[RING_TILE];                  // their rank among the CTA's events of the same option
-    __shared__ uint32_t warp_sums[32];
-    __shared__ uint32_t cnt_s[SCG_MAX_OPTIONS], base_s[SCG_MAX_OPTIONS], tot_s[SCG_MAX_OPTIONS], run_s[SCG_MAX_OPTIONS];
-    __shared__ uint32_t slot0_s[SCG_MAX_OPTIONS];
-    __shared__ uint32_t n_tile_ev;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+// CTA c of both ring kernels owns the contiguous tiles [c * tiles_per_cta, ...) of the flat [step][env] event-byte array
+// (n bytes, read as aligned 32-bit words: the view starts `mis` = ev % 4 bytes early).  ring_word: the word at byte
+// offset v0 of that view, bytes outside the events [mis, nv) cleared.
+__device__ __forceinline__ uint32_t ring_word(const uint32_t *__restrict__ evw, int mis, long long nv, long long v0) {
+    if (v0 >= nv) return 0u;
+    uint32_t w = __ldg(evw + (v0 >> 2));
+    if (v0 < mis) w &= 0xFFFFFFFFu << (8 * (mis - (int)v0));
+    if (v0 + 4 > nv) w &= 0xFFFFFFFFu >> (8 * (int)(v0 + 4 - nv));
+    return w;
+}
+
+// pass A: this CTA's event count per option -> scratch[blockIdx.x][o]
+__global__ void __launch_bounds__(RING_NT) k_ring_count(int n, const uint8_t *__restrict__ ev, unsigned int *scratch,
+                                                        int tiles_per_cta) {
+    __shared__ uint32_t cnt_s[SCG_MAX_OPTIONS];
+    const int tid = threadIdx.x;
     const int mis = (int)(reinterpret_cast<uintptr_t>(ev) & 3);
     const uint32_t *evw = reinterpret_cast<const uint32_t *>(ev - mis);
-    const long long nv = (long long)n + mis;            // bytes [mis, nv) of the aligned view are the events
+    const long long nv = (long long)n + mis;
     const long long cta_lo = (long long)blockIdx.x * tiles_per_cta * RING_TILE;
-    auto load_word = [&](long long v0) -> uint32_t {    // the aligned word at byte offset v0, bytes outside [mis, nv) cleared
-        if (v0 >= nv) return 0u;
-        uint32_t w = __ldg(evw + (v0 >> 2));
-        if (v0 < mis) w &= 0xFFFFFFFFu << (8 * (mis - (int)v0));
-        if (v0 + 4 > nv) w &= 0xFFFFFFFFu >> (8 * (int)(v0 + 4 - nv));
-        return w;
-    };
-    if (tid < SCG_MAX_OPTIONS) { cnt_s[tid] = 0; run_s[tid] = 0; slot0_s[tid] = tid < K ? (uint32_t)((unsigned long long)ex_count[tid] % cap) : 0u; }
+    if (tid < SCG_MAX_OPTIONS) cnt_s[tid] = 0;
     __syncthreads();
-    // pass A: this CTA's event count per option
     for (int t = 0; t < tiles_per_cta; ++t) {
-        uint32_t w = load_word(cta_lo + (long long)t * RING_TILE + tid * 4) & 0x8F8F8F8Fu;
+        uint32_t w = ring_word(evw, mis, nv, cta_lo + (long long)t * RING_TILE + tid * 4) & 0x8F8F8F8Fu;
         while (w & 0x80808080u) {
             const int j = (__ffs(w & 0x80808080u) - 1) >> 3;
             atomicAdd(&cnt_s[(w >> (8 * j)) & SCG_EV_OPT], 1u);
@@ -97,15 +97,24 @@ __global__ void __launch_bounds__(RING_NT) k_ring(int n, int K, const uint8_t *_
     }
     __syncthreads();
     if (tid < SCG_MAX_OPTIONS) scratch[blockIdx.x * SCG_MAX_OPTIONS + tid] = cnt_s[tid];
-    // grid barrier (all CTAs are co-resident: gridDim.x <= RING_CTAS): generation-counted arrivals
-    __syncthreads();
-    if (tid == 0) {
-        __threadfence();
-        atomicAdd(scratch + RING_BAR, 1u);
-        while ((int)(*reinterpret_cast<volatile unsigned int *>(scratch + RING_BAR) - target) < 0) { }
-        __threadfence();
-    }
-    __syncthreads();
+}
+
+// pass B, on the counts of every CTA that k_ring_count (same grid) left in scratch
+__global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint8_t *__restrict__ ev, const float2 *__restrict__ pos,
+                                                        float *ex_xy, uint8_t *ex_label, long long *ex_count, uint32_t cap,
+                                                        unsigned int *scratch, int tiles_per_cta) {
+    __shared__ uint32_t lst[RING_TILE];                 // this tile's events in flat order: option | hit << 4 | byte index << 8
+    __shared__ uint32_t rk[RING_TILE];                  // their rank among the CTA's events of the same option
+    __shared__ uint32_t warp_sums[32];
+    __shared__ uint32_t base_s[SCG_MAX_OPTIONS], tot_s[SCG_MAX_OPTIONS], run_s[SCG_MAX_OPTIONS];
+    __shared__ uint32_t slot0_s[SCG_MAX_OPTIONS];
+    __shared__ uint32_t n_tile_ev;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int mis = (int)(reinterpret_cast<uintptr_t>(ev) & 3);
+    const uint32_t *evw = reinterpret_cast<const uint32_t *>(ev - mis);
+    const long long nv = (long long)n + mis;
+    const long long cta_lo = (long long)blockIdx.x * tiles_per_cta * RING_TILE;
+    if (tid < SCG_MAX_OPTIONS) { run_s[tid] = 0; slot0_s[tid] = tid < K ? (uint32_t)((unsigned long long)ex_count[tid] % cap) : 0u; }
     // every CTA's per-option totals: threads (c, o) load them with independent loads, 16 threads form this CTA's bases
     for (int i = tid; i < (int)gridDim.x * SCG_MAX_OPTIONS; i += RING_NT) rk[i] = __ldcg(scratch + i);
     __syncthreads();
@@ -120,12 +129,12 @@ __global__ void __launch_bounds__(RING_NT) k_ring(int n, int K, const uint8_t *_
         tot_s[tid] = tt;
     }
     __syncthreads();
-    // pass B: per tile, the ordered event list (block scan), per-option ranks (warp o walks the list with ballots),
-    // then one thread per event places it.  rank = position among this launch's events of the option in (step, env)
-    // order; only the last `cap` of them are written, so every slot has exactly one writer.
+    // per tile, the ordered event list (block scan), per-option ranks (warp o walks the list with ballots), then one
+    // thread per event places it.  rank = position among this pass's events of the option in (step, env) order; only
+    // the last `cap` of them are written, so every slot has exactly one writer.
     for (int t = 0; t < tiles_per_cta; ++t) {
         const long long v0 = cta_lo + (long long)t * RING_TILE + tid * 4;
-        const uint32_t w = load_word(v0);
+        const uint32_t w = ring_word(evw, mis, nv, v0);
         const uint32_t flags = w & 0x80808080u;
         uint32_t total = 0;
         uint32_t off = ring_block_scan(__popc(flags), warp_sums, &n_tile_ev);
@@ -184,21 +193,20 @@ extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
         if (!ctx->d_ring) {
             SCG_CUDA_OK(cudaMalloc((void **)&ctx->d_ring, RING_WORDS * sizeof(unsigned int)));
             SCG_CUDA_OK(cudaMemsetAsync(ctx->d_ring, 0, RING_WORDS * sizeof(unsigned int), st));
-            ctx->ring_gen = 0;
         }
         const long long n = (long long)T * ag->B;
         if (n > 0x7fffffffll) return SCG_ELIMIT;
         const long long n_tiles = (n + 3 + RING_TILE - 1) / RING_TILE;              // (+3: the aligned view may start up to 3 bytes early)
         const int tiles_per_cta = (int)((n_tiles + RING_CTAS - 1) / RING_CTAS);
         const int grid = (int)std::max<long long>(1, (n_tiles + tiles_per_cta - 1) / tiles_per_cta);
-        // the barrier counter counts arrivals of all launches so far: this launch is complete at (sum of earlier grids) + grid
-        ctx->ring_gen += (unsigned int)grid;
         const size_t off = (size_t)ag->ring_len * ag->B;
         int rcp;
         if ((rcp = scg_prof_push(ctx, 4, st, false))) return rcp;
-        k_ring<<<grid, RING_NT, 0, st>>>((int)n, ag->K, ag->ev_hist + off, reinterpret_cast<const float2 *>(ag->ev_pos) + off,
-                                         ag->ex_xy, ag->ex_label, reinterpret_cast<long long *>(ag->ex_count),
-                                         ag->example_capacity, ctx->d_ring, ctx->ring_gen, tiles_per_cta);
+        k_ring_count<<<grid, RING_NT, 0, st>>>((int)n, ag->ev_hist + off, ctx->d_ring, tiles_per_cta);
+        SCG_LAUNCH_CHECK();
+        k_ring_place<<<grid, RING_NT, 0, st>>>((int)n, ag->K, ag->ev_hist + off, reinterpret_cast<const float2 *>(ag->ev_pos) + off,
+                                               ag->ex_xy, ag->ex_label, reinterpret_cast<long long *>(ag->ex_count),
+                                               ag->example_capacity, ctx->d_ring, tiles_per_cta);
         SCG_LAUNCH_CHECK();
         if ((rcp = scg_prof_push(ctx, 4, st, true))) return rcp;
     }
@@ -336,23 +344,14 @@ int scg_launch_top(scg_ctx *ctx, const scg_agent_t *ag, cudaStream_t st) {
 
 struct ManageArgs {
     scg_agent_t ag;
-    scg_ctl_t *mirror;               // host-mapped copy of ctl, written last
+    scg_mirror *mirror;              // host-mapped copy of ctl, written last
+    uint32_t mirror_seq;             // the even sequence word the mirror holds after this write
     int world, rank;
     unsigned char *peer[XCHG_MAX_WORLD];
     size_t m_off;
     uint32_t *status;
     long long timeout_cycles;
 };
-
-__device__ __forceinline__ void manage_accum(float px, float py, float lab, const float th[SCG_N_PSI], float g[SCG_N_PSI]) {
-    const float psi[SCG_N_PSI] = {1.f, px, py, px * px, px * py, py * py};
-    float z = 0.f;
-#pragma unroll
-    for (int j = 0; j < SCG_N_PSI; ++j) z = fmaf(th[j], psi[j], z);
-    const float d = 1.0f / (1.0f + expf(-z)) - lab;
-#pragma unroll
-    for (int j = 0; j < SCG_N_PSI; ++j) g[j] = fmaf(d, psi[j], g[j]);
-}
 
 // Sum `nval` (<= XCHG_M_WORDS) per-rank values over the ranks through the peer-memory block: publish, signal every peer,
 // wait for every peer, add in rank order (identical on every rank).  vals: shared memory, in/out.  One flag round;
@@ -433,9 +432,9 @@ __global__ void __launch_bounds__(MANAGE_NT) k_manage(const __grid_constant__ Ma
             float gs[SCG_N_PSI] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
 #pragma unroll
             for (int k = 0; k < MANAGE_CACHE; ++k)
-                if (tid + k * MANAGE_NT < N) manage_accum(cx[k], cy[k], cl[k], th, gs);
+                if (tid + k * MANAGE_NT < N) scg_clf_accum(cx[k], cy[k], cl[k], th, gs);
             for (int i = tid + MANAGE_CACHE * MANAGE_NT; i < N; i += MANAGE_NT)
-                manage_accum(X[2 * i], X[2 * i + 1], (float)Y[i], th, gs);
+                scg_clf_accum(X[2 * i], X[2 * i + 1], (float)Y[i], th, gs);
 #pragma unroll
             for (int j = 0; j < SCG_N_PSI; ++j) {
                 const float v = scg_warp_sum(gs[j]);
@@ -471,7 +470,7 @@ __global__ void __launch_bounds__(MANAGE_NT) k_manage(const __grid_constant__ Ma
             if (tid < XCHG_M_WORDS) xv[tid] = 0.f;
             __syncthreads();
             if (g.merge_overlap > 0.f) {
-                // inside-counts of the positive examples, per older option (theta_gi was just written: not needed here)
+                // inside-counts of the positive examples, per older option
                 for (int j = 0; j < gi; ++j) {
                     float c = 0.f, np = 0.f;
                     for (int i = tid; i < N; i += MANAGE_NT) {
@@ -486,8 +485,6 @@ __global__ void __launch_bounds__(MANAGE_NT) k_manage(const __grid_constant__ Ma
                     np = scg_warp_sum(np);
                     if (lane == 0) { atomicAdd(&xv[j], c); if (j == 0) atomicAdd(&xv[SCG_MAX_OPTIONS], np); }
                 }
-                if (gi == 0) {      // no older option: still count the positives (not used)
-                }
                 __syncthreads();
                 if (a.world > 1) manage_exchange(a, xv, SCG_MAX_OPTIONS + 1, seq, &s_abort);
                 const float npos = xv[SCG_MAX_OPTIONS];
@@ -496,8 +493,9 @@ __global__ void __launch_bounds__(MANAGE_NT) k_manage(const __grid_constant__ Ma
                     if (frac >= g.merge_overlap) pm |= 1u << j;
                 }
                 const float gx = g.goal_x, gy = g.goal_y;
-                const float zg = scg_init_logit(g.theta + gi * SCG_N_PSI, gx, gy, __fmul_rn(gx, gx), __fmul_rn(gx, gy), __fmul_rn(gy, gy));
-                // (theta_gi as written above: every thread reads it after the barrier)
+                // theta_gi from the registers that hold the fit (this kernel wrote it: not for the read-only path)
+                const float zg = scg_init_logit_of([&](int j) { return th[j]; }, gx, gy, __fmul_rn(gx, gx), __fmul_rn(gx, gy),
+                                                   __fmul_rn(gy, gy));
                 if (zg >= 0.f) pm |= SCG_GOAL_BIT;
             } else {
                 pm = ((1u << (gi + 1)) - 1u) | SCG_GOAL_BIT;
@@ -515,23 +513,31 @@ __global__ void __launch_bounds__(MANAGE_NT) k_manage(const __grid_constant__ Ma
         }
     }
     __syncthreads();
-    // host mirror: everything but the sequence word, fence, then the sequence word
-    if (tid == 0) ctl->manage_calls += 1;
+    // host mirror (a seqlock, read by scg_agent_poll): odd sequence word, the block, even sequence word
+    volatile uint32_t *seq = &a.mirror->seq;
+    if (tid == 0) {
+        ctl->manage_calls += 1;
+        *seq = a.mirror_seq - 1u;
+        __threadfence_system();
+    }
     __syncthreads();
     constexpr int NW = (int)(sizeof(scg_ctl_t) / 4);
     const uint32_t *src = reinterpret_cast<const uint32_t *>(ctl);
-    volatile uint32_t *dst = reinterpret_cast<volatile uint32_t *>(a.mirror);
-    if (tid < NW && tid != 4) dst[tid] = src[tid];
+    volatile uint32_t *dst = reinterpret_cast<volatile uint32_t *>(&a.mirror->ctl);
+    if (tid < NW) dst[tid] = src[tid];
     __threadfence_system();
     __syncthreads();
-    if (tid == 0) dst[4] = src[4];
+    if (tid == 0) *seq = a.mirror_seq;
 }
 
+// guards scg_ctx::ctl_snap: scg_agent_poll may be called from several host threads at once
+static std::mutex ctl_snap_mutex;
+
 static int ensure_mirror(scg_ctx *ctx) {
-    if (ctx->h_ctl) return 0;
-    SCG_CUDA_OK(cudaHostAlloc((void **)&ctx->h_ctl, sizeof(scg_ctl_t), cudaHostAllocMapped));
-    memset(ctx->h_ctl, 0, sizeof(scg_ctl_t));
-    SCG_CUDA_OK(cudaHostGetDevicePointer((void **)&ctx->d_hctl, (void *)ctx->h_ctl, 0));
+    if (ctx->h_mirror) return 0;
+    SCG_CUDA_OK(cudaHostAlloc((void **)&ctx->h_mirror, sizeof(scg_mirror), cudaHostAllocMapped));
+    memset(ctx->h_mirror, 0, sizeof(scg_mirror));
+    SCG_CUDA_OK(cudaHostGetDevicePointer((void **)&ctx->d_mirror, (void *)ctx->h_mirror, 0));
     return 0;
 }
 
@@ -546,7 +552,8 @@ extern "C" int scg_agent_manage(scg_ctx_t *ctx, scg_agent_t *ag, scg_xchg_t *xch
     ManageArgs a;
     memset(&a, 0, sizeof(a));
     a.ag = *ag;
-    a.mirror = ctx->d_hctl;
+    a.mirror = ctx->d_mirror;
+    a.mirror_seq = ctx->mirror_seq += 2;
     a.world = xchg ? xchg->world : 1;
     a.rank = xchg ? xchg->rank : 0;
     if (xchg) {
@@ -564,7 +571,7 @@ extern "C" int scg_agent_manage(scg_ctx_t *ctx, scg_agent_t *ag, scg_xchg_t *xch
     if ((rc = scg_prof_push(ctx, 5, (cudaStream_t)stream, true))) return rc;
     if (ctx->deterministic) {   // reproducible runs: the host sizes the next launches with exact knowledge
         SCG_CUDA_OK(cudaStreamSynchronize((cudaStream_t)stream));
-        ag->n_active = std::max(ag->n_active, (int)ctx->h_ctl->n_active);
+        ag->n_active = std::max(ag->n_active, (int)ctx->h_mirror->ctl.n_active);
     }
     return 0;
 }
@@ -573,14 +580,29 @@ extern "C" int scg_agent_poll(scg_ctx_t *ctx, scg_ctl_t *out) {
     if (!ctx || !out) return SCG_EINVAL;
     int rc = ensure_mirror(ctx);
     if (rc) return rc;
-    const volatile uint32_t *src = reinterpret_cast<const volatile uint32_t *>(ctx->h_ctl);
-    uint32_t *dst = reinterpret_cast<uint32_t *>(out);
-    // the kernel writes the sequence word last: re-read until it is stable around the copy
-    for (int tries = 0; tries < 4; ++tries) {
-        const uint32_t s0 = src[4];
+    const volatile uint32_t *seq = &ctx->h_mirror->seq;
+    const volatile uint32_t *src = reinterpret_cast<const volatile uint32_t *>(&ctx->h_mirror->ctl);
+    // a copy taken while the sequence word stayed the same even value is consistent.  A writer holds the word odd for
+    // a few microseconds: retry for up to 1 ms, then fall back to the last consistent copy (a stale copy is a valid
+    // lower bound, and a device that stopped in the middle of a write cannot hang the host)
+    const auto t_end = std::chrono::steady_clock::now() + std::chrono::milliseconds(1);
+    do {
+        const uint32_t s0 = *seq;
+        if (s0 & 1u) continue;
+        std::atomic_thread_fence(std::memory_order_acquire);
+        scg_ctl_t c;
+        uint32_t *dst = reinterpret_cast<uint32_t *>(&c);
         for (size_t i = 0; i < sizeof(scg_ctl_t) / 4; ++i) dst[i] = src[i];
-        if (src[4] == s0) break;
-    }
+        std::atomic_thread_fence(std::memory_order_acquire);
+        if (*seq == s0) {
+            *out = c;
+            std::lock_guard<std::mutex> lk(ctl_snap_mutex);
+            ctx->ctl_snap = c;
+            return 0;
+        }
+    } while (std::chrono::steady_clock::now() < t_end);
+    std::lock_guard<std::mutex> lk(ctl_snap_mutex);
+    *out = ctx->ctl_snap;
     return 0;
 }
 
@@ -591,8 +613,17 @@ extern "C" int scg_agent_set_ctl(scg_ctx_t *ctx, scg_agent_t *ag, const scg_ctl_
     if (rc) return rc;
     // staged through the mirror (pinned): the copy is asynchronous and ordered on the stream
     SCG_CUDA_OK(cudaStreamSynchronize((cudaStream_t)stream));   // a manage kernel in flight may still write the mirror
-    memcpy(ctx->h_ctl, in, sizeof(scg_ctl_t));
-    SCG_CUDA_OK(cudaMemcpyAsync(ag->ctl, ctx->h_ctl, sizeof(scg_ctl_t), cudaMemcpyHostToDevice, (cudaStream_t)stream));
+    volatile uint32_t *seq = &ctx->h_mirror->seq;
+    *seq = ctx->mirror_seq + 1u;
+    std::atomic_thread_fence(std::memory_order_release);
+    memcpy(&ctx->h_mirror->ctl, in, sizeof(scg_ctl_t));
+    std::atomic_thread_fence(std::memory_order_release);
+    *seq = ctx->mirror_seq += 2;
+    {
+        std::lock_guard<std::mutex> lk(ctl_snap_mutex);
+        ctx->ctl_snap = *in;
+    }
+    SCG_CUDA_OK(cudaMemcpyAsync(ag->ctl, &ctx->h_mirror->ctl, sizeof(scg_ctl_t), cudaMemcpyHostToDevice, (cudaStream_t)stream));
     SCG_CUDA_OK(cudaStreamSynchronize((cudaStream_t)stream));
     ag->n_active = in->n_active;
     return 0;

@@ -170,24 +170,15 @@ __device__ __forceinline__ void clf_load(int N, const float *__restrict__ X, con
         c.lab[k] = in ? (float)y[i] : 0.f;
     }
 }
-__device__ __forceinline__ void clf_accum(float px, float py, float lab, const float th[SCG_N_PSI], float g[SCG_N_PSI]) {
-    const float psi[SCG_N_PSI] = {1.f, px, py, px * px, px * py, py * py};
-    float z = 0.f;
-#pragma unroll
-    for (int j = 0; j < SCG_N_PSI; ++j) z = fmaf(th[j], psi[j], z);
-    const float d = 1.0f / (1.0f + expf(-z)) - lab;
-#pragma unroll
-    for (int j = 0; j < SCG_N_PSI; ++j) g[j] = fmaf(d, psi[j], g[j]);
-}
 __device__ __forceinline__ void clf_grad_block(int N, const float *__restrict__ X, const uint8_t *__restrict__ y,
                                                const ClfCache &c, const float th[SCG_N_PSI], float g_out[SCG_N_PSI],
                                                float *sm) {
     float g[SCG_N_PSI] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
 #pragma unroll
     for (int k = 0; k < CLF_CACHE; ++k)
-        if ((int)(threadIdx.x + k * blockDim.x) < N) clf_accum(c.x[k], c.y[k], c.lab[k], th, g);
+        if ((int)(threadIdx.x + k * blockDim.x) < N) scg_clf_accum(c.x[k], c.y[k], c.lab[k], th, g);
     for (int i = threadIdx.x + CLF_CACHE * blockDim.x; i < N; i += blockDim.x)
-        clf_accum(X[2 * i], X[2 * i + 1], (float)y[i], th, g);
+        scg_clf_accum(X[2 * i], X[2 * i + 1], (float)y[i], th, g);
     int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
 #pragma unroll
     for (int j = 0; j < SCG_N_PSI; ++j) {

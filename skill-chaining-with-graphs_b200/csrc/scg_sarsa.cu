@@ -594,7 +594,7 @@ __global__ void __launch_bounds__(256) k_reduce(int n_partials, int n, const flo
 }
 
 // slabs -> dW on stream st
-static int reduce_slabs(scg_ctx *ctx, int n_slabs, int n, float *dW, cudaStream_t st, bool overlap_prev = false) {
+static int reduce_slabs(scg_ctx *ctx, int n_slabs, int n, float *dW, cudaStream_t st) {
     const int nx_max = (ctx->K * SCG_A * ctx->F + 255) / 256;
     if (ctx->deterministic && !ctx->d_red) {
         SCG_CUDA_OK(cudaMalloc((void **)&ctx->d_red, (size_t)SCG_RED_SLICES * ctx->K * SCG_A * ctx->F * sizeof(float)));
@@ -602,20 +602,8 @@ static int reduce_slabs(scg_ctx *ctx, int n_slabs, int n, float *dW, cudaStream_
         SCG_CUDA_OK(cudaMemsetAsync(ctx->d_tickets, 0, (size_t)nx_max * sizeof(unsigned int), st));
     }
     dim3 g((n + 255) / 256, std::min(n_slabs, SCG_RED_SLICES));
-    // overlap_prev: the kernel launched just before this one (the example-ring pass) is independent of the reduction, so
-    // the reduction may start under it (programmatic dependent launch; k_ring releases its dependents at its start)
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = g;
-    cfg.blockDim = dim3(256);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = overlap_prev ? 1 : 0;
-    SCG_CUDA_OK(cudaLaunchKernelEx(&cfg, k_reduce, n_slabs, n, (const float *)ctx->d_partial, ctx->d_red,
-                                   ctx->deterministic ? ctx->d_tickets : (unsigned int *)nullptr, dW));
-    ++g_scg_launches;
+    k_reduce<<<g, 256, 0, st>>>(n_slabs, n, ctx->d_partial, ctx->d_red, ctx->deterministic ? ctx->d_tickets : nullptr, dW);
+    SCG_LAUNCH_CHECK();
     return 0;
 }
 
@@ -755,10 +743,10 @@ int scg_launch_window(scg_ctx *ctx, int B, int T, int k_used, const float *rec, 
     return grid;
 }
 
-int scg_reduce_window(scg_ctx *ctx, int n_slabs, int k_used, float *dW, cudaStream_t st, bool overlap_prev) {
+int scg_reduce_window(scg_ctx *ctx, int n_slabs, int k_used, float *dW, cudaStream_t st) {
     int rc;
     if ((rc = scg_prof_push(ctx, 2, st, false))) return rc;
-    if ((rc = reduce_slabs(ctx, n_slabs, k_used * SCG_A * ctx->F, dW, st, overlap_prev && !ctx->prof_on))) return rc;
+    if ((rc = reduce_slabs(ctx, n_slabs, k_used * SCG_A * ctx->F, dW, st))) return rc;
     return scg_prof_push(ctx, 2, st, true);
 }
 
@@ -789,7 +777,7 @@ extern "C" int scg_ctx_destroy(scg_ctx_t *c) {
     if (c->host_ev) cudaEventDestroy(c->host_ev);
     for (int i = 0; i < 2; ++i) if (c->host_st[i]) cudaStreamDestroy(c->host_st[i]);
     for (int i = 0; i < 2 * SCG_HOST_PARTS_MAX + 1; ++i) if (c->host_evs[i]) cudaEventDestroy(c->host_evs[i]);
-    if (c->h_ctl) cudaFreeHost(c->h_ctl);
+    if (c->h_mirror) cudaFreeHost(c->h_mirror);
     if (c->d_ring) cudaFree(c->d_ring);
     for (int i = 0; i < 2 * c->prof_cap; ++i) cudaEventDestroy(c->prof_ev[i]);
     free(c->prof_ev);
@@ -819,7 +807,7 @@ extern "C" int scg_sarsa_update(scg_ctx_t *ctx, int B, const float *x, const flo
     // the dense update is the forward-view sweep over a window of one step
     const int n = scg_launch_window(ctx, B, 1, ctx->K, ctx->d_rec, trace, gamma_lambda, dW, st);
     if (n <= 0) return n == 0 ? SCG_EINVAL : n;
-    return scg_reduce_window(ctx, n, ctx->K, dW, st, false);
+    return scg_reduce_window(ctx, n, ctx->K, dW, st);
 }
 
 extern "C" int scg_apply(int order, int K, float *W, float *Wt, float *dW, int *cnt, float alpha, int window_steps,

@@ -681,10 +681,12 @@ def test_top_level_learner_matches_oracle(scg, torch, order, K, n_active, name, 
 
 # ---- controller on the device: example rings and promote-and-fit -------------------------------------------
 @pytest.mark.parametrize("B,cap,launch,hist,horizon", [(3000, 64, "window", 64, 1 << 30), (3000, 64, "step", 8, 1), (777, 4096, "window", 8, 2),
-                                                       (40000, 1000, "window", 64, 1 << 30), (5000, 300, "window", 12, 1 << 30)])
+                                                       (40000, 1000, "window", 64, 1 << 30), (5000, 300, "window", 12, 1 << 30),
+                                                       (70000, 1000, "window", 64, 1 << 30)])
 def test_example_rings_match_oracle_past_capacity(scg, torch, B, cap, launch, hist, horizon):
     """The rings hold the oracle's examples in the oracle's slots - steps in order, envs in order within a step - also
-    when a ring wraps several times inside one launch (cap 64, thousands of terminations per window)."""
+    when a ring wraps several times inside one launch (cap 64, thousands of terminations per window), and when a pass
+    spans more than one tile per CTA (B = 70000: the 8-step pass of windows 1 and 2 is 137 tiles of 4 KB)."""
     from oracle_replay import activate, default_theta
     K, n_active = 4, 2
     # hist: steps of event history on the device (8 = two windows: a ring pass at every flush; 64: only when somebody
@@ -829,6 +831,58 @@ def test_promotion_the_host_has_not_seen_yet_is_still_correct(scg, torch):
         assert torch.equal(a.n_success, b.n_success) and torch.equal(a.t_opt, b.t_opt)
         assert_close(b.options.W.cpu().numpy(), a.options.W.cpu().numpy(), rtol=1e-5, what=f"order {order}: W")
         assert_close(b.options._trace.cpu().numpy(), a.options._trace.cpu().numpy(), rtol=1e-5, what=f"order {order}: traces")
+
+
+def test_poll_returns_consistent_snapshots_while_the_device_promotes(scg, torch):
+    """scg_agent_poll from a second host thread while the main thread queues steps and promotions (chain mode, every
+    manage() promotes until the last slot): every snapshot is one state the controller was in - mask, count, promotions
+    and the new slot's parents agree - and manage_calls never goes back."""
+    import ctypes as C
+    import threading
+    from skill_chaining_with_graphs_b200._lib import CtlStruct, check
+    lib = scg.load_library()
+    K = 12
+    gag = scg.SkillChainAgent(scg.AgentConfig(map="easy", batch=4096, order=1, max_options=K, gestation_successes=0,
+                                              clf_steps=4, sync_interval=4))
+    bad, n_polls, stop = [], [0], threading.Event()
+
+    def poll():
+        m, last_calls = CtlStruct(), 0
+        while not stop.is_set():
+            check(lib.scg_agent_poll(gag.options.ctx, C.byref(m)))
+            n, calls = int(m.n_active), int(m.manage_calls)
+            ok = (n >= 1 and m.active_mask == (1 << n) - 1 and m.n_promotions == n - 1 and m.parents[n] == 1 << (n - 1)
+                  and calls >= last_calls)
+            if not ok and len(bad) < 5:
+                bad.append(dict(n_active=n, active_mask=int(m.active_mask), n_promotions=int(m.n_promotions),
+                                parents=[int(v) for v in m.parents[:K]], manage_calls=(last_calls, calls)))
+            last_calls = calls
+            n_polls[0] += 1
+
+    def reset():            # option 0 active, slot 1 gestating, no promotions: through scg_agent_set_ctl
+        gag.controller_state(sync=True)
+        c = gag._ctl
+        c.n_active, c.active_mask, c.n_promotions = 1, 1, 0
+        for k in range(K):
+            c.parents[k] = 0
+        c.parents[0], c.parents[1] = 1 << 31, 1
+        gag._push_ctl()
+
+    reset()
+    th = threading.Thread(target=poll)
+    th.start()
+    try:
+        for _ in range(10):
+            for _ in range(K - 1):
+                gag.run(4)
+                gag.manage()
+            assert gag.controller_state()["n_active"] == K - 1
+            reset()
+    finally:
+        stop.set()
+        th.join()
+    assert not bad, bad
+    assert n_polls[0] > 100
 
 
 def _two_rank_agents_one_device(scg, torch, Bh, streams, **kw):
