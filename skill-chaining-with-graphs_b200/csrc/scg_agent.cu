@@ -45,47 +45,6 @@ struct StepArgs {
     float *top;   // this step's slab of the top-level update records: [B][8] (top_slots > 0)
 };
 
-// bulk-TMA staging of up to three global blocks into shared memory behind one mbarrier
-__device__ __forceinline__ void stage3(unsigned char *dst0, const void *src0, int bytes0, unsigned char *dst1,
-                                       const void *src1, int bytes1, unsigned char *dst2, const void *src2, int bytes2,
-                                       unsigned long long *bar) {
-    uint32_t bar_a = smem_u32(bar);
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a),
-                     "r"(bytes0 + bytes1 + bytes2)
-                     : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                         smem_u32(dst0)),
-                     "l"(src0), "r"(bytes0), "r"(bar_a)
-                     : "memory");
-        if (bytes1 > 0)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             smem_u32(dst1)),
-                         "l"(src1), "r"(bytes1), "r"(bar_a)
-                         : "memory");
-        if (bytes2 > 0)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                             smem_u32(dst2)),
-                         "l"(src2), "r"(bytes2), "r"(bar_a)
-                         : "memory");
-    }
-    uint32_t ok = 0;
-    while (!ok) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok)
-            : "r"(bar_a)
-            : "memory");
-    }
-}
-
 // Q_slot(z, .) for the lanes of `mask` (a warp-uniform ballot), compacted: N1 lanes share one of those envs, one leading
 // multi-index digit c0 each, and the partial sums are folded back to the env's own lane.  `z` and `slot` are the env's
 // phasors and weight-table slot (valid on the lanes of mask); q receives the 5 values on those lanes.
@@ -379,14 +338,15 @@ static int launch_step_tt(const StepArgs &args, size_t smem, cudaStream_t st) {
     int per_sm = 0;
     int rcc = scg_configure(cfgc, kern, NTH, smem, &per_sm);
     if (rcc) return rcc;
-    if (per_sm < 1) return SCG_ELIMIT;
+    const int sms = scg_num_sms();
+    if (per_sm < 1 || sms < 1) return SCG_ELIMIT;
     constexpr int WPC = NTH / 32;                       // warps (tiles in flight) per CTA
     const int n_tiles = (args.b_end - args.b_begin + 31) / 32;
     // enough CTAs for one warp per tile if they all fit at once, else every resident slot
     int grid = (n_tiles + WPC - 1) / WPC;
-    if (grid > SCG_NUM_SMS) {   // same number of CTAs on every SM: as many rounds of 148 as the tiles need, if resident
-        const int rounds = std::min(per_sm, (grid + SCG_NUM_SMS - 1) / SCG_NUM_SMS);
-        grid = SCG_NUM_SMS * rounds;
+    if (grid > sms) {   // same number of CTAs on every SM: as many rounds of one CTA per SM as the tiles need, if resident
+        const int rounds = std::min(per_sm, (grid + sms - 1) / sms);
+        grid = sms * rounds;
     }
     grid = std::max(grid, 1);
     cudaLaunchConfig_t cfg = {};

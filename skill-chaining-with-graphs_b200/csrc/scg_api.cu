@@ -3,6 +3,14 @@
 
 uint64_t g_scg_launches = 0;
 
+int scg_num_sms() {
+    static int sms[SCG_MAX_DEVICES];
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= SCG_MAX_DEVICES) return 0;
+    if (sms[dev] == 0 && cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) sms[dev] = 0;
+    return sms[dev];
+}
+
 extern "C" const char *scg_error_string(int code) {
     if (code == 0) return "ok";
     if (code == SCG_EINVAL) return "scg: invalid argument";

@@ -7,7 +7,6 @@
 
 #define SCG_A SCG_N_ACTIONS
 #define SCG_WREC_FLOATS 8
-#define SCG_NUM_SMS 148
 
 // window step record (agent pipeline and scg_sarsa_update), 32 bytes per env-step:
 //   [0..3]  x, y, vx, vy of the state the update is for     [4] delta     [5] meta bits     [6],[7] unused
@@ -48,9 +47,21 @@ extern uint64_t g_scg_launches;  // host-side launch counter (scg_api.cu)
 
 static inline int scg_pow4(int n1) { return n1 * n1 * n1 * n1; }
 
+#define SCG_MAX_DEVICES 32
+
+// SMs of the current device, read once per device (scg_api.cu); 0 if it cannot be read, and a launch sized from that
+// fails its launch check
+int scg_num_sms();
+
+// blocks for n items at `threads` per block, at most blocks_per_sm_cap per SM (at least one)
+static inline int scg_grid(int n, int threads, int blocks_per_sm_cap) {
+    const int blocks = (n + threads - 1) / threads, cap = scg_num_sms() * blocks_per_sm_cap;
+    if (cap < 1) return 0;
+    return blocks < 1 ? 1 : (blocks < cap ? blocks : cap);
+}
+
 // Per-device cache of a kernel's dynamic shared-memory opt-in and occupancy (cudaFuncSetAttribute is per device,
 // and one process may drive several devices).
-#define SCG_MAX_DEVICES 32
 struct ScgKernelCfg {
     size_t configured[SCG_MAX_DEVICES];
     int per_sm[SCG_MAX_DEVICES];
@@ -482,8 +493,8 @@ __device__ __forceinline__ float scg_warp_sum(float v) {
     return v;
 }
 
-// one example's term of the logistic loss gradient: g += (sigmoid(theta . psi) - label) * psi (classifier fits of
-// scg_q.cu and scg_ctl.cu)
+// ---- logistic initiation classifier fit (k_clf_grad / k_clf_fit in scg_q.cu, k_manage in scg_ctl.cu) --------------
+// one example's term of the logistic loss gradient: g += (sigmoid(theta . psi) - label) * psi
 __device__ __forceinline__ void scg_clf_accum(float px, float py, float lab, const float th[SCG_N_PSI], float g[SCG_N_PSI]) {
     const float psi[SCG_N_PSI] = {1.f, px, py, px * px, px * py, py * py};
     float z = 0.f;
@@ -492,5 +503,96 @@ __device__ __forceinline__ void scg_clf_accum(float px, float py, float lab, con
     const float d = 1.0f / (1.0f + expf(-z)) - lab;
 #pragma unroll
     for (int j = 0; j < SCG_N_PSI; ++j) g[j] = fmaf(d, psi[j], g[j]);
+}
+
+// The fits run in one CTA.  Each thread keeps up to CLF_CACHE of its examples in registers, so the gradient-descent loop
+// touches global memory only for the examples beyond blockDim.x * CLF_CACHE.
+#define CLF_CACHE 8
+struct ClfCache {
+    float x[CLF_CACHE], y[CLF_CACHE], lab[CLF_CACHE];
+};
+__device__ __forceinline__ void clf_load(int N, const float *__restrict__ X, const uint8_t *__restrict__ y, ClfCache &c) {
+#pragma unroll
+    for (int k = 0; k < CLF_CACHE; ++k) {
+        const int i = threadIdx.x + k * blockDim.x;
+        const bool in = i < N;
+        c.x[k] = in ? X[2 * i] : 0.f;
+        c.y[k] = in ? X[2 * i + 1] : 0.f;
+        c.lab[k] = in ? (float)y[i] : 0.f;
+    }
+}
+// sum_i (p_i - y_i) psi_i over the N examples -> g_sum on every thread: per-thread partial sums, warp shuffles, then warp 0
+// folds the per-warp sums in warp order.  sm: 33 * SCG_N_PSI floats of shared memory.
+__device__ __forceinline__ void clf_grad_sum(int N, const float *__restrict__ X, const uint8_t *__restrict__ y,
+                                             const ClfCache &c, const float th[SCG_N_PSI], float g_sum[SCG_N_PSI],
+                                             float *sm) {
+    float g[SCG_N_PSI] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int k = 0; k < CLF_CACHE; ++k)
+        if ((int)(threadIdx.x + k * blockDim.x) < N) scg_clf_accum(c.x[k], c.y[k], c.lab[k], th, g);
+    for (int i = threadIdx.x + CLF_CACHE * blockDim.x; i < N; i += blockDim.x)
+        scg_clf_accum(X[2 * i], X[2 * i + 1], (float)y[i], th, g);
+    int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+#pragma unroll
+    for (int j = 0; j < SCG_N_PSI; ++j) {
+        float v = scg_warp_sum(g[j]);
+        if (lane == 0) sm[warp * SCG_N_PSI + j] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < 32) {   // warp 0 folds the per-warp sums: lane (w % 32) holds warp w's value of component j
+#pragma unroll
+        for (int j = 0; j < SCG_N_PSI; ++j) {
+            float v = (lane < nw) ? sm[lane * SCG_N_PSI + j] : 0.f;
+            v = scg_warp_sum(v);
+            if (lane == 0) sm[32 * SCG_N_PSI + j] = v;
+        }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < SCG_N_PSI; ++j) g_sum[j] = sm[32 * SCG_N_PSI + j];
+    __syncthreads();
+}
+// one gradient-descent step on the mean gradient g_sum / n
+__device__ __forceinline__ void clf_step(float th[SCG_N_PSI], float lr, const float g_sum[SCG_N_PSI], float n) {
+#pragma unroll
+    for (int j = 0; j < SCG_N_PSI; ++j) th[j] = __fsub_rn(th[j], __fmul_rn(lr, __fdiv_rn(g_sum[j], n)));
+}
+
+// ---- weight apply (k_apply in scg_sarsa.cu, k_sync in scg_xchg.cu) -------------------------------------------------
+// Element i of W [K][5][F]:  W += (alpha * alpha_scale_f) * (delta * (steps / c))  when its slot's count c > 0;  refresh
+// the packed copy Wt;  dW <- 0.  delta is this element of the window's dW (summed over ranks by k_sync).  Slots
+// k >= K_opt hold the top-level learner (oracle/option.py): step size alpha_top, mean over the window's events.
+template <int N1>
+__device__ __forceinline__ void scg_apply_elem(int i, int c, int K_opt, float alpha, float alpha_top, float steps, float delta,
+                                               float *W, float *Wt, float *dW) {
+    constexpr int F = N1 * N1 * N1 * N1;
+    const int f = i % F, ka = i / F, a = ka % SCG_A, k = ka / SCG_A;
+    float w = W[i];
+    if (c > 0) {
+        int d = f, ss = 0;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { int q = d % N1; ss += q * q; d /= N1; }
+        const float as = (ss == 0) ? 1.0f : (float)(1.0 / sqrt((double)ss));
+        const bool top = k >= K_opt;
+        const float scale = __fdiv_rn(top ? 1.0f : steps, (float)c);
+        w = __fadd_rn(w, __fmul_rn(__fmul_rn(top ? alpha_top : alpha, as), __fmul_rn(delta, scale)));
+        W[i] = w;
+    }
+    Wt[(size_t)k * WtLayout<N1>::SLOT_FLOATS + WtLayout<N1>::index(a, f)] = w;
+    dW[i] = 0.f;
+}
+
+// True on every thread of the last CTA of the grid to get here; every thread of the CTA must call it.  The CTA's
+// earlier writes are visible grid-wide before the ticket moves.  atomicInc wraps the ticket back to 0 on the last CTA,
+// so the same ticket serves the next launch on the same stream.
+__device__ __forceinline__ bool scg_last_block(unsigned int *ticket) {
+    __shared__ bool last;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        last = atomicInc(ticket, gridDim.x - 1) == gridDim.x - 1;
+    }
+    __syncthreads();
+    return last;
 }
 #endif  // __CUDACC__

@@ -173,13 +173,7 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
         __syncthreads();
     }
     // the last CTA to finish advances the counts (every CTA has read them by then)
-    __shared__ bool last;
-    if (tid == 0) {
-        __threadfence();
-        last = atomicInc(scratch + RING_DONE, gridDim.x - 1) == gridDim.x - 1;
-    }
-    __syncthreads();
-    if (last && tid < K) ex_count[tid] += (long long)tot_s[tid];
+    if (scg_last_block(scratch + RING_DONE) && tid < K) ex_count[tid] += (long long)tot_s[tid];
 }
 
 extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
@@ -303,6 +297,18 @@ __global__ void __launch_bounds__(TOP_NT) k_top(int n, int K, int top_slots, con
     if (tid < top_slots) atomicAdd(cnt + K + tid, ne);
 }
 
+template <int N1>
+static int launch_top(const scg_agent_t *ag, int n, int grid, size_t smem, cudaStream_t st) {
+    static ScgKernelCfg cfgc = {};
+    int per_sm = 0;
+    int rc = scg_configure(cfgc, k_top<N1>, TOP_NT, smem, &per_sm);
+    if (rc) return rc;
+    k_top<N1><<<grid, TOP_NT, smem, st>>>(n, ag->K, ag->top_slots, ag->ev_hist + (size_t)(ag->ev_len - ag->win_len) * ag->B,
+                                          reinterpret_cast<const float4 *>(ag->win_top), ag->dW, ag->cnt);
+    SCG_LAUNCH_CHECK();
+    return 0;
+}
+
 // fold the open window's top-level update records (slabs 0 .. win_len-1) into dW / cnt
 int scg_launch_top(scg_ctx *ctx, const scg_agent_t *ag, cudaStream_t st) {
     if (ag->top_slots <= 0 || ag->win_len <= 0 || ag->B <= 0) return 0;
@@ -311,36 +317,16 @@ int scg_launch_top(scg_ctx *ctx, const scg_agent_t *ag, cudaStream_t st) {
     if (n > 0x7fffffffll) return SCG_ELIMIT;
     const int grid = (int)std::max<long long>(1, std::min<long long>(TOP_CTAS, (n + 4095) / 4096));
     const int chunk = (int)((n + grid - 1) / grid);
-    const int N1 = ctx->order + 1;
-    const size_t smem = ((((size_t)ag->K * ctx->F + 3) & ~(size_t)3)) * sizeof(float) + (size_t)TOP_EB * 4 * N1 * sizeof(float2) +
+    const size_t smem = ((((size_t)ag->K * ctx->F + 3) & ~(size_t)3)) * sizeof(float) + (size_t)TOP_EB * 4 * (ctx->order + 1) * sizeof(float2) +
                         TOP_EB * (sizeof(float) + sizeof(int)) + (size_t)chunk * sizeof(int);
     if (smem > 200 * 1024) return SCG_ELIMIT;
-    const float4 *top = reinterpret_cast<const float4 *>(ag->win_top);
     int rc = 0;
-#define LAUNCH_TOP(N)                                                                                              \
-    {                                                                                                               \
-        static ScgKernelCfg cfgc = {};                                                                              \
-        int per_sm = 0;                                                                                             \
-        rc = scg_configure(cfgc, k_top<N>, TOP_NT, smem, &per_sm);                                                  \
-        if (!rc) k_top<N><<<grid, TOP_NT, smem, st>>>((int)n, ag->K, ag->top_slots, ag->ev_hist + (size_t)(ag->ev_len - ag->win_len) * ag->B, top, ag->dW, ag->cnt); \
-    }
-    switch (ctx->order) {
-        case 1: LAUNCH_TOP(2); break;
-        case 2: LAUNCH_TOP(3); break;
-        case 3: LAUNCH_TOP(4); break;
-        case 4: LAUNCH_TOP(5); break;
-        case 5: LAUNCH_TOP(6); break;
-        default: return SCG_ELIMIT;
-    }
-#undef LAUNCH_TOP
-    if (rc) return rc;
-    SCG_LAUNCH_CHECK();
-    return 0;
+    DISPATCH_ORDER(ctx->order, rc = launch_top<N1>(ag, (int)n, grid, smem, st));
+    return rc;
 }
 
 // ---- the promote-and-fit kernel ---------------------------------------------------------------------------------
 #define MANAGE_NT 1024
-#define MANAGE_CACHE 8     // examples per thread kept in registers (rings up to 8192 examples never re-read memory)
 
 struct ManageArgs {
     scg_agent_t ag;
@@ -363,20 +349,10 @@ __device__ __forceinline__ bool manage_exchange(const ManageArgs &a, float *vals
     float *mb = reinterpret_cast<float *>(mine + XCHG_M_BUF) + (seq & 1u) * XCHG_M_WORDS;
     if (tid < nval) mb[tid] = vals[tid];
     __syncthreads();
-    if (tid < a.world && tid != a.rank) {
-        __threadfence_system();
-        st_release_sys(reinterpret_cast<uint32_t *>(a.peer[tid] + a.m_off + XCHG_M_FLAG) + a.rank, seq);
-        const uint32_t *lf = reinterpret_cast<const uint32_t *>(mine + XCHG_M_FLAG) + tid;
-        const long long t0 = clock64();
-        while ((int32_t)(ld_acquire_sys(lf) - seq) < 0) {
-            if (clock64() - t0 > a.timeout_cycles) {
-                *reinterpret_cast<volatile uint32_t *>(a.status) = 1u;
-                __threadfence_system();
-                *s_abort = 1;
-                break;
-            }
-        }
-    }
+    if (tid < a.world && tid != a.rank &&
+        !xchg_signal_wait(reinterpret_cast<uint32_t *>(a.peer[tid] + a.m_off + XCHG_M_FLAG) + a.rank,
+                          reinterpret_cast<const uint32_t *>(mine + XCHG_M_FLAG) + tid, seq, a.status, a.timeout_cycles))
+        *s_abort = 1;
     __syncthreads();
     if (tid < nval && !*s_abort) {
         float v = 0.f;
@@ -391,12 +367,12 @@ __device__ __forceinline__ bool manage_exchange(const ManageArgs &a, float *vals
 }
 
 __global__ void __launch_bounds__(MANAGE_NT) k_manage(const __grid_constant__ ManageArgs a) {
-    __shared__ float sm[33 * 8];
+    __shared__ float sm[33 * SCG_N_PSI];
     __shared__ float xv[XCHG_M_WORDS];           // values summed over ranks: a fit step's (6 sums, N) / the merge counts
     __shared__ int s_go, s_abort;
     const scg_agent_t &g = a.ag;
     scg_ctl_t *ctl = g.ctl;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x, lane = tid & 31;
     const int K = g.K;
     if (tid == 0) {
         const int gi = ctl->n_active;
@@ -416,49 +392,29 @@ __global__ void __launch_bounds__(MANAGE_NT) k_manage(const __grid_constant__ Ma
         const int N = (int)(have < (long long)g.example_capacity ? have : (long long)g.example_capacity);
         const float *X = g.ex_xy + (size_t)gi * g.example_capacity * 2;
         const uint8_t *Y = g.ex_label + (size_t)gi * g.example_capacity;
-        float cx[MANAGE_CACHE], cy[MANAGE_CACHE], cl[MANAGE_CACHE];
-#pragma unroll
-        for (int k = 0; k < MANAGE_CACHE; ++k) {
-            const int i = tid + k * MANAGE_NT;
-            const bool in = i < N;
-            cx[k] = in ? X[2 * i] : 0.f;
-            cy[k] = in ? X[2 * i + 1] : 0.f;
-            cl[k] = in ? (float)Y[i] : 0.f;
-        }
+        ClfCache cache;
+        clf_load(N, X, Y, cache);
         float th[SCG_N_PSI] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
         unsigned char *mine = a.world > 1 ? a.peer[a.rank] + a.m_off : nullptr;
         uint32_t seq = (a.world > 1) ? *reinterpret_cast<uint32_t *>(mine + XCHG_M_SEQ) : 0u;
         for (int it = 0; it < g.clf_steps && !s_abort; ++it) {
-            float gs[SCG_N_PSI] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+            float gs[SCG_N_PSI];
+            clf_grad_sum(N, X, Y, cache, th, gs, sm);
+            float ntot = (float)N;
+            if (a.world > 1) {     // the step of one fit on the union of all ranks' rings
+                if (tid == 0) {
 #pragma unroll
-            for (int k = 0; k < MANAGE_CACHE; ++k)
-                if (tid + k * MANAGE_NT < N) scg_clf_accum(cx[k], cy[k], cl[k], th, gs);
-            for (int i = tid + MANAGE_CACHE * MANAGE_NT; i < N; i += MANAGE_NT)
-                scg_clf_accum(X[2 * i], X[2 * i + 1], (float)Y[i], th, gs);
-#pragma unroll
-            for (int j = 0; j < SCG_N_PSI; ++j) {
-                const float v = scg_warp_sum(gs[j]);
-                if (lane == 0) sm[warp * 8 + j] = v;
-            }
-            __syncthreads();
-            if (warp == 0) {
-#pragma unroll
-                for (int j = 0; j < SCG_N_PSI; ++j) {
-                    float v = sm[lane * 8 + j];          // 32 warps
-                    v = scg_warp_sum(v);
-                    if (lane == 0) xv[j] = v;
+                    for (int j = 0; j < SCG_N_PSI; ++j) xv[j] = gs[j];
+                    xv[6] = ntot;
                 }
-                if (lane == 0) xv[6] = (float)N;
-            }
-            __syncthreads();
-            if (a.world > 1) manage_exchange(a, xv, 7, seq, &s_abort);
-            const float ntot = xv[6];
-            if (ntot > 0.f) {      // no examples anywhere: theta stays 0 (initiation set = everywhere), as in the oracle
+                __syncthreads();
+                manage_exchange(a, xv, 7, seq, &s_abort);
 #pragma unroll
-                for (int j = 0; j < SCG_N_PSI; ++j)
-                    th[j] = __fsub_rn(th[j], __fmul_rn(g.clf_lr, __fdiv_rn(xv[j], ntot)));
+                for (int j = 0; j < SCG_N_PSI; ++j) gs[j] = xv[j];
+                ntot = xv[6];
             }
-            __syncthreads();
+            // no examples anywhere: theta stays 0 (initiation set = everywhere), as in the oracle
+            if (ntot > 0.f) clf_step(th, g.clf_lr, gs, ntot);
         }
         if (!s_abort && tid < SCG_N_PSI) g.theta[gi * SCG_N_PSI + tid] = th[tid];
         __syncthreads();

@@ -12,13 +12,7 @@
 // three 16-byte loads), warp-uniform when the warp's envs execute the same option.  The contraction is
 // (B x F).(F x 5): far too skinny for tcgen05 tiles, so it stays on the FP32 pipe.
 // Roofline: FP32, 18 F flop per (env, option).
-#include <algorithm>
-
 #include "scg_common.cuh"
-
-static int grid_for(int B, int threads) {
-    return std::max(1, std::min((B + threads - 1) / threads, SCG_NUM_SMS * 16));
-}
 
 // ---- features (debug / parity operator; the hot path never writes phi to HBM) ------------------
 template <int N1>
@@ -153,53 +147,7 @@ __global__ void k_clf_decide(int B, const float *__restrict__ x, const float *__
     }
 }
 
-// mean_i (p_i - y_i) psi_i with a single CTA: per-thread partial sums, warp shuffles, smem.  Each thread keeps up to
-// CLF_CACHE of its examples in registers, so the gradient-descent loop of k_clf_fit touches global memory only for
-// the examples beyond 1024 * CLF_CACHE.
-#define CLF_CACHE 8
-struct ClfCache {
-    float x[CLF_CACHE], y[CLF_CACHE], lab[CLF_CACHE];
-};
-__device__ __forceinline__ void clf_load(int N, const float *__restrict__ X, const uint8_t *__restrict__ y, ClfCache &c) {
-#pragma unroll
-    for (int k = 0; k < CLF_CACHE; ++k) {
-        const int i = threadIdx.x + k * blockDim.x;
-        const bool in = i < N;
-        c.x[k] = in ? X[2 * i] : 0.f;
-        c.y[k] = in ? X[2 * i + 1] : 0.f;
-        c.lab[k] = in ? (float)y[i] : 0.f;
-    }
-}
-__device__ __forceinline__ void clf_grad_block(int N, const float *__restrict__ X, const uint8_t *__restrict__ y,
-                                               const ClfCache &c, const float th[SCG_N_PSI], float g_out[SCG_N_PSI],
-                                               float *sm) {
-    float g[SCG_N_PSI] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-    for (int k = 0; k < CLF_CACHE; ++k)
-        if ((int)(threadIdx.x + k * blockDim.x) < N) scg_clf_accum(c.x[k], c.y[k], c.lab[k], th, g);
-    for (int i = threadIdx.x + CLF_CACHE * blockDim.x; i < N; i += blockDim.x)
-        scg_clf_accum(X[2 * i], X[2 * i + 1], (float)y[i], th, g);
-    int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-#pragma unroll
-    for (int j = 0; j < SCG_N_PSI; ++j) {
-        float v = scg_warp_sum(g[j]);
-        if (lane == 0) sm[warp * SCG_N_PSI + j] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x < 32) {   // warp 0 folds the per-warp sums: lane (w % 32) holds warp w's value of component j
-#pragma unroll
-        for (int j = 0; j < SCG_N_PSI; ++j) {
-            float v = (lane < nw) ? sm[lane * SCG_N_PSI + j] : 0.f;
-            v = scg_warp_sum(v);
-            if (lane == 0) sm[32 * SCG_N_PSI + j] = v / (float)N;
-        }
-    }
-    __syncthreads();
-#pragma unroll
-    for (int j = 0; j < SCG_N_PSI; ++j) g_out[j] = sm[32 * SCG_N_PSI + j];
-    __syncthreads();
-}
-
+// mean_i (p_i - y_i) psi_i and the batch gradient-descent fit, each in a single CTA (clf_grad_sum, scg_common.cuh)
 __global__ void __launch_bounds__(1024) k_clf_grad(int N, const float *__restrict__ X, const uint8_t *__restrict__ y,
                                                    const float *__restrict__ theta_k, float *__restrict__ grad) {
     __shared__ float sm[33 * SCG_N_PSI];
@@ -208,8 +156,8 @@ __global__ void __launch_bounds__(1024) k_clf_grad(int N, const float *__restric
     for (int j = 0; j < SCG_N_PSI; ++j) th[j] = theta_k[j];
     ClfCache c;
     clf_load(N, X, y, c);
-    clf_grad_block(N, X, y, c, th, g, sm);
-    if (threadIdx.x < SCG_N_PSI) grad[threadIdx.x] = g[threadIdx.x];
+    clf_grad_sum(N, X, y, c, th, g, sm);
+    if (threadIdx.x < SCG_N_PSI) grad[threadIdx.x] = g[threadIdx.x] / (float)N;
 }
 
 __global__ void __launch_bounds__(1024) k_clf_fit(int N, const float *__restrict__ X, const uint8_t *__restrict__ y,
@@ -221,9 +169,8 @@ __global__ void __launch_bounds__(1024) k_clf_fit(int N, const float *__restrict
     ClfCache c;
     clf_load(N, X, y, c);
     for (int it = 0; it < steps; ++it) {
-        clf_grad_block(N, X, y, c, th, g, sm);
-#pragma unroll
-        for (int j = 0; j < SCG_N_PSI; ++j) th[j] = __fsub_rn(th[j], __fmul_rn(lr, g[j]));
+        clf_grad_sum(N, X, y, c, th, g, sm);
+        clf_step(th, lr, g, (float)N);
     }
     if (threadIdx.x < SCG_N_PSI) theta_k[threadIdx.x] = th[threadIdx.x];
 }
@@ -235,7 +182,7 @@ extern "C" int scg_features(int order, int B, const float *x, const float *y, co
     if (B < 0 || (B > 0 && (!x || !y || !vx || !vy || !phi))) return SCG_EINVAL;
     if (B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
-    DISPATCH_ORDER(order, k_features<N1><<<grid_for(B, 128), 128, 0, st>>>(B, x, y, vx, vy, phi));
+    DISPATCH_ORDER(order, k_features<N1><<<scg_grid(B, 128, 16), 128, 0, st>>>(B, x, y, vx, vy, phi));
     SCG_LAUNCH_CHECK();
     return 0;
 }
@@ -246,7 +193,7 @@ extern "C" int scg_pack_weights(int order, int K, const float *W, float *Wt, voi
     if (order < 1 || order > SCG_MAX_ORDER || K < 1 || K > SCG_MAX_OPTIONS) return SCG_ELIMIT;
     if (!W || !Wt) return SCG_EINVAL;
     int F = scg_pow4(order + 1);
-    DISPATCH_ORDER(order, k_pack_weights<N1><<<grid_for(K * WtLayout<N1>::P, 256), 256, 0, (cudaStream_t)stream>>>(K, W, Wt));
+    DISPATCH_ORDER(order, k_pack_weights<N1><<<scg_grid(K * WtLayout<N1>::P, 256, 16), 256, 0, (cudaStream_t)stream>>>(K, W, Wt));
     SCG_LAUNCH_CHECK();
     return 0;
 }
@@ -257,7 +204,7 @@ extern "C" int scg_q_eval(int order, int K, int B, const float *x, const float *
     if (B < 0 || (B > 0 && (!x || !y || !vx || !vy || !option || !Wt || !Q))) return SCG_EINVAL;
     if (B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
-    DISPATCH_ORDER(order, k_q_eval<N1><<<grid_for(B, 128), 128, 0, st>>>(K, B, x, y, vx, vy, option, Wt, Q));
+    DISPATCH_ORDER(order, k_q_eval<N1><<<scg_grid(B, 128, 16), 128, 0, st>>>(K, B, x, y, vx, vy, option, Wt, Q));
     SCG_LAUNCH_CHECK();
     return 0;
 }
@@ -266,7 +213,7 @@ extern "C" int scg_select(int B, const float *Q, float epsilon, uint64_t seed, u
                           uint32_t env_offset, int *action, void *stream) {
     if (B < 0 || (B > 0 && (!Q || !action))) return SCG_EINVAL;
     if (B == 0) return 0;
-    k_select<<<grid_for(B, 256), 256, 0, (cudaStream_t)stream>>>(B, Q, epsilon, seed, step, stream_id, env_offset, action);
+    k_select<<<scg_grid(B, 256, 16), 256, 0, (cudaStream_t)stream>>>(B, Q, epsilon, seed, step, stream_id, env_offset, action);
     SCG_LAUNCH_CHECK();
     return 0;
 }
@@ -281,7 +228,7 @@ extern "C" int scg_td_error(int order, int K, int B, const float *x, const float
         return SCG_EINVAL;
     if (B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
-    DISPATCH_ORDER(order, k_td<N1><<<grid_for(B, 128), 128, 0, st>>>(K, B, x, y, vx, vy, a, r, x2, y2, vx2, vy2, a2,
+    DISPATCH_ORDER(order, k_td<N1><<<scg_grid(B, 128, 16), 128, 0, st>>>(K, B, x, y, vx, vy, a, r, x2, y2, vx2, vy2, a2,
                                                                        done, option, Wt, gamma, delta));
     SCG_LAUNCH_CHECK();
     return 0;
@@ -291,7 +238,7 @@ extern "C" int scg_clf_eval(int B, const float *x, const float *y, const float *
     if (K < 1 || K > SCG_MAX_OPTIONS) return SCG_ELIMIT;
     if (B < 0 || (B > 0 && (!x || !y || !theta || !p))) return SCG_EINVAL;
     if (B == 0) return 0;
-    k_clf_eval<<<grid_for(B, 256), 256, 0, (cudaStream_t)stream>>>(B, x, y, theta, K, p);
+    k_clf_eval<<<scg_grid(B, 256, 16), 256, 0, (cudaStream_t)stream>>>(B, x, y, theta, K, p);
     SCG_LAUNCH_CHECK();
     return 0;
 }
@@ -300,7 +247,7 @@ extern "C" int scg_clf_decide(int B, const float *x, const float *y, const float
     if (K < 1 || K > SCG_MAX_OPTIONS) return SCG_ELIMIT;
     if (B < 0 || (B > 0 && (!x || !y || !theta || !inside))) return SCG_EINVAL;
     if (B == 0) return 0;
-    k_clf_decide<<<grid_for(B, 256), 256, 0, (cudaStream_t)stream>>>(B, x, y, theta, K, inside);
+    k_clf_decide<<<scg_grid(B, 256, 16), 256, 0, (cudaStream_t)stream>>>(B, x, y, theta, K, inside);
     SCG_LAUNCH_CHECK();
     return 0;
 }

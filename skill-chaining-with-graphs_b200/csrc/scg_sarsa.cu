@@ -624,39 +624,16 @@ __global__ void k_make_rec(int B, const float *__restrict__ x, const float *__re
     }
 }
 
-// W += (alpha * alpha_scale_f) * (dW * (steps / cnt_k));  refresh the packed copy;  dW <- 0
-// Slots k >= K_opt hold the top-level learner (oracle/option.py): step size alpha_top, mean over the window's events.
+// W += (alpha * alpha_scale_f) * (dW * (steps / cnt_k));  refresh the packed copy;  dW <- 0  (scg_apply_elem)
 template <int N1>
 __global__ void k_apply(int K, int K_opt, float *__restrict__ W, float *__restrict__ Wt, float *__restrict__ dW,
                         int *cnt, float alpha, float alpha_top, float steps, unsigned int *ticket) {
     constexpr int F = N1 * N1 * N1 * N1;
     int n = K * SCG_A * F;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        int f = i % F, ka = i / F, a = ka % SCG_A, k = ka / SCG_A;
-        int c = cnt[k];
-        float w = W[i];
-        if (c > 0) {
-            int d = f, ss = 0;
-#pragma unroll
-            for (int j = 0; j < 4; ++j) { int q = d % N1; ss += q * q; d /= N1; }
-            float as = (ss == 0) ? 1.0f : (float)(1.0 / sqrt((double)ss));
-            const bool top = k >= K_opt;
-            float scale = __fdiv_rn(top ? 1.0f : steps, (float)c);
-            w = __fadd_rn(w, __fmul_rn(__fmul_rn(top ? alpha_top : alpha, as), __fmul_rn(dW[i], scale)));
-            W[i] = w;
-        }
-        Wt[(size_t)k * WtLayout<N1>::SLOT_FLOATS + WtLayout<N1>::index(a, f)] = w;
-        dW[i] = 0.f;
-    }
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        scg_apply_elem<N1>(i, cnt[i / (SCG_A * F)], K_opt, alpha, alpha_top, steps, dW[i], W, Wt, dW);
     // the last block to finish zeroes cnt for the next window (every block has read it by then): no extra launch
-    __shared__ bool last;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        last = atomicInc(ticket, gridDim.x - 1) == gridDim.x - 1;
-    }
-    __syncthreads();
-    if (last && threadIdx.x < K) cnt[threadIdx.x] = 0;
+    if (scg_last_block(ticket) && threadIdx.x < K) cnt[threadIdx.x] = 0;
 }
 
 // ---- launch plumbing ----------------------------------------------------------------------------
@@ -693,7 +670,7 @@ static int launch_window_tm(scg_ctx *ctx, int B, int T, int k_used, const float4
     int rcc = scg_configure(cfgc, kern, NTT, smem, &per_sm);
     if (rcc) return rcc;
     if (per_sm < 1) return SCG_ELIMIT;
-    int grid = std::max(1, std::min(B, SCG_NUM_SMS * per_sm));
+    int grid = scg_grid(B, 1, per_sm);
     int rc = ensure_partials(ctx, grid);
     if (rc) return rc;
     kern<<<grid, NTT, smem, st>>>(B, k_used, T, rec, trace, ctx->d_partial, gl, dW, ctx->K);
@@ -800,8 +777,7 @@ extern "C" int scg_sarsa_update(scg_ctx_t *ctx, int B, const float *x, const flo
         SCG_CUDA_OK(cudaMalloc((void **)&ctx->d_rec, (size_t)B * SCG_WREC_FLOATS * sizeof(float)));
         ctx->rec_capacity = B;
     }
-    int grid = std::max(1, std::min((B + 255) / 256, SCG_NUM_SMS * 8));
-    k_make_rec<<<grid, 256, 0, st>>>(B, x, y, vx, vy, a, option, delta, done, mask, ctx->K,
+    k_make_rec<<<scg_grid(B, 256, 8), 256, 0, st>>>(B, x, y, vx, vy, a, option, delta, done, mask, ctx->K,
                                      reinterpret_cast<float4 *>(ctx->d_rec), cnt);
     SCG_LAUNCH_CHECK();
     // the dense update is the forward-view sweep over a window of one step
@@ -822,7 +798,7 @@ extern "C" int scg_apply_top(int order, int K, int K_opt, float *W, float *Wt, f
     cudaStream_t st = (cudaStream_t)stream;
     float steps = (float)std::max(window_steps, 1);
     int F = scg_pow4(order + 1);
-    int grid = std::max(1, std::min((K * SCG_A * F + 255) / 256, SCG_NUM_SMS * 8));
+    int grid = scg_grid(K * SCG_A * F, 256, 8);
     // one "blocks done" counter per (device, stream): launches on one stream are ordered, so the counter (which atomicInc
     // wraps back to 0) is reusable launch after launch; applies running concurrently on other streams have their own
     struct Slot { int dev; cudaStream_t st; unsigned int *ticket; };

@@ -236,7 +236,7 @@ __global__ void __launch_bounds__(256) k_step(const unsigned char *__restrict__ 
                                               float *vy2, float *__restrict__ reward, int *__restrict__ flags) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) unsigned long long bar;
-    stage_blob(smem, gblob, blob_bytes, &bar);
+    stage3(smem, gblob, blob_bytes, nullptr, nullptr, 0, nullptr, nullptr, 0, &bar);
     const StepMap m = make_step_map(smem);
     for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
         float px = x[b], py = y[b], pvx = vx[b], pvy = vy[b];
@@ -264,12 +264,6 @@ __global__ void k_reset(const unsigned char *__restrict__ gblob, int B, const ui
     }
 }
 
-static int step_grid(int B, int threads) {
-    int blocks = (B + threads - 1) / threads;
-    int cap = SCG_NUM_SMS * 8;
-    return std::max(1, std::min(blocks, cap));
-}
-
 int scg_launch_step(const scg_map_t *map, int B, const float *x, const float *y, const float *vx, const float *vy,
                     const int *action, float *x2, float *y2, float *vx2, float *vy2, float *reward, int *flags,
                     int cull, cudaStream_t st) {
@@ -280,7 +274,7 @@ int scg_launch_step(const scg_map_t *map, int B, const float *x, const float *y,
     int occ = 0, rcc;
     if ((rcc = scg_configure(cfg_t, k_step<true>, threads, (size_t)smem, &occ))) return rcc;
     if ((rcc = scg_configure(cfg_f, k_step<false>, threads, (size_t)smem, &occ))) return rcc;
-    int grid = step_grid(B, threads);
+    int grid = scg_grid(B, threads, 8);
     if (cull)
         k_step<true><<<grid, threads, smem, st>>>(map->d_blob, smem, B, x, y, vx, vy, action, x2, y2, vx2, vy2, reward, flags);
     else
@@ -302,7 +296,7 @@ extern "C" int scg_reset(const scg_map_t *map, int B, const uint8_t *mask, float
                          uint64_t seed, uint32_t step, uint32_t env_offset, void *stream) {
     if (!map || B < 0 || (B > 0 && (!x || !y || !vx || !vy))) return SCG_EINVAL;
     if (B == 0) return 0;
-    k_reset<<<step_grid(B, 256), 256, 0, (cudaStream_t)stream>>>(map->d_blob, B, mask, x, y, vx, vy, seed, step, env_offset);
+    k_reset<<<scg_grid(B, 256, 8), 256, 0, (cudaStream_t)stream>>>(map->d_blob, B, mask, x, y, vx, vy, seed, step, env_offset);
     SCG_LAUNCH_CHECK();
     return 0;
 }

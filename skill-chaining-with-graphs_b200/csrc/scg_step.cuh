@@ -8,25 +8,36 @@
 #include "scg_common.cuh"
 
 // ---------------------------------------------------------------------------------------------
-// device: TMA bulk staging of the map blob
+// device: TMA bulk staging of the map blob (and of the agent step's weight slots)
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void stage_blob(unsigned char *smem, const unsigned char *gblob, int bytes,
-                                           unsigned long long *bar) {
-    uint32_t bar_a = smem_u32(bar);
+// bulk-TMA staging of up to three global blocks into shared memory behind one mbarrier (blocks 1 and 2 may be empty)
+__device__ __forceinline__ void stage3(unsigned char *dst0, const void *src0, int bytes0, unsigned char *dst1,
+                                       const void *src1, int bytes1, unsigned char *dst2, const void *src2, int bytes2,
+                                       unsigned long long *bar) {
+    uint32_t bar_a = scg_smem_u32(bar);
     if (threadIdx.x == 0) {
         asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar_a));
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
     if (threadIdx.x == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a), "r"(bytes) : "memory");
-        asm volatile(
-            "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                smem_u32(smem)),
-            "l"(gblob), "r"(bytes), "r"(bar_a)
-            : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_a),
+                     "r"(bytes0 + bytes1 + bytes2)
+                     : "memory");
+        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                         scg_smem_u32(dst0)),
+                     "l"(src0), "r"(bytes0), "r"(bar_a)
+                     : "memory");
+        if (bytes1 > 0)
+            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                             scg_smem_u32(dst1)),
+                         "l"(src1), "r"(bytes1), "r"(bar_a)
+                         : "memory");
+        if (bytes2 > 0)
+            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                             scg_smem_u32(dst2)),
+                         "l"(src2), "r"(bytes2), "r"(bar_a)
+                         : "memory");
     }
     uint32_t ok = 0;
     while (!ok) {

@@ -63,23 +63,13 @@ __global__ void __launch_bounds__(XCHG_SLICE, 8) k_sync(const __grid_constant__ 
     }
     __syncthreads();
     // 2. signal every peer, 3. wait for every peer (one thread per peer)
-    if (i < a.world && i != a.rank) {
-        __threadfence_system();
-        uint32_t *pf = reinterpret_cast<uint32_t *>(a.peer[i]) + (size_t)a.rank * a.slices + c;
-        st_release_sys(pf, a.seq);
-        const uint32_t *lf = reinterpret_cast<const uint32_t *>(mine) + (size_t)i * a.slices + c;
-        const long long t0 = clock64();
-        while ((int32_t)(ld_acquire_sys(lf) - a.seq) < 0) {
-            if (clock64() - t0 > a.timeout_cycles) {  // the peer never came: fatal for this exchange (see the header)
-                *reinterpret_cast<volatile uint32_t *>(a.status) = 1u;
-                __threadfence_system();
-                s_timeout = 1;
-                break;
-            }
-        }
-    }
+    if (i < a.world && i != a.rank &&
+        !xchg_signal_wait(reinterpret_cast<uint32_t *>(a.peer[i]) + (size_t)a.rank * a.slices + c,
+                          reinterpret_cast<const uint32_t *>(mine) + (size_t)i * a.slices + c, a.seq, a.status,
+                          a.timeout_cycles))
+        s_timeout = 1;                                // the peer never came: fatal for this exchange (see the header)
     __syncthreads();
-    if (s_timeout) return;                            // no apply, dW of this slice kept
+    if (s_timeout) return;                            // no apply, dW of this slice kept (the whole CTA returns)
     // 4. sum in rank order, apply
     // every peer's copy of this slice: the NVLink loads of (up to) eight peers are issued before the first one is
     // consumed - one round trip per sync on an 8-GPU box, not one per peer - then added in rank order.  The 32-word
@@ -119,32 +109,10 @@ __global__ void __launch_bounds__(XCHG_SLICE, 8) k_sync(const __grid_constant__ 
         if (c == 0 && a.nsucc_global) a.nsucc_global[i] = (int)(succ > 0x7fffffffll ? 0x7fffffffll : succ);
     }
     __syncthreads();
-    if (j < a.n) {   // same arithmetic as k_apply (scg_sarsa.cu)
-        const int f = j % F, ka = j / F, act = ka % SCG_A, k = ka / SCG_A;
-        const int cn = s_cnt[k];
-        float w = a.W[j];
-        if (cn > 0) {
-            int d = f, ss = 0;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) { int dg = d % N1; ss += dg * dg; d /= N1; }
-            const float as = (ss == 0) ? 1.0f : (float)(1.0 / sqrt((double)ss));
-            const bool top = k >= a.K_opt;       // top-level learner slots: alpha_top, mean over the window's events
-            const float scale = __fdiv_rn(top ? 1.0f : a.steps, (float)cn);
-            w = __fadd_rn(w, __fmul_rn(__fmul_rn(top ? a.alpha_top : a.alpha, as), __fmul_rn(v, scale)));
-            a.W[j] = w;
-        }
-        a.Wt[(size_t)k * WtLayout<N1>::SLOT_FLOATS + WtLayout<N1>::index(act, f)] = w;
-        a.dW[j] = 0.f;
-    }
+    if (j < a.n)
+        scg_apply_elem<N1>(j, s_cnt[j / (SCG_A * F)], a.K_opt, a.alpha, a.alpha_top, a.steps, v, a.W, a.Wt, a.dW);
     // the last CTA to finish zeroes cnt for the next window (every CTA read it when it published)
-    if (i == 0) {
-        __threadfence();
-        const unsigned int t = atomicAdd(a.ticket, 1u);
-        if (t == gridDim.x - 1) {
-            for (int k = 0; k < a.K; ++k) a.cnt[k] = 0;
-            *a.ticket = 0u;
-        }
-    }
+    if (scg_last_block(a.ticket) && i < a.K) a.cnt[i] = 0;
 }
 
 // ---- host side ------------------------------------------------------------------------------------------

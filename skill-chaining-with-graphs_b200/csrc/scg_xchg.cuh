@@ -49,4 +49,22 @@ __device__ __forceinline__ float ld_sys_f32(const float *p) {
     return v;
 }
 
+// One peer's half of a flag round: publish round `seq` in the peer's flag for us (after this thread's earlier writes,
+// system scope), then wait for the peer to raise our flag for it to `seq`.  A peer that does not come within
+// timeout_cycles is fatal for the exchange: raise the sticky host-mapped status and return false.
+__device__ __forceinline__ bool xchg_signal_wait(uint32_t *peer_flag, const uint32_t *own_flag, uint32_t seq, uint32_t *status,
+                                                 long long timeout_cycles) {
+    __threadfence_system();
+    st_release_sys(peer_flag, seq);
+    const long long t0 = clock64();
+    while ((int32_t)(ld_acquire_sys(own_flag) - seq) < 0) {
+        if (clock64() - t0 > timeout_cycles) {
+            *reinterpret_cast<volatile uint32_t *>(status) = 1u;
+            __threadfence_system();
+            return false;
+        }
+    }
+    return true;
+}
+
 #endif

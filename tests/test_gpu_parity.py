@@ -755,6 +755,10 @@ def test_manage_on_device_matches_oracle(scg, torch, graph, merge_overlap):
             promoted.append(w)
             g = oag.n_active - 1
             assert_close(gag.options.theta[g].cpu().numpy(), oag.options.theta[g], what=f"theta of option {g}")
+            # the controller's fit is the stand-alone fit: the same ring from theta = 0 gives the same bits
+            X, y = gag.examples(g)
+            refit = scg.OptionSet(1, 1, 1).fit_initiation(0, X, y, steps=kw["clf_steps"], lr=kw["clf_lr"])
+            assert torch.equal(refit, gag.options.theta[g]), f"theta of option {g}: {refit} refit, {gag.options.theta[g]} device"
         c = gag.controller_state()
         assert c["n_active"] == oag.n_active and c["active_mask"] == int(sum(1 << k for k in range(K) if oag.active[k]))
         assert c["parents"] == [int(v) for v in oag.parents]
