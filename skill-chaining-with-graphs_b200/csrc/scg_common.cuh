@@ -582,15 +582,15 @@ __device__ __forceinline__ void scg_apply_elem(int i, int c, int K_opt, float al
     dW[i] = 0.f;
 }
 
-// True on every thread of the last CTA of the grid to get here; every thread of the CTA must call it.  The CTA's
-// earlier writes are visible grid-wide before the ticket moves.  atomicInc wraps the ticket back to 0 on the last CTA,
-// so the same ticket serves the next launch on the same stream.
-__device__ __forceinline__ bool scg_last_block(unsigned int *ticket) {
+// True on every thread of the last of the n CTAs sharing `ticket` to get here; every thread of the CTA must call it.
+// The CTA's earlier writes are visible grid-wide before the ticket moves.  atomicInc wraps the ticket back to 0 on the
+// last CTA, so the same ticket serves the next launch on the same stream.
+__device__ __forceinline__ bool scg_last_block(unsigned int *ticket, unsigned int n) {
     __shared__ bool last;
     __syncthreads();
     if (threadIdx.x == 0) {
         __threadfence();
-        last = atomicInc(ticket, gridDim.x - 1) == gridDim.x - 1;
+        last = atomicInc(ticket, n - 1) == n - 1;
     }
     __syncthreads();
     return last;

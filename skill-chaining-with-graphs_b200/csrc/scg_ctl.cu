@@ -173,7 +173,7 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
         __syncthreads();
     }
     // the last CTA to finish advances the counts (every CTA has read them by then)
-    if (scg_last_block(scratch + RING_DONE) && tid < K) ex_count[tid] += (long long)tot_s[tid];
+    if (scg_last_block(scratch + RING_DONE, gridDim.x) && tid < K) ex_count[tid] += (long long)tot_s[tid];
 }
 
 extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {

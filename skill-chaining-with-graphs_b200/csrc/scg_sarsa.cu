@@ -75,72 +75,114 @@ struct WinCtlList {
     int nseg, pad;
 };
 
-template <int N1, int VEC, int NT, int CH, bool MULTI, int MINB, bool CTRL, bool LISTP, bool L2PF, bool SPLITP>
-__global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, int K, int T, const float4 *__restrict__ rec, float *trace,
-                                               float *__restrict__ partial, float gl, float *dW, int K_all) {
-    using V = typename VecT<VEC>::type;
-    constexpr bool LIST = LISTP && !MULTI;
-    using WinCtl = std::conditional_t<LIST, WinCtlList, WinCtlT<MULTI ? SCG_WIN_MAX : SCG_WIN_TB>>;
-    constexpr int F = N1 * N1 * N1 * N1;
-    constexpr int AF = SCG_A * F;
-    constexpr int NCHR = F / VEC;          // chunks per action row
-    constexpr int NN = N1 * N1;
-    constexpr int TABN = SCG_WIN_TB * 2 * NN;             // entries of one table buffer
+// One sweep configuration per order: only what is chosen.  NT work threads; CTRL: one extra warp only runs the per-env
+// scan (worth it when a CTA has many work warps: orders 4 and 5); LIST: step lists instead of bit-mask loops; L2PF: the
+// next trace is prefetched into L2 instead of registers; SPLIT: two warps per env, one scans, one builds the tables;
+// MINB: minimum CTAs per SM (the register budget).  Step lists and split warps are single-block mechanisms: the
+// multi-block sweep (T > 8) runs without them.
+struct WinCfgBase {
+    static constexpr bool CTRL = false, LIST = true, L2PF = false, SPLIT = false;
+    static constexpr int MINB = 1;
+};
+template <int N1_> struct WinCfg;
+template <> struct WinCfg<2> : WinCfgBase { static constexpr int N1 = 2, NT = 32; };
+template <> struct WinCfg<3> : WinCfgBase { static constexpr int N1 = 3, NT = 96; };
+template <> struct WinCfg<5> : WinCfgBase { static constexpr int N1 = 5, NT = 640; };
+// Order 3: two warps per env.  With the next trace prefetched into L2 instead of registers the sweep needs 140 registers
+// (7 CTAs per SM) and loses nothing when squeezed to 128 (8 CTAs, while 8 accumulators fit: WinCfgO3Split).  With more
+// option slots in use (larger accumulators) it runs without the split warps or the squeeze (WinCfg<4>).
+struct WinCfgO3Split : WinCfgBase {
+    static constexpr int N1 = 4, NT = 64, MINB = 8;
+    static constexpr bool L2PF = true, SPLIT = true;
+};
+template <> struct WinCfg<4> : WinCfgBase {
+    static constexpr int N1 = 4, NT = 64;
+    static constexpr bool L2PF = true;
+};
+// Order 5: one CTA per SM, 11 work warps + a scan warp; next trace prefetched in registers (L2 prefetch: 1.98 vs 1.75 ms -
+// one CTA cannot cover the L2 latency); bit-mask loop (step lists: 1.74 vs 1.70 ms).
+template <> struct WinCfg<6> : WinCfgBase {
+    static constexpr int N1 = 6, NT = 352;
+    static constexpr bool CTRL = true, LIST = false;
+};
+
+// What follows from a configuration: the feature chunking and the sweep's shared memory, in bytes from the start of
+// the dynamic block: the accumulator [k_used][A*F] (rounded up to 16 bytes), the two table buffers, the two control
+// blocks and glpow[36] (gl^n).  The kernel carves its pointers from it and the host sizes the launch with it.
+template <class Cfg, bool MULTI>
+struct WinLayout {
+    static constexpr int N1 = Cfg::N1, NN = N1 * N1, F = NN * NN, AF = SCG_A * F;
+    static constexpr int VEC = N1 % 2 == 0 ? 4 : 1;       // floats per chunk
+    static constexpr bool LIST = Cfg::LIST && !MULTI, SPLIT = Cfg::SPLIT && !MULTI;
+    using Ctl = std::conditional_t<LIST, WinCtlList, WinCtlT<MULTI ? SCG_WIN_MAX : SCG_WIN_TB>>;
     // Storage of one step's tables, in float2: P01 (NN entries) then P23 in two halves of 16-byte groups (entries
     // (4g, 4g+1) of every group g of four, then entries (4g+2, 4g+3)).  DUP9 (order 5): the 9 groups of a half cannot
     // sit in 8 distinct bank quads, and a quarter-warp reads 8 consecutive groups (mod 9) with one 16-byte load: 7 of 9
     // quarters hit groups 0 and 8 together - two wavefronts (6.4 per load measured).  So a half is 16 slots: groups 0..7,
     // then eight copies of group 8, copy m in the bank quad of group m; the thread that needs group 8 reads the copy in
     // the quad its quarter leaves free.
-    constexpr bool DUP9 = VEC == 4 && NN / 4 == 9;
-    constexpr int HS = DUP9 ? 32 : NN / 2;                // float2 per half of P23
-    constexpr int TSZ = VEC == 4 ? NN + 2 * HS : 2 * NN;  // float2 per step
-    constexpr int TABS = SCG_WIN_TB * TSZ;                // float2 per table buffer
+    static constexpr bool DUP9 = VEC == 4 && NN / 4 == 9;
+    static constexpr int HS = DUP9 ? 32 : NN / 2;                 // float2 per half of P23
+    static constexpr int TSZ = VEC == 4 ? NN + 2 * HS : 2 * NN;   // float2 per step
+    static constexpr int TABS = SCG_WIN_TB * TSZ;                 // float2 per table buffer
+    static constexpr int N_TAB = 2 * TABS, N_CTL = 2, N_GLPOW = 36;   // float2, Ctl, float
+    __host__ __device__ static constexpr size_t acc_floats(int k_used) { return ((size_t)k_used * AF + 3) & ~(size_t)3; }
+    __host__ __device__ static constexpr size_t bytes(int k_used) {
+        return acc_floats(k_used) * sizeof(float) + N_TAB * sizeof(float2) + N_CTL * sizeof(Ctl) + N_GLPOW * sizeof(float);
+    }
+};
+
+template <class Cfg, bool MULTI>
+__global__ void __launch_bounds__(Cfg::NT + (Cfg::CTRL ? 32 : 0), Cfg::MINB)
+k_window(int B, int K, int T, const float4 *__restrict__ rec, float *trace, float *__restrict__ partial, float gl,
+         float *dW, int K_all) {
+    using L = WinLayout<Cfg, MULTI>;
+    constexpr int N1 = Cfg::N1, NT = Cfg::NT, VEC = L::VEC, NN = L::NN, F = L::F, AF = L::AF;
+    constexpr int HS = L::HS, TSZ = L::TSZ, TABS = L::TABS;
+    constexpr bool CTRL = Cfg::CTRL, L2PF = Cfg::L2PF, LIST = L::LIST, SPLIT = L::SPLIT, DUP9 = L::DUP9;
+    using V = typename VecT<VEC>::type;
+    using WinCtl = typename L::Ctl;
+    constexpr int NCHR = F / VEC;          // chunks per action row
+    constexpr int TABN = SCG_WIN_TB * 2 * NN;             // entries of one table buffer
     // SPLIT (two warps per env): warp 0 runs the per-env scan, warp 1 builds all the table entries - the two jobs take
     // about as long, so neither warp waits for the other at the per-item barrier.  The 16 state pairs the entries need
     // (8 steps x positions / velocities) are loaded by 16 lanes, one each, and handed round with shuffles.
-    constexpr bool SPLIT = SPLITP && !CTRL && !MULTI && NT == 64 && 2 * NN == 32;
+    static_assert(!Cfg::SPLIT || (!CTRL && NT == 64 && 2 * NN == 32), "split warps: one scan warp and one builder warp");
     constexpr int BT = SPLIT ? 32 : NT;                   // threads that build table entries
     constexpr int EPT = (TABN + BT - 1) / BT;             // table entries built per builder thread
     constexpr int TSTRIDE = TSZ * (int)sizeof(float2);    // bytes between the tables of consecutive steps
-    static_assert(F % VEC == 0 && NT * CH >= NCHR && NT >= 32 && SCG_WIN_MAX <= 32, "layout");
+    static_assert(F % VEC == 0 && NT >= NCHR && NT >= 32 && SCG_WIN_MAX <= 32, "layout");
     static_assert(VEC == 1 || NN % VEC == 0, "a chunk shares its (c0, c1) digits");
     extern __shared__ __align__(128) unsigned char smem_raw[];
     float *acc = reinterpret_cast<float *>(smem_raw);                                      // [K][AF]
-    float2 *tab = reinterpret_cast<float2 *>(acc + (((size_t)K * AF + 3) & ~(size_t)3));   // [2][TABS]
-    WinCtl *ctl = reinterpret_cast<WinCtl *>(tab + 2 * TABS);                              // [2]
-    float *glpow = reinterpret_cast<float *>(ctl + 2);                                     // [36]: gl^n
+    float2 *tab = reinterpret_cast<float2 *>(acc + L::acc_floats(K));                      // [2][TABS]
+    WinCtl *ctl = reinterpret_cast<WinCtl *>(tab + L::N_TAB);                              // [2]
+    float *glpow = reinterpret_cast<float *>(ctl + L::N_CTL);                              // [N_GLPOW]: gl^n
 
     const int tid = threadIdx.x;
-    // CTRL: one extra warp (threads NT .. NT+31) only runs the per-env scan, so that no work warp is slower than the
-    // others at the per-env barrier (worth it when a CTA has many work warps: orders 4 and 5)
+    // CTRL: the scan warp is threads NT .. NT+31, so that no work warp is slower than the others at the per-env barrier
     constexpr int NTT = NT + (CTRL ? 32 : 0);
     const bool scan_warp = CTRL ? (tid >= NT) : (tid < 32);
     const bool worker = tid < NT;
     const bool builder = SPLIT ? tid >= 32 : worker;
     const int bt = SPLIT ? tid - 32 : tid;                // builder index (SPLIT: lane = half * NN + ij)
-    // thread t owns chunks t, t + NT, ... of every action row (each a coalesced access across the CTA)
-    bool own[CH];
-#pragma unroll
-    for (int j = 0; j < CH; ++j) own[j] = tid + j * NT < NCHR;
+    // thread t owns chunk t of every action row (a coalesced access across the CTA)
+    const bool own = tid < NCHR;
     const int NBLK = MULTI ? (T + SCG_WIN_TB - 1) / SCG_WIN_TB : 1;
     // per-thread constants: table offsets (bytes) of the owned features' (c0, c1) and (c2, c3) entries ...
-    int off01[CH], off23[CH];
-#pragma unroll
-    for (int j = 0; j < CH; ++j) {
-        const int f0 = (own[j] ? tid + j * NT : 0) * VEC;
-        off01[j] = (f0 / NN) * (int)sizeof(float2);
-        // P23: scalar form one float2 per (c2, c3); vector form: the 16-byte slot of the chunk's group in the first half
-        // (the second half is HS float2 further on); DUP9: group 8 is read from the copy in the bank quad that the
-        // other seven lanes of this quarter-warp leave free
-        if constexpr (VEC == 4) {
-            const int c = own[j] ? tid + j * NT : 0;
-            int slot = c % (NN / 4);
-            if (DUP9 && slot == 8) slot = 8 + (8 * (c / 8) + 8) % 9;
-            off23[j] = NN * (int)sizeof(float2) + slot * 16;
-        } else {
-            off23[j] = (NN + f0 % NN) * (int)sizeof(float2);
-        }
+    const int f0 = (own ? tid : 0) * VEC;
+    const int off01 = (f0 / NN) * (int)sizeof(float2);
+    // P23: scalar form one float2 per (c2, c3); vector form: the 16-byte slot of the chunk's group in the first half
+    // (the second half is HS float2 further on); DUP9: group 8 is read from the copy in the bank quad that the other
+    // seven lanes of this quarter-warp leave free
+    int off23;
+    if constexpr (VEC == 4) {
+        const int c = own ? tid : 0;
+        int slot = c % (NN / 4);
+        if (DUP9 && slot == 8) slot = 8 + (8 * (c / 8) + 8) % 9;
+        off23 = NN * (int)sizeof(float2) + slot * 16;
+    } else {
+        off23 = (NN + f0 % NN) * (int)sizeof(float2);
     }
     // ... and, for the EPT table entries this thread builds: step within the block, which state pair, digits,
     // the affine map of the raw state pair to [0, 1] (positions: identity; velocities: (v + 2) / 4) folded into the
@@ -174,7 +216,7 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
     for (int i = tid; i < K * AF; i += NTT) acc[i] = 0.f;
     if (tid == 0) {
         float p = 1.f;
-        for (int n = 0; n < 36; ++n) { glpow[n] = p; p *= gl; }
+        for (int n = 0; n < L::N_GLPOW; ++n) { glpow[n] = p; p *= gl; }
     }
 
     const int stride = gridDim.x;
@@ -190,16 +232,13 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
     // prefetch registers
     float2 r_sv[SPLIT ? 1 : EPT];                        // state pair of the steps this thread builds entries for
     float2 r_dm = make_float2(0.f, 0.f);                 // (delta, meta) of step tid (first block of an env only)
-    V e[CH][SCG_A], d[CH][SCG_A];
-    V e_nx[L2PF ? 1 : CH][L2PF ? 1 : SCG_A];            // register prefetch of the next env's trace (!L2PF)
+    V e[SCG_A], d[SCG_A];
+    V e_nx[L2PF ? 1 : SCG_A];                            // register prefetch of the next env's trace (!L2PF)
     uint32_t o_cur = 0;
 #pragma unroll
-    for (int j = 0; j < CH; ++j) {
-#pragma unroll
-        for (int r = 0; r < SCG_A; ++r) {
-            if constexpr (VEC == 4) { e[j][r] = vzero4(); d[j][r] = vzero4(); }
-            else { e[j][r] = 0.f; d[j][r] = 0.f; }
-        }
+    for (int r = 0; r < SCG_A; ++r) {
+        if constexpr (VEC == 4) { e[r] = vzero4(); d[r] = vzero4(); }
+        else { e[r] = 0.f; d[r] = 0.f; }
     }
 
     auto load_rec = [&](WinItem it) {                    // records of a work item -> registers
@@ -235,14 +274,11 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
     };
     auto load_trace = [&](int b) {
         const V *tp = reinterpret_cast<const V *>(trace + (size_t)b * AF);
+        if (own) {
 #pragma unroll
-        for (int j = 0; j < CH; ++j) {
-            if (own[j]) {
-#pragma unroll
-                for (int r = 0; r < SCG_A; ++r) {
-                    if constexpr (L2PF) e[j][r] = tp[r * NCHR + tid + j * NT];
-                    else e_nx[j][r] = tp[r * NCHR + tid + j * NT];
-                }
+            for (int r = 0; r < SCG_A; ++r) {
+                if constexpr (L2PF) e[r] = tp[r * NCHR + tid];
+                else e_nx[r] = tp[r * NCHR + tid];
             }
         }
     };
@@ -357,18 +393,15 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
             // contribution goes straight to dW with atomics (rare and transient; ids beyond K_all are ignored)
             if (o_cur < (uint32_t)K_all) {
                 float *gp = dW + (size_t)o_cur * AF;
+                if (own) {
 #pragma unroll
-                for (int j = 0; j < CH; ++j) {
-                    if (own[j]) {
-#pragma unroll
-                        for (int r = 0; r < SCG_A; ++r) {
-                            float *q = gp + (size_t)(r * NCHR + tid + j * NT) * VEC;
-                            if constexpr (VEC == 4) {
-                                atomicAdd(q, d[j][r].x); atomicAdd(q + 1, d[j][r].y);
-                                atomicAdd(q + 2, d[j][r].z); atomicAdd(q + 3, d[j][r].w);
-                            } else {
-                                atomicAdd(q, d[j][r]);
-                            }
+                    for (int r = 0; r < SCG_A; ++r) {
+                        float *q = gp + (size_t)(r * NCHR + tid) * VEC;
+                        if constexpr (VEC == 4) {
+                            atomicAdd(q, d[r].x); atomicAdd(q + 1, d[r].y);
+                            atomicAdd(q + 2, d[r].z); atomicAdd(q + 3, d[r].w);
+                        } else {
+                            atomicAdd(q, d[r]);
                         }
                     }
                 }
@@ -376,17 +409,13 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
             return;
         }
         V *ap = reinterpret_cast<V *>(acc + (size_t)o_cur * AF);
+        if (own) {
 #pragma unroll
-        for (int j = 0; j < CH; ++j) {
-            if (own[j]) {
-#pragma unroll
-                for (int r = 0; r < SCG_A; ++r) {
-                    V cur = ap[r * NCHR + tid + j * NT];
-                    if constexpr (VEC == 4)
-                        cur = make_float4(cur.x + d[j][r].x, cur.y + d[j][r].y, cur.z + d[j][r].z, cur.w + d[j][r].w);
-                    else cur = cur + d[j][r];
-                    ap[r * NCHR + tid + j * NT] = cur;
-                }
+            for (int r = 0; r < SCG_A; ++r) {
+                V cur = ap[r * NCHR + tid];
+                if constexpr (VEC == 4) cur = make_float4(cur.x + d[r].x, cur.y + d[r].y, cur.z + d[r].z, cur.w + d[r].w);
+                else cur = cur + d[r];
+                ap[r * NCHR + tid] = cur;
             }
         }
     };
@@ -411,10 +440,7 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
             if (nx2.blk == 0 && nx2.b < B) prefetch_trace(nx2.b);
         } else if (cur.blk == 0) {
 #pragma unroll
-            for (int j = 0; j < CH; ++j) {
-#pragma unroll
-                for (int r = 0; r < SCG_A; ++r) e[j][r] = e_nx[j][r];
-            }
+            for (int r = 0; r < SCG_A; ++r) e[r] = e_nx[r];
         }
         // next item's tables (into the other buffer), then the loads for the items after it
         if (nxt.b < B) build(nxt, par ^ 1, nxt.blk == 0 ? epar ^ 1 : epar);
@@ -431,44 +457,35 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
             const float carry = cb.carry, scale = cb.scale;
             o_cur = cb.seg_o[0];
 #pragma unroll
-            for (int j = 0; j < CH; ++j) {
-#pragma unroll
-                for (int r = 0; r < SCG_A; ++r) {
-                    d[j][r] = vscale(e[j][r], carry);    // carry-in: gl G_0 e_start
-                    e[j][r] = vscale(e[j][r], scale);
-                }
+            for (int r = 0; r < SCG_A; ++r) {
+                d[r] = vscale(e[r], carry);              // carry-in: gl G_0 e_start
+                e[r] = vscale(e[r], scale);
             }
         }
         const int nseg = cb.nseg;
         auto change_option = [&](uint32_t so) {          // the env changed option inside the window (after a termination)
             flush_d();
 #pragma unroll
-            for (int j = 0; j < CH; ++j) {
-#pragma unroll
-                for (int r = 0; r < SCG_A; ++r) {
-                    if constexpr (VEC == 4) d[j][r] = vzero4(); else d[j][r] = 0.f;
-                }
+            for (int r = 0; r < SCG_A; ++r) {
+                if constexpr (VEC == 4) d[r] = vzero4(); else d[r] = 0.f;
             }
             o_cur = so;
         };
-        // one step's contribution to row r of the owned chunks; tb: the step's pair tables
-        auto step_row = [&](const char *tb, float G, float c, V (&dd)[CH][SCG_A], V (&ee)[CH][SCG_A], int r) {
-#pragma unroll
-            for (int j = 0; j < CH; ++j) {               // independent chunks: their loads and FMAs interleave
-                const float2 p = *reinterpret_cast<const float2 *>(tb + off01[j]);
-                V ph;
-                if constexpr (VEC == 4) {
-                    const float4 q01 = *reinterpret_cast<const float4 *>(tb + off23[j]);
-                    const float4 q23 = *reinterpret_cast<const float4 *>(tb + off23[j] + HS * (int)sizeof(float2));
-                    ph = make_float4(fmaf(p.x, q01.x, -p.y * q01.y), fmaf(p.x, q01.z, -p.y * q01.w),
-                                     fmaf(p.x, q23.x, -p.y * q23.y), fmaf(p.x, q23.z, -p.y * q23.w));
-                } else {
-                    const float2 q = *reinterpret_cast<const float2 *>(tb + off23[j]);
-                    ph = fmaf(p.x, q.x, -p.y * q.y);
-                }
-                dd[j][r] = vfma(G, ph, dd[j][r]);
-                ee[j][r] = vfma(c, ph, ee[j][r]);
+        // one step's contribution to row r of the owned chunk; tb: the step's pair tables
+        auto step_row = [&](const char *tb, float G, float c, int r) {
+            const float2 p = *reinterpret_cast<const float2 *>(tb + off01);
+            V ph;
+            if constexpr (VEC == 4) {
+                const float4 q01 = *reinterpret_cast<const float4 *>(tb + off23);
+                const float4 q23 = *reinterpret_cast<const float4 *>(tb + off23 + HS * (int)sizeof(float2));
+                ph = make_float4(fmaf(p.x, q01.x, -p.y * q01.y), fmaf(p.x, q01.z, -p.y * q01.w),
+                                 fmaf(p.x, q23.x, -p.y * q23.y), fmaf(p.x, q23.z, -p.y * q23.w));
+            } else {
+                const float2 q = *reinterpret_cast<const float2 *>(tb + off23);
+                ph = fmaf(p.x, q.x, -p.y * q.y);
             }
+            d[r] = vfma(G, ph, d[r]);
+            e[r] = vfma(c, ph, e[r]);
         };
         if constexpr (LIST) {
             const char *tbase = reinterpret_cast<const char *>(tab);
@@ -485,7 +502,7 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
 #pragma unroll 1
                     for (int i = lo; i < hi; ++i) {      // (two steps per trip, to spare the copy: measured equal)
                         const float4 nx = cb.ent[i + 1];
-                        step_row(tbase + __float_as_int(en.z), en.x, en.y, d, e, r);
+                        step_row(tbase + __float_as_int(en.z), en.x, en.y, r);
                         en = nx;
                     }
                     lo = hi;
@@ -515,7 +532,7 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
                     const int tt = __ffs(mm) - 1;
                     mm &= mm - 1;
                     const float2 g2 = gc[tt];
-                    step_row(tb0 + tt * TSTRIDE, g2.x, g2.y, d, e, r);
+                    step_row(tb0 + tt * TSTRIDE, g2.x, g2.y, r);
                 }
             }
         }
@@ -523,12 +540,9 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
         if (cur.blk == NBLK - 1) {
             flush_d();
             V *tp = reinterpret_cast<V *>(trace + (size_t)cur.b * AF);
+            if (own) {
 #pragma unroll
-            for (int j = 0; j < CH; ++j) {
-                if (own[j]) {
-#pragma unroll
-                    for (int r = 0; r < SCG_A; ++r) tp[r * NCHR + tid + j * NT] = e[j][r];
-                }
+                for (int r = 0; r < SCG_A; ++r) tp[r * NCHR + tid] = e[r];
             }
         }
         __syncthreads();   // the tables just built become readable, the ones just read become writable
@@ -549,7 +563,6 @@ __global__ void __launch_bounds__(NT + (CTRL ? 32 : 0), MINB) k_window(int B, in
 #define SCG_RED_SLICES 96
 __global__ void __launch_bounds__(256) k_reduce(int n_partials, int n, const float *__restrict__ partial, float *red,
                                                 unsigned int *tickets, float *__restrict__ dW) {
-    __shared__ bool last;
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     const int gy = gridDim.y;
     float mine = 0.f;
@@ -567,18 +580,11 @@ __global__ void __launch_bounds__(256) k_reduce(int n_partials, int n, const flo
     }
     if (!tickets) {                              // fast mode: one atomic per address per slice (order not fixed)
         if (j < n) atomicAdd(dW + j, mine);
-        return;
+        return;                                  // (the whole grid returns here: no CTA is left waiting on a ticket)
     }
     if (j < n) red[(size_t)blockIdx.y * n + j] = mine;
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const unsigned int t = atomicAdd(tickets + blockIdx.x, 1u);
-        last = (t == (unsigned int)gy - 1u);
-        if (last) tickets[blockIdx.x] = 0u;      // ready for the next reduction
-    }
-    __syncthreads();
-    if (last && j < n) {
+    // the last of the gy CTAs of column x adds the slice sums; the fence orders its reads after the ticket
+    if (scg_last_block(tickets + blockIdx.x, gy) && j < n) {
         __threadfence();
         float t0 = 0.f, t1 = 0.f, t2 = 0.f, t3 = 0.f;     // fixed association: four interleaved chains, then a fixed tree
         int y = 0;
@@ -633,7 +639,7 @@ __global__ void k_apply(int K, int K_opt, float *__restrict__ W, float *__restri
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
         scg_apply_elem<N1>(i, cnt[i / (SCG_A * F)], K_opt, alpha, alpha_top, steps, dW[i], W, Wt, dW);
     // the last block to finish zeroes cnt for the next window (every block has read it by then): no extra launch
-    if (scg_last_block(ticket) && threadIdx.x < K) cnt[threadIdx.x] = 0;
+    if (scg_last_block(ticket, gridDim.x) && threadIdx.x < K) cnt[threadIdx.x] = 0;
 }
 
 // ---- launch plumbing ----------------------------------------------------------------------------
@@ -648,26 +654,25 @@ static int ensure_partials(scg_ctx *ctx, int n) {
     return 0;
 }
 
-template <int N1>
-static size_t window_smem(const scg_ctx *ctx, int k_used, bool multi, bool list = true) {
-    constexpr int NN = N1 * N1;
-    return (((size_t)k_used * SCG_A * ctx->F + 3) & ~(size_t)3) * sizeof(float) +
-           (size_t)2 * SCG_WIN_TB * (N1 == 6 ? NN + 64 : 2 * NN) * sizeof(float2) +
-           2 * (multi ? sizeof(WinCtlT<SCG_WIN_MAX>) : (list ? sizeof(WinCtlList) : sizeof(WinCtlT<SCG_WIN_TB>))) + 36 * sizeof(float);
+// bytes of dynamic shared memory the sweep takes (multi: the multi-block sweep of a window longer than 8 steps)
+template <class Cfg>
+static size_t window_smem(int k_used, bool multi) {
+    return multi ? WinLayout<Cfg, true>::bytes(k_used) : WinLayout<Cfg, false>::bytes(k_used);
 }
 
 // k_used: options that can appear in the window's records (ids 0 .. k_used-1): the CTA accumulator, the slabs and
 // the reduction only cover those, which is what lets two CTAs share an SM at order 5 while the chain is short
-template <int N1, int VEC, int NT, int CH, bool MULTI, int MINB, bool CTRL, bool LISTP, bool L2PF, bool SPLITP>
-static int launch_window_tm(scg_ctx *ctx, int B, int T, int k_used, const float4 *rec, float *trace, float gl,
-                            float *dW, cudaStream_t st) {
-    const size_t smem = window_smem<N1>(ctx, k_used, MULTI, LISTP);
+template <class Cfg>
+static int launch_window(scg_ctx *ctx, int B, int T, int k_used, const float4 *rec, float *trace, float gl, float *dW,
+                         cudaStream_t st) {
+    const bool multi = T > SCG_WIN_TB;
+    const size_t smem = window_smem<Cfg>(k_used, multi);
     if (smem > 227 * 1024) return SCG_ELIMIT;   // the CTA accumulator must fit in shared memory
-    auto kern = k_window<N1, VEC, NT, CH, MULTI, MINB, CTRL, LISTP, L2PF, SPLITP>;
-    constexpr int NTT = NT + (CTRL ? 32 : 0);
-    static ScgKernelCfg cfgc = {};
+    auto kern = multi ? k_window<Cfg, true> : k_window<Cfg, false>;
+    constexpr int NTT = Cfg::NT + (Cfg::CTRL ? 32 : 0);
+    static ScgKernelCfg cfgc[2] = {};
     int per_sm = 0;
-    int rcc = scg_configure(cfgc, kern, NTT, smem, &per_sm);
+    int rcc = scg_configure(cfgc[multi], kern, NTT, smem, &per_sm);
     if (rcc) return rcc;
     if (per_sm < 1) return SCG_ELIMIT;
     int grid = scg_grid(B, 1, per_sm);
@@ -676,13 +681,6 @@ static int launch_window_tm(scg_ctx *ctx, int B, int T, int k_used, const float4
     kern<<<grid, NTT, smem, st>>>(B, k_used, T, rec, trace, ctx->d_partial, gl, dW, ctx->K);
     SCG_LAUNCH_CHECK();
     return grid;
-}
-
-template <int N1, int VEC, int NT, int CH, int MINB = 1, bool CTRL = false, bool LISTP = true, bool L2PF = false, bool SPLITP = false>
-static int launch_window_t(scg_ctx *ctx, int B, int T, int k_used, const float4 *rec, float *trace, float gl,
-                           float *dW, cudaStream_t st) {
-    if (T <= SCG_WIN_TB) return launch_window_tm<N1, VEC, NT, CH, false, MINB, CTRL, LISTP, L2PF, SPLITP>(ctx, B, T, k_used, rec, trace, gl, dW, st);
-    return launch_window_tm<N1, VEC, NT, CH, true, MINB, CTRL, false, L2PF, false>(ctx, B, T, k_used, rec, trace, gl, dW, st);
 }
 
 int scg_prof_push(scg_ctx *ctx, int kind, cudaStream_t st, bool end);
@@ -695,26 +693,11 @@ int scg_launch_window(scg_ctx *ctx, int B, int T, int k_used, const float *rec, 
     const float4 *r4 = reinterpret_cast<const float4 *>(rec);
     int grid = 0, rc;
     if ((rc = scg_prof_push(ctx, 1, st, false))) return rc;
-    switch (ctx->order) {
-        // <N1, floats per chunk, threads, chunks per thread, min CTAs per SM, scan warp, step lists, L2 prefetch>
-        case 1: grid = launch_window_t<2, 4, 32, 1>(ctx, B, T, k_used, r4, trace, gl, dW, st); break;
-        case 2: grid = launch_window_t<3, 1, 96, 1>(ctx, B, T, k_used, r4, trace, gl, dW, st); break;
-        case 3:
-            // two warps per env.  With the next trace prefetched into L2 instead of registers the sweep needs 140
-            // registers (7 CTAs per SM) and loses nothing when squeezed to 128 (8 CTAs, while 8 accumulators fit);
-            // with more option slots in use (larger accumulators) the same sweep without the split warps or the squeeze
-            if (8 * (window_smem<4>(ctx, k_used, T > SCG_WIN_TB) + 1024) <= 227 * 1024)
-                grid = launch_window_t<4, 4, 64, 1, 8, false, true, true, true>(ctx, B, T, k_used, r4, trace, gl, dW, st);
-            else grid = launch_window_t<4, 4, 64, 1, 1, false, true, true>(ctx, B, T, k_used, r4, trace, gl, dW, st);
-            break;
-        case 4: grid = launch_window_t<5, 1, 640, 1>(ctx, B, T, k_used, r4, trace, gl, dW, st); break;
-        case 5:
-            // one CTA per SM: 11 work warps + a warp that only runs the per-env scan; next trace prefetched in registers
-            // (L2 prefetch: 1.98 vs 1.75 ms - one CTA cannot cover the L2 latency); bit-mask loop (step lists: 1.74 vs 1.70 ms)
-            grid = launch_window_t<6, 4, 352, 1, 1, true, false>(ctx, B, T, k_used, r4, trace, gl, dW, st);
-            break;
-        default: return SCG_ELIMIT;
-    }
+    // order 3: the split, squeezed sweep while the shared memory of 8 CTAs (and the 1 KB each reserves) fits an SM
+    const bool o3_split = 8 * (window_smem<WinCfgO3Split>(k_used, T > SCG_WIN_TB) + 1024) <= 227 * 1024;
+    DISPATCH_ORDER(ctx->order, grid = N1 == 4 && o3_split
+                                          ? launch_window<WinCfgO3Split>(ctx, B, T, k_used, r4, trace, gl, dW, st)
+                                          : launch_window<WinCfg<N1>>(ctx, B, T, k_used, r4, trace, gl, dW, st));
     if (grid <= 0) return grid == 0 ? SCG_EINVAL : grid;
     if ((rc = scg_prof_push(ctx, 1, st, true))) return rc < 0 ? rc : -rc;
     return grid;

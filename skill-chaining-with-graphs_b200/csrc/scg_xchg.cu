@@ -112,7 +112,7 @@ __global__ void __launch_bounds__(XCHG_SLICE, 8) k_sync(const __grid_constant__ 
     if (j < a.n)
         scg_apply_elem<N1>(j, s_cnt[j / (SCG_A * F)], a.K_opt, a.alpha, a.alpha_top, a.steps, v, a.W, a.Wt, a.dW);
     // the last CTA to finish zeroes cnt for the next window (every CTA read it when it published)
-    if (scg_last_block(a.ticket) && i < a.K) a.cnt[i] = 0;
+    if (scg_last_block(a.ticket, gridDim.x) && i < a.K) a.cnt[i] = 0;
 }
 
 // ---- host side ------------------------------------------------------------------------------------------

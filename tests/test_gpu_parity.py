@@ -986,9 +986,21 @@ def test_two_rank_agents_on_one_device_equal_single_agent_and_union_fit(scg, tor
 
 
 # ---- windowed pipeline -------------------------------------------------------------------------------
-@pytest.mark.parametrize("order,K,window,name", [(3, 4, 8, "easy"), (2, 3, 5, "easy"), (5, 8, 8, "hard"), (1, 2, 3, "easy"),
-                                                 (4, 2, 4, "hard"), (3, 4, 20, "easy")])
-def test_windowed_sweep_equals_oracle_dense_traces(scg, torch, order, K, window, name):
+# (order, K, window, map, active options).  Windows longer than 8 steps run the multi-block sweep.  At order 3, five
+# option slots in use (four active options and the gestating slot) no longer fit the eight CTAs of the split sweep, so
+# the last row runs its fallback.
+_WINDOW_ROWS = [(3, 4, 8, "easy", 1), (2, 3, 5, "easy", 1), (5, 8, 8, "hard", 1), (1, 2, 3, "easy", 1),
+                (4, 2, 4, "hard", 1), (3, 4, 20, "easy", 1), (1, 2, 12, "easy", 1), (2, 3, 9, "easy", 1),
+                (4, 2, 16, "hard", 1), (5, 8, 12, "hard", 1), (3, 5, 12, "easy", 4)]
+# initiation sets of the active options, in chain order: x >= 0.5, y >= 0.7, x <= 0.3, y <= 0.3 (the gestating slot
+# takes the rest)
+_WINDOW_THETA = [[-1.0, 2.0, 0.0, 0.0, 0.0, 0.0], [-1.4, 0.0, 2.0, 0.0, 0.0, 0.0], [0.6, -2.0, 0.0, 0.0, 0.0, 0.0],
+                 [0.6, 0.0, -2.0, 0.0, 0.0, 0.0]]
+
+
+@pytest.mark.parametrize("order,K,window,name,n_active", _WINDOW_ROWS,
+                         ids=["-".join(map(str, r if r[4] > 1 else r[:4])) for r in _WINDOW_ROWS])
+def test_windowed_sweep_equals_oracle_dense_traces(scg, torch, order, K, window, name, n_active):
     """One window of fused steps with frozen weights: the GPU's forward-view sweep must reproduce the
     oracle's DENSE per-step traces and dW (the parity target is the dense form's numbers)."""
     B = 700 if order >= 4 else 2500
@@ -996,14 +1008,14 @@ def test_windowed_sweep_equals_oracle_dense_traces(scg, torch, order, K, window,
     oag, gag = _paired_agents(scg, torch, B, order, K, name, 7, **kw)
     gag2 = None
     theta = np.zeros((K, 6), dtype=np.float32)
-    theta[0] = [-1.0, 2.0, 0.0, 0.0, 0.0, 0.0]
+    theta[:n_active] = _WINDOW_THETA[:n_active]
     oag.options.theta[:] = theta
-    oag.active[0] = True
-    oag.n_active = 1
-    oag.parents[1] = 1
+    oag.active[:n_active] = True
+    oag.n_active = n_active
     gag.options.theta.copy_(torch.as_tensor(theta))
-    gag.active_mask, gag.n_active = 1, 1
-    gag.parents_host[1] = 1
+    gag.active_mask, gag.n_active = (1 << n_active) - 1, n_active
+    for k in range(1, n_active + 1):            # chain mode: option k reaches for option k-1's initiation set
+        oag.parents[k] = gag.parents_host[k] = 1 << (k - 1)
     gag._push_parents()
     gag.win_cap = window
     # rebuild the window buffer for the requested window length
@@ -1023,6 +1035,7 @@ def test_windowed_sweep_equals_oracle_dense_traces(scg, torch, order, K, window,
         assert_close(gag.delta.cpu().numpy(), out["delta"])
     assert out is not None and int(gag._struct.win_len) == (n_steps % window)
     assert np.array_equal(gag.options.cnt.cpu().numpy(), oag.options.cnt)
+    assert (oag.options.cnt[:n_active + 1] > 0).all()                     # every option slot in use has steps
     assert_close(gag.options.trace.cpu().numpy(), oag.options.trace)      # property flushes the window
     assert_close(gag.options.dW.cpu().numpy(), oag.options.dW)
     assert int(gag._struct.win_len) == 0
