@@ -117,6 +117,8 @@ int scg_ctx_destroy(scg_ctx_t *ctx);
  * atomics) and the double-precision sum of finished returns in `stats` (integer-valued rewards: exact in practice).
  * off (default): one atomic per address per slice, ~1 us per step faster at configs[1]. */
 int scg_ctx_set_deterministic(scg_ctx_t *ctx, int on);
+/* One dense Sarsa(lambda) step over all of the context's K option slots; any K <= SCG_MAX_OPTIONS (16) at every order
+ * (at order 5 the slots beyond 8 accumulate in global memory instead of shared memory). */
 int scg_sarsa_update(scg_ctx_t *ctx, int B, const float *x, const float *y, const float *vx,
                      const float *vy, const int *a, const int *option, const float *delta,
                      const uint8_t *done, const uint8_t *mask /* may be NULL */, float gamma_lambda,
@@ -219,7 +221,8 @@ typedef struct scg_agent {
  * win_len reaches win_cap.  Clear carry_valid whenever state, action, option or weights are changed
  * from outside (scg_apply changes the weights: callers clear it after every apply). */
 int scg_agent_step(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
-/* Fold the open window into dW and the traces (no-op when win_len == 0). */
+/* Fold the open window into dW and the traces (no-op when win_len == 0).  Accepts any K <= SCG_MAX_OPTIONS (16, the
+ * top-level slots included) at every order and batch size. */
 int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* Append the option-termination examples of the recorded, not yet processed steps to the example rings
  * (oracle/agent.py step, item 6).  The step kernel only leaves an event byte and a start position per termination; the

@@ -15,7 +15,7 @@ extern "C" const char *scg_error_string(int code) {
     if (code == 0) return "ok";
     if (code == SCG_EINVAL) return "scg: invalid argument";
     if (code == SCG_ENOMEM) return "scg: host allocation failed";
-    if (code == SCG_ELIMIT) return "scg: size exceeds a compiled-in limit (order 1..5, K <= 16, K*5*F*4 <= 227 KiB)";
+    if (code == SCG_ELIMIT) return "scg: size exceeds a compiled-in limit (order 1..5, K <= 16 option slots including the top-level ones)";
     if (code == SCG_EPEER) return "scg: a peer rank did not arrive at a cross-GPU weight exchange within the timeout; the replicas are out of step";
     if (code > 0) return cudaGetErrorString((cudaError_t)code);
     return "scg: unknown error";

@@ -214,13 +214,16 @@ extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
 // Mirrors oracle/option.py OptionSet.top_update.  The step kernel left, for every env-step at which an option terminated
 // (event byte), a record (s0, delta_top, option) in win_top.  k_top folds them into the top-level slots of dW:
 //     dW[K + o / 5][o % 5][f] += delta_top * phi_f(s0)          and  cnt[K ..] += number of events.
-// A CTA scans a contiguous chunk of the event bytes, then processes its events TOP_EB at a time: a few threads build the
-// phasor powers exp(i pi c s0_j) of the batch (one sincospi each), then every thread forms its features as products of
-// four table entries and accumulates into the CTA's shared-memory copy of the top-level rows; one atomicAdd per touched
-// element at the end.
+// A CTA walks a contiguous chunk of the event bytes in rounds of TOP_LIST bytes: it scans a round's bytes into a shared
+// list of event indices, then processes those events TOP_EB at a time: a few threads build the phasor powers
+// exp(i pi c s0_j) of the batch (one sincospi each), then every thread forms its features as products of four table
+// entries and accumulates into the CTA's shared-memory copy of the top-level rows, which carries over between rounds;
+// one atomicAdd per touched element at the end.  The list bounds the shared memory whatever B * win_len is; a chunk of
+// up to TOP_LIST bytes (B * win_len up to about 1.2 M) is one round.
 #define TOP_NT 256
 #define TOP_EB 8
 #define TOP_CTAS 148
+#define TOP_LIST 8192
 
 template <int N1>
 __global__ void __launch_bounds__(TOP_NT) k_top(int n, int K, int top_slots, const uint8_t *__restrict__ ev,
@@ -232,19 +235,14 @@ __global__ void __launch_bounds__(TOP_NT) k_top(int n, int K, int top_slots, con
     float2 *tab = reinterpret_cast<float2 *>(acc + (((size_t)K * F + 3) & ~(size_t)3));   // [TOP_EB][4][N1], 16-byte aligned
     float *dl = reinterpret_cast<float *>(tab + TOP_EB * 4 * N1);           // [TOP_EB] delta_top
     int *oo = reinterpret_cast<int *>(dl + TOP_EB);                         // [TOP_EB] option
-    int *list = oo + TOP_EB;                                                 // [chunk] flat indices of this CTA's events
-    __shared__ int n_ev;
+    int *list = oo + TOP_EB;                                 // [min(chunk, TOP_LIST)] flat indices of a round's events
+    __shared__ int n_ev;                                     // events of this CTA so far (all rounds)
     const int tid = threadIdx.x;
     const int chunk = (n + gridDim.x - 1) / gridDim.x;
     const int beg = min(n, (int)blockIdx.x * chunk), end = min(n, beg + chunk);
     for (int i = tid; i < K * F; i += TOP_NT) acc[i] = 0.f;
     if (tid == 0) n_ev = 0;
     __syncthreads();
-    for (int i = beg + tid; i < end; i += TOP_NT)
-        if (ev[i] & SCG_EV_TERM) list[atomicAdd(&n_ev, 1)] = i;
-    __syncthreads();
-    const int ne = n_ev;
-    if (ne == 0) return;
     // per-thread constants: digits of the owned features, packed 4 x 4 bits
     uint32_t dig[FPT];
 #pragma unroll
@@ -254,39 +252,51 @@ __global__ void __launch_bounds__(TOP_NT) k_top(int n, int K, int top_slots, con
         const int c3 = f % N1, c2 = (f / N1) % N1, c1 = (f / (N1 * N1)) % N1, c0 = f / (N1 * N1 * N1);
         dig[k] = (uint32_t)c0 | ((uint32_t)c1 << 4) | ((uint32_t)c2 << 8) | ((uint32_t)c3 << 12);
     }
-    for (int e0 = 0; e0 < ne; e0 += TOP_EB) {
-        const int nb = min(TOP_EB, ne - e0);
-        if (tid < nb * 4 * N1) {                                 // table entry (event, dimension j, power c)
-            const int e = tid / (4 * N1), r = tid - e * 4 * N1, j = r / N1, c = r - j * N1;
-            const float4 s0 = __ldg(top + (size_t)list[e0 + e] * 2);
-            const float raw = j == 0 ? s0.x : (j == 1 ? s0.y : (j == 2 ? s0.z : s0.w));
-            const float sh = j < 2 ? raw : __fmul_rn(__fadd_rn(raw, 2.0f), 0.25f);
-            float sn, cs;
-            sincospif((float)c * sh, &sn, &cs);
-            tab[tid] = make_float2(cs, sn);
-        }
-        if (tid < nb) {
-            const float4 r1 = __ldg(top + (size_t)list[e0 + tid] * 2 + 1);
-            dl[tid] = r1.x;
-            oo[tid] = min(max(__float_as_int(r1.y), 0), K - 1);
-        }
+    int seen = 0;                                            // events of the earlier rounds
+    for (int r0 = 0; r0 < end - beg; r0 += TOP_LIST) {
+        // (after the first round: every thread has read n_ev, and the last batch's barrier has released the list)
+        if (r0 > 0) __syncthreads();
+        const int rend = beg + min(end - beg, r0 + TOP_LIST);
+        for (int i = beg + r0 + tid; i < rend; i += TOP_NT)
+            if (ev[i] & SCG_EV_TERM) list[atomicAdd(&n_ev, 1) - seen] = i;
         __syncthreads();
-        for (int e = 0; e < nb; ++e) {
-            const float2 *t = tab + e * 4 * N1;
-            const float d = dl[e];
-            float *row = acc + (size_t)oo[e] * F;
+        const int ne = n_ev - seen;
+        seen += ne;
+        for (int e0 = 0; e0 < ne; e0 += TOP_EB) {
+            const int nb = min(TOP_EB, ne - e0);
+            if (tid < nb * 4 * N1) {                             // table entry (event, dimension j, power c)
+                const int e = tid / (4 * N1), r = tid - e * 4 * N1, j = r / N1, c = r - j * N1;
+                const float4 s0 = __ldg(top + (size_t)list[e0 + e] * 2);
+                const float raw = j == 0 ? s0.x : (j == 1 ? s0.y : (j == 2 ? s0.z : s0.w));
+                const float sh = j < 2 ? raw : __fmul_rn(__fadd_rn(raw, 2.0f), 0.25f);
+                float sn, cs;
+                sincospif((float)c * sh, &sn, &cs);
+                tab[tid] = make_float2(cs, sn);
+            }
+            if (tid < nb) {
+                const float4 r1 = __ldg(top + (size_t)list[e0 + tid] * 2 + 1);
+                dl[tid] = r1.x;
+                oo[tid] = min(max(__float_as_int(r1.y), 0), K - 1);
+            }
+            __syncthreads();
+            for (int e = 0; e < nb; ++e) {
+                const float2 *t = tab + e * 4 * N1;
+                const float d = dl[e];
+                float *row = acc + (size_t)oo[e] * F;
 #pragma unroll
-            for (int k = 0; k < FPT; ++k) {
-                const int f = tid + k * TOP_NT;
-                if (f < F) {
-                    const float2 p = scg_cmul(scg_cmul(t[dig[k] & 15], t[N1 + ((dig[k] >> 4) & 15)]),
-                                              scg_cmul(t[2 * N1 + ((dig[k] >> 8) & 15)], t[3 * N1 + (dig[k] >> 12)]));
-                    row[f] = fmaf(d, p.x, row[f]);
+                for (int k = 0; k < FPT; ++k) {
+                    const int f = tid + k * TOP_NT;
+                    if (f < F) {
+                        const float2 p = scg_cmul(scg_cmul(t[dig[k] & 15], t[N1 + ((dig[k] >> 4) & 15)]),
+                                                  scg_cmul(t[2 * N1 + ((dig[k] >> 8) & 15)], t[3 * N1 + (dig[k] >> 12)]));
+                        row[f] = fmaf(d, p.x, row[f]);
+                    }
                 }
             }
+            __syncthreads();
         }
-        __syncthreads();
     }
+    if (seen == 0) return;
     for (int i = tid; i < K * F; i += TOP_NT) {
         const float v = acc[i];
         if (v != 0.f) {
@@ -294,7 +304,7 @@ __global__ void __launch_bounds__(TOP_NT) k_top(int n, int K, int top_slots, con
             atomicAdd(dW + ((size_t)(K + j / SCG_A) * SCG_A + (j % SCG_A)) * F + f, v);
         }
     }
-    if (tid < top_slots) atomicAdd(cnt + K + tid, ne);
+    if (tid < top_slots) atomicAdd(cnt + K + tid, seen);
 }
 
 template <int N1>
@@ -318,8 +328,7 @@ int scg_launch_top(scg_ctx *ctx, const scg_agent_t *ag, cudaStream_t st) {
     const int grid = (int)std::max<long long>(1, std::min<long long>(TOP_CTAS, (n + 4095) / 4096));
     const int chunk = (int)((n + grid - 1) / grid);
     const size_t smem = ((((size_t)ag->K * ctx->F + 3) & ~(size_t)3)) * sizeof(float) + (size_t)TOP_EB * 4 * (ctx->order + 1) * sizeof(float2) +
-                        TOP_EB * (sizeof(float) + sizeof(int)) + (size_t)chunk * sizeof(int);
-    if (smem > 200 * 1024) return SCG_ELIMIT;
+                        TOP_EB * (sizeof(float) + sizeof(int)) + (size_t)std::min(chunk, TOP_LIST) * sizeof(int);
     int rc = 0;
     DISPATCH_ORDER(ctx->order, rc = launch_top<N1>(ag, (int)n, grid, smem, st));
     return rc;

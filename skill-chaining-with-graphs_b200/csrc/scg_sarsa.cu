@@ -130,9 +130,19 @@ struct WinLayout {
     __host__ __device__ static constexpr size_t bytes(int k_used) {
         return acc_floats(k_used) * sizeof(float) + N_TAB * sizeof(float2) + N_CTL * sizeof(Ctl) + N_GLPOW * sizeof(float);
     }
+    // option slots whose accumulator stays in shared memory: the most for which the layout fits a CTA's 227 KiB.  Only
+    // order 5 holds fewer than SCG_MAX_OPTIONS (8); its spill sweep accumulates the slots beyond in global memory.
+    static constexpr int K_SM = [] {
+        int k = SCG_MAX_OPTIONS;
+        while (k > 1 && bytes(k) > 227 * 1024) --k;
+        return k;
+    }();
 };
 
-template <class Cfg, bool MULTI>
+// SPILL: more option slots are in use (K) than the shared accumulator holds (L::K_SM).  Slots K_SM .. K-1 accumulate in
+// this CTA's own slab rows in global memory, which the reduction reads anyway: the thread that owns a chunk zeroes it,
+// adds to it and leaves it there, so each element still has one writer and a fixed order of additions.
+template <class Cfg, bool MULTI, bool SPILL>
 __global__ void __launch_bounds__(Cfg::NT + (Cfg::CTRL ? 32 : 0), Cfg::MINB)
 k_window(int B, int K, int T, const float4 *__restrict__ rec, float *trace, float *__restrict__ partial, float gl,
          float *dW, int K_all) {
@@ -153,9 +163,11 @@ k_window(int B, int K, int T, const float4 *__restrict__ rec, float *trace, floa
     constexpr int TSTRIDE = TSZ * (int)sizeof(float2);    // bytes between the tables of consecutive steps
     static_assert(F % VEC == 0 && NT >= NCHR && NT >= 32 && SCG_WIN_MAX <= 32, "layout");
     static_assert(VEC == 1 || NN % VEC == 0, "a chunk shares its (c0, c1) digits");
+    static_assert(!SPILL || L::K_SM < SCG_MAX_OPTIONS, "a spill sweep only where the slots do not all fit on chip");
+    const int KS = SPILL ? L::K_SM : K;                  // option slots accumulated in shared memory
     extern __shared__ __align__(128) unsigned char smem_raw[];
-    float *acc = reinterpret_cast<float *>(smem_raw);                                      // [K][AF]
-    float2 *tab = reinterpret_cast<float2 *>(acc + L::acc_floats(K));                      // [2][TABS]
+    float *acc = reinterpret_cast<float *>(smem_raw);                                      // [KS][AF]
+    float2 *tab = reinterpret_cast<float2 *>(acc + L::acc_floats(KS));                     // [2][TABS]
     WinCtl *ctl = reinterpret_cast<WinCtl *>(tab + L::N_TAB);                              // [2]
     float *glpow = reinterpret_cast<float *>(ctl + L::N_CTL);                              // [N_GLPOW]: gl^n
 
@@ -213,7 +225,18 @@ k_window(int B, int K, int T, const float4 *__restrict__ rec, float *trace, floa
     }
     auto ent_tt = [&](int k) { return REG ? e_tt[0] + k * (BT / (2 * NN)) : e_tt[REG ? 0 : k]; };
     auto ent_at = [&](int k) { return REG ? e_at[0] + k * BT : e_at[REG ? 0 : k]; };
-    for (int i = tid; i < K * AF; i += NTT) acc[i] = 0.f;
+    for (int i = tid; i < KS * AF; i += NTT) acc[i] = 0.f;
+    if constexpr (SPILL) {
+        if (own) {
+            V *sp = reinterpret_cast<V *>(partial + ((size_t)blockIdx.x * K + KS) * AF);
+            for (int o = KS; o < K; ++o, sp += SCG_A * NCHR) {
+#pragma unroll
+                for (int r = 0; r < SCG_A; ++r) {
+                    if constexpr (VEC == 4) sp[r * NCHR + tid] = vzero4(); else sp[r * NCHR + tid] = 0.f;
+                }
+            }
+        }
+    }
     if (tid == 0) {
         float p = 1.f;
         for (int n = 0; n < L::N_GLPOW; ++n) { glpow[n] = p; p *= gl; }
@@ -408,16 +431,24 @@ k_window(int B, int K, int T, const float4 *__restrict__ rec, float *trace, floa
             }
             return;
         }
-        V *ap = reinterpret_cast<V *>(acc + (size_t)o_cur * AF);
-        if (own) {
+        auto add_d = [&](V *ap) {
+            if (own) {
 #pragma unroll
-            for (int r = 0; r < SCG_A; ++r) {
-                V cur = ap[r * NCHR + tid];
-                if constexpr (VEC == 4) cur = make_float4(cur.x + d[r].x, cur.y + d[r].y, cur.z + d[r].z, cur.w + d[r].w);
-                else cur = cur + d[r];
-                ap[r * NCHR + tid] = cur;
+                for (int r = 0; r < SCG_A; ++r) {
+                    V cur = ap[r * NCHR + tid];
+                    if constexpr (VEC == 4) cur = make_float4(cur.x + d[r].x, cur.y + d[r].y, cur.z + d[r].z, cur.w + d[r].w);
+                    else cur = cur + d[r];
+                    ap[r * NCHR + tid] = cur;
+                }
+            }
+        };
+        if constexpr (SPILL) {
+            if (o_cur >= (uint32_t)KS) {                 // a slot beyond the shared accumulator: this CTA's slab row
+                add_d(reinterpret_cast<V *>(partial + ((size_t)blockIdx.x * K + o_cur) * AF));
+                return;
             }
         }
+        add_d(reinterpret_cast<V *>(acc + (size_t)o_cur * AF));
     };
 
     WinItem cur = {(int)blockIdx.x, 0};
@@ -552,7 +583,7 @@ k_window(int B, int K, int T, const float4 *__restrict__ rec, float *trace, floa
         nxt = nx2;
     }
     float *out = partial + (size_t)blockIdx.x * K * AF;
-    for (int i = tid; i < K * AF; i += NTT) out[i] = acc[i];
+    for (int i = tid; i < KS * AF; i += NTT) out[i] = acc[i];   // (SPILL: rows KS .. K-1 are already there)
 }
 
 // dW[j] += sum over the per-CTA slabs.  Block (x, y) sums every SCG_RED_SLICES-th slab, four loads in flight per thread
@@ -661,18 +692,23 @@ static size_t window_smem(int k_used, bool multi) {
 }
 
 // k_used: options that can appear in the window's records (ids 0 .. k_used-1): the CTA accumulator, the slabs and
-// the reduction only cover those, which is what lets two CTAs share an SM at order 5 while the chain is short
+// the reduction only cover those, which is what lets two CTAs share an SM at order 5 while the chain is short.  When
+// k_used slots do not fit the shared accumulator (order 5, more than 8 slots) the spill sweep keeps the first K_SM on
+// chip; the spill variant only exists where SCG_MAX_OPTIONS slots do not fit.
 template <class Cfg>
 static int launch_window(scg_ctx *ctx, int B, int T, int k_used, const float4 *rec, float *trace, float gl, float *dW,
                          cudaStream_t st) {
     const bool multi = T > SCG_WIN_TB;
-    const size_t smem = window_smem<Cfg>(k_used, multi);
-    if (smem > 227 * 1024) return SCG_ELIMIT;   // the CTA accumulator must fit in shared memory
-    auto kern = multi ? k_window<Cfg, true> : k_window<Cfg, false>;
+    constexpr int KS1 = WinLayout<Cfg, false>::K_SM, KSM = WinLayout<Cfg, true>::K_SM;
+    const int k_sm = multi ? KSM : KS1;
+    const bool spill = k_used > k_sm;
+    const size_t smem = window_smem<Cfg>(std::min(k_used, k_sm), multi);
+    auto kern = multi ? (spill ? k_window<Cfg, true, (KSM < SCG_MAX_OPTIONS)> : k_window<Cfg, true, false>)
+                      : (spill ? k_window<Cfg, false, (KS1 < SCG_MAX_OPTIONS)> : k_window<Cfg, false, false>);
     constexpr int NTT = Cfg::NT + (Cfg::CTRL ? 32 : 0);
-    static ScgKernelCfg cfgc[2] = {};
+    static ScgKernelCfg cfgc[2][2] = {};
     int per_sm = 0;
-    int rcc = scg_configure(cfgc[multi], kern, NTT, smem, &per_sm);
+    int rcc = scg_configure(cfgc[multi][spill], kern, NTT, smem, &per_sm);
     if (rcc) return rcc;
     if (per_sm < 1) return SCG_ELIMIT;
     int grid = scg_grid(B, 1, per_sm);
@@ -716,8 +752,9 @@ extern "C" int scg_ctx_create(int order, int K, scg_ctx_t **out) {
     scg_ctx *c = (scg_ctx *)calloc(1, sizeof(scg_ctx));
     if (!c) return SCG_ENOMEM;
     c->order = order; c->K = K; c->F = scg_pow4(order + 1);
-    // (the dense per-step operator scg_sarsa_update keeps a [K][A*F] accumulator per CTA and refuses sizes beyond
-    // shared memory when it is called; the agent pipeline's sweep only accumulates the option slots in use)
+    // (the dense per-step operator scg_sarsa_update sweeps all K slots, the agent pipeline's sweep only the slots in
+    // use; where they do not all fit a CTA's shared accumulator - order 5, more than 8 - the rest accumulate in global
+    // memory, so every K <= SCG_MAX_OPTIONS runs at every order)
     *out = c;   // the per-CTA dW slabs are allocated by the first sweep (ensure_partials)
     return 0;
 }
