@@ -182,8 +182,9 @@ typedef struct scg_agent {
                                         SMDP learner whose weights are slots K .. K+n-1 of W / Wt / dW / cnt (K + n <= 16) */
     float alpha_top, epsilon_top;
     int32_t init_horizon;            /* an example is positive iff the option hit a target within this many steps of its start */
-    float merge_overlap, goal_x, goal_y; int32_t reserved1;   /* option graph: merge detection threshold (0: every older option
-                                        and the goal are targets), the goal position (oracle/agent.py merged_parents) */
+    float merge_overlap, goal_x, goal_y;   /* option graph: merge detection threshold (0: every older option and the goal
+                                        are targets), the goal position (oracle/agent.py merged_parents) */
+    uint32_t episode_capacity;       /* records in the episode log ring (ep_log); 0 with ev_ep = ep_log = NULL: no log */
     /* per-env state (device) */
     float *x, *y, *vx, *vy;          /* current state s */
     float *x2, *y2, *vx2, *vy2;      /* the other state buffer: a step writes s' here, then the two swap */
@@ -214,6 +215,16 @@ typedef struct scg_agent {
     int32_t *n_success_global;       /* [K] n_success summed over ranks as of the last cross-GPU sync (multi-rank runs) */
     /* global statistics (device), 4 x 64 bit: [0] episodes, [1] goals (uint64), [2] sum of finished returns (double) */
     int64_t *stats;
+    /* episode log (optional: all NULL / 0 = off, and the kernels do exactly the work they do without it).  When on, the
+     * step kernel marks every episode end in its event byte and keeps (return, length) beside it; the ring pass appends
+     * the episode ends to ep_log in (step, env) order:
+     *   record i (16 bytes) at slot i % episode_capacity: uint32 step (agent step at which the episode ended),
+     *   uint32 env (global env id), float return, int32 length | goal << 31 (goal 0: the episode timed out).
+     * The last episode_capacity records survive.  ev_ep and ep_log are both NULL or both set, with episode_capacity > 0
+     * and ep_log_count set. */
+    float *ev_ep;                    /* [ev_cap][B][2] at an episode end: its return, its length (int32 bits) */
+    uint32_t *ep_log;                /* [episode_capacity][4] the records */
+    int64_t *ep_log_count;           /* [1] episodes ever logged; the next one goes to slot ep_log_count % episode_capacity */
 } scg_agent_t;
 
 /* One lock-step agent step.  Updates the struct: swaps (x..vy) with (x2..vy2) so that x..vy is the new
@@ -229,7 +240,9 @@ int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
  * rings are brought up to date here - by scg_agent_manage, when the event history is full, or on request - so the pass
  * runs once per controller interval, not once per window.  Deterministic: the examples of a step are appended in env order, steps in order,
  * exactly the oracle's sequence, whatever the launch geometry; when more than `example_capacity` examples of one option
- * arrive, the last `example_capacity` survive.  Called by flush and manage; call it before reading the rings. */
+ * arrive, the last `example_capacity` survive.  Called by flush and manage; call it before reading the rings.
+ * With the episode log on it also brings the log up to date: the same pass appends the episode ends of those steps to
+ * ep_log, in the same (step, env) order, and advances *ep_log_count.  Call it before reading the log. */
 int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* The option-creation controller (oracle/agent.py manage) as ONE kernel on `stream`, no host round trip: if the
  * gestating option g = ctl->n_active has at least gestation_successes successes (n_success[g]; across ranks:

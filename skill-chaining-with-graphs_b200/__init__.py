@@ -15,7 +15,7 @@ operator raises if libscg_b200.so or a CUDA device is missing.
 from ._lib import LIB_PATH, EXPORTS, ScgError, load as load_library
 from .pinball import PinballMap, PinballEnv, unpack_flags
 from .option import FourierBasis, OptionSet, Option
-from .agent import SkillChainAgent, AgentConfig
+from .agent import SkillChainAgent, AgentConfig, merge_episodes
 
 __all__ = ["LIB_PATH", "EXPORTS", "ScgError", "load_library", "PinballMap", "PinballEnv", "unpack_flags",
-           "FourierBasis", "OptionSet", "Option", "SkillChainAgent", "AgentConfig"]
+           "FourierBasis", "OptionSet", "Option", "SkillChainAgent", "AgentConfig", "merge_episodes"]

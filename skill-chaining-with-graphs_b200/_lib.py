@@ -41,7 +41,7 @@ class AgentStruct(C.Structure):
         ("alpha", C.c_float), ("window_steps", C.c_int32), ("win_cap", C.c_int32), ("win_len", C.c_int32),
         ("ev_cap", C.c_int32), ("ev_len", C.c_int32), ("ring_len", C.c_int32), ("gestation_successes", C.c_int32), ("clf_steps", C.c_int32), ("clf_lr", C.c_float),
         ("top_slots", C.c_int32), ("alpha_top", C.c_float), ("epsilon_top", C.c_float), ("init_horizon", C.c_int32),
-        ("merge_overlap", C.c_float), ("goal_x", C.c_float), ("goal_y", C.c_float), ("reserved1", C.c_int32),
+        ("merge_overlap", C.c_float), ("goal_x", C.c_float), ("goal_y", C.c_float), ("episode_capacity", C.c_uint32),
         ("x", C.c_void_p), ("y", C.c_void_p), ("vx", C.c_void_p), ("vy", C.c_void_p),
         ("x2", C.c_void_p), ("y2", C.c_void_p), ("vx2", C.c_void_p), ("vy2", C.c_void_p),
         ("action", C.c_void_p), ("option", C.c_void_p), ("t_opt", C.c_void_p), ("ep_steps", C.c_void_p),
@@ -55,6 +55,7 @@ class AgentStruct(C.Structure):
         ("ex_count", C.c_void_p), ("n_success", C.c_void_p), ("n_fail", C.c_void_p),
         ("n_success_global", C.c_void_p),
         ("stats", C.c_void_p),
+        ("ev_ep", C.c_void_p), ("ep_log", C.c_void_p), ("ep_log_count", C.c_void_p),
     ]
 
 

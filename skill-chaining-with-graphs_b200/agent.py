@@ -50,6 +50,8 @@ class AgentConfig:
     clf_steps: int = 200
     clf_lr: float = 1.0
     event_history: int = 64       # steps of option-termination events kept on the device between example-ring passes
+    episode_log: int = 0          # records in the device episode log ring (every finished episode: step, env, return,
+                                  # length, goal; read with episodes()); 0: no log
     init_horizon: int = 1 << 30   # an example is positive iff the option hit a target within this many steps of its start
     merge_overlap: float = 0.0    # graph mode: an older option's initiation set becomes a target of the next option iff at
                                   # least this fraction of the promoted option's positive examples lies inside it (0: all)
@@ -126,6 +128,17 @@ class SkillChainAgent:
         self._n_success_global = torch.zeros(_lib.MAX_OPTIONS, **i32)
         self.n_success, self.n_fail, self.n_success_global = self._n_success[:K], self._n_fail[:K], self._n_success_global[:K]
         self.stats = torch.zeros(4, dtype=torch.int64, device=dev)
+        # episode log (optional): the step kernel marks episode ends in the event bytes and keeps (return, length) in
+        # ev_ep; the ring pass appends them to the log ring _ep_log ([capacity][4]: step, env, return bits,
+        # length | goal << 31) and counts them in _ep_log_count
+        if int(cfg.episode_log) < 0:
+            raise ValueError("episode_log must be >= 0")
+        if cfg.episode_log:
+            self.ev_ep = torch.zeros((self.ev_cap, max(B, 1), 2), **f32)
+            self._ep_log = torch.zeros((int(cfg.episode_log), 4), **i32)
+            self._ep_log_count = torch.zeros(1, dtype=torch.int64, device=dev)
+        else:
+            self.ev_ep = self._ep_log = self._ep_log_count = None
         # initial state, option and action (oracle/agent.py __init__)
         s = self._sbuf[0]
         if initial_states is not None:
@@ -263,6 +276,40 @@ class SkillChainAgent:
         self._ring()
         return self._ex_count
 
+    # -- episode log ------------------------------------------------------------------------------
+    def episodes(self, since=0, gather=False):
+        """The finished episodes logged on the device (AgentConfig.episode_log > 0), brought up to date first (ring pass).
+        Returns a dict of NumPy arrays in (step, env) order - step (uint32: the agent step at which the episode ended),
+        env (uint32: global env id), ret (float32: task return), length (int32: steps), goal (bool: reached the goal,
+        else timed out) - for the records with index >= `since` that are still in the ring, and `total`, the number of
+        episodes ever logged.  Polling with since = the previous call's total returns each episode once; when more than
+        the capacity arrived in between, the oldest are gone (total - since - len(step) of them).
+        gather=True (several ranks): every rank's records, all-gathered over the process group and merged by (step, env);
+        `since` is then one value per rank (or one for all), `total` the sum and `totals` the per-rank counts."""
+        torch = self.torch
+        if not self.cfg.episode_log:
+            raise _lib.ScgError("the episode log is off: build the agent with AgentConfig(episode_log=capacity)")
+        multi = gather and world_size(self.pg) > 1
+        if multi:
+            since = since[torch.distributed.get_rank(self.pg)] if np.ndim(since) else since
+        self._ring()
+        total = int(self._ep_log_count.item())
+        cap = int(self.cfg.episode_log)
+        lo = max(int(since), total - cap, 0)
+        n = max(total - lo, 0)
+        s0 = lo % cap
+        if s0 + n <= cap:
+            rows = self._ep_log[s0:s0 + n]
+        else:                               # the range wraps around the end of the ring
+            rows = torch.cat([self._ep_log[s0:], self._ep_log[:s0 + n - cap]])
+        out = decode_episode_records(rows.cpu().numpy())
+        out["total"] = total
+        if not multi:
+            return out
+        parts = [None] * world_size(self.pg)
+        torch.distributed.all_gather_object(parts, out, group=self.pg)
+        return merge_episodes(parts)
+
     # -- plumbing --------------------------------------------------------------------------------
 
     def _make_struct(self):
@@ -289,6 +336,9 @@ class SkillChainAgent:
             setattr(g, name, getattr(self, name).data_ptr())
         g.ex_xy, g.ex_label, g.ex_count = self._ex_xy.data_ptr(), self._ex_label.data_ptr(), self._ex_count.data_ptr()
         g.win_top = self.win_top.data_ptr() if cfg.top_level else None
+        if cfg.episode_log:
+            g.episode_capacity = int(cfg.episode_log)
+            g.ev_ep, g.ep_log, g.ep_log_count = self.ev_ep.data_ptr(), self._ep_log.data_ptr(), self._ep_log_count.data_ptr()
         g.trace, g.W, g.Wt, g.theta = o._trace.data_ptr(), o.W.data_ptr(), o.Wt.data_ptr(), o.theta.data_ptr()
         g.dW, g.cnt = o._dW.data_ptr(), o._cnt.data_ptr()
         return g
@@ -567,6 +617,8 @@ class SkillChainAgent:
         o, g = self.options, self._struct
         c = self.controller_state(sync=True)
         arrs = {k.lstrip("_"): getattr(self, k).cpu().numpy() for k in self._CKPT_TENSORS}
+        if self.cfg.episode_log:
+            arrs.update(ep_log=self._ep_log.cpu().numpy(), ep_log_count=self._ep_log_count.cpu().numpy())
         arrs.update(W=o.W.cpu().numpy(), theta=o.theta.cpu().numpy(), trace=o._trace.cpu().numpy(),
                     dW=o._dW.cpu().numpy(), cnt=o._cnt.cpu().numpy(), state=self.s.cpu().numpy(),
                     parents=np.array(c["parents"], dtype=np.uint32),
@@ -591,6 +643,15 @@ class SkillChainAgent:
         o._cnt.copy_(torch.as_tensor(z["cnt"]))
         o.pack()
         self.s.copy_(torch.as_tensor(z["state"]))
+        if self.cfg.episode_log:     # (a checkpoint without a log resumes with an empty one)
+            log, total = np.zeros((int(self.cfg.episode_log), 4), dtype=np.int32), 0
+            if "ep_log" in z.files and "ep_log_count" in z.files:
+                old, total = z["ep_log"], int(z["ep_log_count"][0])
+                # the records that fit this agent's ring keep their index i, so they sit at slot i % capacity
+                idx = np.arange(max(0, total - min(len(log), len(old))), total, dtype=np.int64)
+                log[idx % len(log)] = old[idx % len(old)]
+            self._ep_log.copy_(torch.as_tensor(log))
+            self._ep_log_count.fill_(total)
         self.torch.cuda.current_stream().synchronize()
         self._poll()
         self.parents_host[:] = z["parents"]
@@ -639,3 +700,24 @@ class SkillChainAgent:
         mean_ret = float(self.last_return[fin].double().mean()) if n_fin else float("nan")
         return dict(steps=steps, finished=n_fin, goals=int(self.stats[1]), goals_this_call=int(self.stats[1]) - goals0,
                     mean_return=mean_ret, n_active=self.controller_state(sync=True)["n_active"], env_steps=steps * self.cfg.batch)
+
+
+def decode_episode_records(rec):
+    """[n][4] int32 episode-log records (include/scg_b200.h: step, env, return bits, length | goal << 31) -> dict of
+    NumPy arrays step, env (uint32), ret (float32), length (int32), goal (bool)."""
+    rec = np.ascontiguousarray(rec, dtype=np.int32).reshape(-1, 4)
+    u = rec.view(np.uint32)
+    return dict(step=u[:, 0].copy(), env=u[:, 1].copy(), ret=rec[:, 2].copy().view(np.float32),
+                length=(u[:, 3] & 0x7FFFFFFF).astype(np.int32), goal=(u[:, 3] >> 31).astype(bool))
+
+
+def merge_episodes(parts):
+    """Merge the episodes() results of several ranks (a list in rank order) into one in (step, env) order; `total` is
+    the sum of their totals and `totals` the list of them."""
+    keys = ("step", "env", "ret", "length", "goal")
+    cat = {k: np.concatenate([p[k] for p in parts]) for k in keys}
+    order = np.lexsort((cat["env"], cat["step"]))
+    out = {k: v[order] for k, v in cat.items()}
+    out["totals"] = [int(p["total"]) for p in parts]
+    out["total"] = sum(out["totals"])
+    return out

@@ -43,6 +43,7 @@ struct StepArgs {
     uint8_t *ev;  // this step's slab of the event bytes: [B]
     float2 *pos;  // this step's slab of option start positions: [B]
     float *top;   // this step's slab of the top-level update records: [B][8] (top_slots > 0)
+    float2 *ep;   // this step's slab of episode ends (return, length as int bits): [B]; NULL: episode log off
 };
 
 // Q_slot(z, .) for the lanes of `mask` (a warp-uniform ballot), compacted: N1 lanes share one of those envs, one leading
@@ -215,6 +216,11 @@ __global__ void __launch_bounds__(NTH, 512 / NTH) k_agent_step(const __grid_cons
                 }
                 // 7: env reset
                 if (reset) {
+                    if (args.ep != nullptr) {   // episode log: the end (always also a termination) goes into the event
+                        const size_t i = (size_t)s * g.B + b;   // byte, its return and length beside it
+                        args.ev[i] |= (uint8_t)(SCG_EV_EPEND | (env_done ? SCG_EV_GOAL : 0u));
+                        args.ep[i] = make_float2(ret, __int_as_float(ep));
+                    }
                     const uint4 rr = scg_draw(g.seed, env, step, SCG_STREAM_RESET);
                     const int ns = mh->n_starts;
                     const int pick = min((int)__fmul_rn(scg_u01(rr.x), (float)ns), ns - 1);
@@ -398,6 +404,7 @@ static int check_agent(const scg_map_t *map, const scg_ctx_t *ctx, const scg_age
     if (ag->ev_cap < 2 * ag->win_cap || ag->ev_len < ag->win_len || ag->ev_len > ag->ev_cap || ag->ring_len < 0 ||
         ag->ring_len > ag->ev_len)
         return SCG_EINVAL;
+    if (!scg_episode_log_ok(ag)) return SCG_EINVAL;
     if (map->hdr.blob_bytes > 160 * 1024) return SCG_ELIMIT;
     return 0;
 }
@@ -441,6 +448,7 @@ static int agent_steps(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, in
     args.ev = ag->ev_hist + (size_t)ag->ev_len * ag->B;
     args.pos = reinterpret_cast<float2 *>(ag->ev_pos) + (size_t)ag->ev_len * ag->B;
     args.top = ag->win_top ? ag->win_top + (size_t)ag->win_len * ag->B * 8 : nullptr;
+    args.ep = ag->ev_ep ? reinterpret_cast<float2 *>(ag->ev_ep) + (size_t)ag->ev_len * ag->B : nullptr;
     args.n_steps = n;
     args.b_begin = b_begin;
     args.b_end = b_end;

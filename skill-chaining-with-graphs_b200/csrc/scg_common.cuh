@@ -18,6 +18,10 @@
 #define SCG_EV_TERM 0x80u   // the option terminated at this step
 #define SCG_EV_HIT 0x40u    // ... by reaching one of its targets (label 1), else label 0
 #define SCG_EV_OPT 0x0Fu    // option id
+// episode log on (scg_agent_t::ev_ep set): an episode ended at this step (always also TERM), with its return and length
+// in the ev_ep plane; GOAL: it ended at the goal, else it timed out
+#define SCG_EV_EPEND 0x20u
+#define SCG_EV_GOAL 0x10u
 
 extern uint64_t g_scg_launches;  // host-side launch counter (scg_api.cu)
 
@@ -596,3 +600,9 @@ __device__ __forceinline__ bool scg_last_block(unsigned int *ticket, unsigned in
     return last;
 }
 #endif  // __CUDACC__
+
+// the episode log's fields: all off (NULL / 0), or the event plane, the log ring, its count and a capacity all set
+static inline bool scg_episode_log_ok(const scg_agent_t *ag) {
+    if (!ag->ev_ep && !ag->ep_log) return true;
+    return ag->ev_ep && ag->ep_log && ag->ep_log_count && ag->episode_capacity > 0;
+}

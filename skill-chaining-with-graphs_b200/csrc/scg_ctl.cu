@@ -11,7 +11,10 @@
 //          (including which examples survive once a ring wraps) do not depend on launch geometry or atomic timing:
 //          per-CTA per-option counts (k_ring_count) -> exclusive prefix -> slot = (ex_count + rank) % capacity
 //          (k_ring_place, launched after it on the same stream), and only the last `capacity` new examples of an option
-//          are written (no two writers per slot).
+//          are written (no two writers per slot).  With the episode log on, episode ends are one more bucket after the 16
+//          options: counted, ranked (by a 17th warp) and placed by the same two kernels into the log ring, in the same
+//          order and with the same one-writer-per-slot rule.  A byte that is both an example and an episode end is
+//          ranked in both buckets.
 // k_manage One CTA.  Reads the gestating option's success count, and if it qualifies fits its logistic initiation
 //          classifier on its ring by batch gradient descent from theta = 0, flips the option to active and wires the
 //          next gestating slot's parents - all in device memory, so the agent loop never waits for the host.  Across
@@ -35,9 +38,15 @@ int scg_prof_push(scg_ctx *ctx, int kind, cudaStream_t st, bool end);
 #define RING_NT 1024
 #define RING_TILE (RING_NT * 4)      // bytes per tile: one 32-bit word per thread, coalesced
 
-// scratch layout (unsigned int): [RING_CTAS][16] per-CTA option counts | done ticket
-#define RING_DONE (RING_CTAS * SCG_MAX_OPTIONS)
+// scratch layout (unsigned int): [RING_CTAS][16] per-CTA option counts | [RING_CTAS] per-CTA episode ends | done ticket
+#define RING_EP (RING_CTAS * SCG_MAX_OPTIONS)
+#define RING_DONE (RING_EP + RING_CTAS)
 #define RING_WORDS (RING_DONE + 1)
+#define RING_BUCKETS (SCG_MAX_OPTIONS + 1)   // bucket 16: episode ends
+// flag bits of an event-list entry next to the option id (bits 0-3) and the byte index (bits 8-19)
+#define RING_L_HIT 0x10u
+#define RING_L_GOAL 0x20u
+#define RING_L_EPEND 0x40u
 
 // exclusive prefix of one value per thread over the CTA (1024 threads); *total receives the sum
 __device__ __forceinline__ uint32_t ring_block_scan(uint32_t v, uint32_t *warp_sums, uint32_t *total) {
@@ -76,19 +85,24 @@ __device__ __forceinline__ uint32_t ring_word(const uint32_t *__restrict__ evw, 
     return w;
 }
 
-// pass A: this CTA's event count per option -> scratch[blockIdx.x][o]
+// pass A: this CTA's event count per option -> scratch[blockIdx.x][o], and (ep_on) its episode ends -> scratch[RING_EP + c]
 __global__ void __launch_bounds__(RING_NT) k_ring_count(int n, const uint8_t *__restrict__ ev, unsigned int *scratch,
-                                                        int tiles_per_cta) {
-    __shared__ uint32_t cnt_s[SCG_MAX_OPTIONS];
+                                                        int tiles_per_cta, int ep_on) {
+    __shared__ uint32_t cnt_s[RING_BUCKETS];
     const int tid = threadIdx.x;
     const int mis = (int)(reinterpret_cast<uintptr_t>(ev) & 3);
     const uint32_t *evw = reinterpret_cast<const uint32_t *>(ev - mis);
     const long long nv = (long long)n + mis;
     const long long cta_lo = (long long)blockIdx.x * tiles_per_cta * RING_TILE;
-    if (tid < SCG_MAX_OPTIONS) cnt_s[tid] = 0;
+    if (tid < RING_BUCKETS) cnt_s[tid] = 0;
     __syncthreads();
     for (int t = 0; t < tiles_per_cta; ++t) {
-        uint32_t w = ring_word(evw, mis, nv, cta_lo + (long long)t * RING_TILE + tid * 4) & 0x8F8F8F8Fu;
+        uint32_t w = ring_word(evw, mis, nv, cta_lo + (long long)t * RING_TILE + tid * 4);
+        if (ep_on) {
+            const uint32_t ne = __reduce_add_sync(0xffffffffu, (uint32_t)__popc(w & 0x20202020u));   // SCG_EV_EPEND bytes
+            if ((tid & 31) == 0 && ne) atomicAdd(&cnt_s[SCG_MAX_OPTIONS], ne);
+        }
+        w &= 0x8F8F8F8Fu;
         while (w & 0x80808080u) {
             const int j = (__ffs(w & 0x80808080u) - 1) >> 3;
             atomicAdd(&cnt_s[(w >> (8 * j)) & SCG_EV_OPT], 1u);
@@ -97,31 +111,50 @@ __global__ void __launch_bounds__(RING_NT) k_ring_count(int n, const uint8_t *__
     }
     __syncthreads();
     if (tid < SCG_MAX_OPTIONS) scratch[blockIdx.x * SCG_MAX_OPTIONS + tid] = cnt_s[tid];
+    if (ep_on && tid == SCG_MAX_OPTIONS) scratch[RING_EP + blockIdx.x] = cnt_s[tid];
 }
+
+// where k_ring_place writes the episode log (ep_log NULL: off)
+struct RingEpisodeLog {
+    uint4 *ep_log;              // [cap] records (step, env, return bits, length | goal << 31)
+    long long *ep_log_count;
+    uint32_t cap;
+    const float2 *ev_ep;        // (return, length bits) at the pass's first byte, flat [step][env] like the bytes
+    uint32_t step0;             // agent step of the pass's first step
+    int B;
+    uint32_t env_offset;
+};
 
 // pass B, on the counts of every CTA that k_ring_count (same grid) left in scratch
 __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint8_t *__restrict__ ev, const float2 *__restrict__ pos,
                                                         float *ex_xy, uint8_t *ex_label, long long *ex_count, uint32_t cap,
-                                                        unsigned int *scratch, int tiles_per_cta) {
-    __shared__ uint32_t lst[RING_TILE];                 // this tile's events in flat order: option | hit << 4 | byte index << 8
+                                                        unsigned int *scratch, int tiles_per_cta, const RingEpisodeLog lg) {
+    __shared__ uint32_t lst[RING_TILE];                 // this tile's events in flat order: option | RING_L_* | byte index << 8
     __shared__ uint32_t rk[RING_TILE];                  // their rank among the CTA's events of the same option
+    __shared__ uint16_t rke[RING_TILE];                 // episode ends: their rank among this tile's episode ends
     __shared__ uint32_t warp_sums[32];
-    __shared__ uint32_t base_s[SCG_MAX_OPTIONS], tot_s[SCG_MAX_OPTIONS], run_s[SCG_MAX_OPTIONS];
-    __shared__ uint32_t slot0_s[SCG_MAX_OPTIONS];
-    __shared__ uint32_t n_tile_ev;
+    __shared__ uint32_t base_s[RING_BUCKETS], tot_s[RING_BUCKETS], run_s[RING_BUCKETS];
+    __shared__ uint32_t slot0_s[RING_BUCKETS];
+    __shared__ uint32_t n_tile_ev, ep0_s;
+    const bool ep_on = lg.ep_log != nullptr;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int mis = (int)(reinterpret_cast<uintptr_t>(ev) & 3);
     const uint32_t *evw = reinterpret_cast<const uint32_t *>(ev - mis);
     const long long nv = (long long)n + mis;
     const long long cta_lo = (long long)blockIdx.x * tiles_per_cta * RING_TILE;
     if (tid < SCG_MAX_OPTIONS) { run_s[tid] = 0; slot0_s[tid] = tid < K ? (uint32_t)((unsigned long long)ex_count[tid] % cap) : 0u; }
+    if (ep_on && tid == SCG_MAX_OPTIONS) { run_s[tid] = 0; slot0_s[tid] = (uint32_t)((unsigned long long)*lg.ep_log_count % lg.cap); }
     // every CTA's per-option totals: threads (c, o) load them with independent loads, 16 threads form this CTA's bases
-    for (int i = tid; i < (int)gridDim.x * SCG_MAX_OPTIONS; i += RING_NT) rk[i] = __ldcg(scratch + i);
+    // (and with the log on, thread 16 those of the episode ends, loaded behind them)
+    const int n_opt_words = (int)gridDim.x * SCG_MAX_OPTIONS;
+    for (int i = tid; i < n_opt_words; i += RING_NT) rk[i] = __ldcg(scratch + i);
+    if (ep_on)
+        for (int i = tid; i < (int)gridDim.x; i += RING_NT) rk[n_opt_words + i] = __ldcg(scratch + RING_EP + i);
     __syncthreads();
-    if (tid < SCG_MAX_OPTIONS) {
+    if (tid < SCG_MAX_OPTIONS || (ep_on && tid == SCG_MAX_OPTIONS)) {
         uint32_t b = 0, tt = 0;
         for (int c = 0; c < (int)gridDim.x; ++c) {
-            const uint32_t v = rk[c * SCG_MAX_OPTIONS + tid];
+            const uint32_t v = tid < SCG_MAX_OPTIONS ? rk[c * SCG_MAX_OPTIONS + tid] : rk[n_opt_words + c];
             if (c < (int)blockIdx.x) b += v;
             tt += v;
         }
@@ -143,7 +176,9 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 const uint32_t e = (w >> (8 * j)) & 0xFFu;
-                if (e & SCG_EV_TERM) lst[off++] = (e & SCG_EV_OPT) | ((e & SCG_EV_HIT) ? 16u : 0u) | ((uint32_t)(tid * 4 + j) << 8);
+                if (e & SCG_EV_TERM)
+                    lst[off++] = (e & SCG_EV_OPT) | ((e & SCG_EV_HIT) ? RING_L_HIT : 0u) | ((e & SCG_EV_GOAL) ? RING_L_GOAL : 0u) |
+                                 ((e & SCG_EV_EPEND) ? RING_L_EPEND : 0u) | ((uint32_t)(tid * 4 + j) << 8);
             }
         }
         __syncthreads();
@@ -157,6 +192,16 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
                 run += __popc(bal);
             }
             if (lane == 0) run_s[warp] = run;
+        } else if (ep_on && warp == SCG_MAX_OPTIONS && total) {     // the episode ends, ranked within the tile
+            uint32_t run = 0;
+            for (uint32_t i0 = 0; i0 < total; i0 += 32) {
+                const uint32_t i = i0 + lane;
+                const bool m = i < total && (lst[i] & RING_L_EPEND);
+                const unsigned bal = __ballot_sync(0xffffffffu, m);
+                if (m) rke[i] = (uint16_t)(run + __popc(bal & ((1u << lane) - 1u)));
+                run += __popc(bal);
+            }
+            if (lane == 0) { ep0_s = run_s[warp]; run_s[warp] += run; }
         }
         __syncthreads();
         for (uint32_t i = tid; i < total; i += RING_NT) {
@@ -167,18 +212,32 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
                 const long long f = cta_lo + (long long)t * RING_TILE + (e >> 8) - mis;     // flat [step][env] index
                 const size_t ei = (size_t)o * cap + slot;
                 *reinterpret_cast<float2 *>(ex_xy + 2 * ei) = __ldg(pos + f);
-                ex_label[ei] = (e & 16u) ? 1 : 0;
+                ex_label[ei] = (e & RING_L_HIT) ? 1 : 0;
+            }
+            if (ep_on && (e & RING_L_EPEND)) {
+                const uint32_t erank = base_s[SCG_MAX_OPTIONS] + ep0_s + rke[i];
+                if ((unsigned long long)erank + lg.cap >= tot_s[SCG_MAX_OPTIONS]) {
+                    const uint32_t slot = (uint32_t)(((unsigned long long)slot0_s[SCG_MAX_OPTIONS] + erank) % lg.cap);
+                    const long long f = cta_lo + (long long)t * RING_TILE + (e >> 8) - mis;
+                    const float2 rl = __ldg(lg.ev_ep + f);
+                    lg.ep_log[slot] = make_uint4(lg.step0 + (uint32_t)(f / lg.B), lg.env_offset + (uint32_t)(f % lg.B),
+                                                 __float_as_uint(rl.x), __float_as_uint(rl.y) | ((e & RING_L_GOAL) ? 0x80000000u : 0u));
+                }
             }
         }
         __syncthreads();
     }
     // the last CTA to finish advances the counts (every CTA has read them by then)
-    if (scg_last_block(scratch + RING_DONE, gridDim.x) && tid < K) ex_count[tid] += (long long)tot_s[tid];
+    if (scg_last_block(scratch + RING_DONE, gridDim.x)) {
+        if (tid < K) ex_count[tid] += (long long)tot_s[tid];
+        if (ep_on && tid == SCG_MAX_OPTIONS) *lg.ep_log_count += (long long)tot_s[tid];
+    }
 }
 
 extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
     if (!ctx || !ag) return SCG_EINVAL;
     if (ag->ring_len < 0 || ag->ring_len > ag->ev_len || ag->ev_len > ag->ev_cap) return SCG_EINVAL;
+    if (!scg_episode_log_ok(ag)) return SCG_EINVAL;
     const int T = ag->ev_len - ag->ring_len;
     cudaStream_t st = (cudaStream_t)stream;
     if (T > 0 && ag->B > 0) {
@@ -196,11 +255,21 @@ extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
         const size_t off = (size_t)ag->ring_len * ag->B;
         int rcp;
         if ((rcp = scg_prof_push(ctx, 4, st, false))) return rcp;
-        k_ring_count<<<grid, RING_NT, 0, st>>>((int)n, ag->ev_hist + off, ctx->d_ring, tiles_per_cta);
+        RingEpisodeLog lg = {};
+        if (ag->ep_log) {
+            lg.ep_log = reinterpret_cast<uint4 *>(ag->ep_log);
+            lg.ep_log_count = reinterpret_cast<long long *>(ag->ep_log_count);
+            lg.cap = ag->episode_capacity;
+            lg.ev_ep = reinterpret_cast<const float2 *>(ag->ev_ep) + off;
+            lg.step0 = ag->step - (uint32_t)ag->ev_len + (uint32_t)ag->ring_len;   // step of history slab ring_len
+            lg.B = ag->B;
+            lg.env_offset = ag->env_offset;
+        }
+        k_ring_count<<<grid, RING_NT, 0, st>>>((int)n, ag->ev_hist + off, ctx->d_ring, tiles_per_cta, lg.ep_log != nullptr);
         SCG_LAUNCH_CHECK();
         k_ring_place<<<grid, RING_NT, 0, st>>>((int)n, ag->K, ag->ev_hist + off, reinterpret_cast<const float2 *>(ag->ev_pos) + off,
                                                ag->ex_xy, ag->ex_label, reinterpret_cast<long long *>(ag->ex_count),
-                                               ag->example_capacity, ctx->d_ring, tiles_per_cta);
+                                               ag->example_capacity, ctx->d_ring, tiles_per_cta, lg);
         SCG_LAUNCH_CHECK();
         if ((rcp = scg_prof_push(ctx, 4, st, true))) return rcp;
     }
