@@ -85,9 +85,26 @@ __device__ __forceinline__ bool edge_hit(float4 ea, float inv, float x, float y,
     return (d2 <= r2) && (dot > 0.f);
 }
 
+__device__ __forceinline__ bool goal_hit(const StepMap &m, float x, float y) {
+    float gx = __fsub_rn(x, m.tx), gy = __fsub_rn(y, m.ty);
+    return __fadd_rn(__fmul_rn(gx, gx), __fmul_rn(gy, gy)) < m.tr2;
+}
+
+// Substeps tested per walk of a cell's candidate list (DESIGN.md section 3, K1: chosen by measurement).
+constexpr int kStepChunk = 4;
+
+// The 20 substeps run in chunks.  A chunk takes the next kStepChunk positions as the sequential loop would compute
+// them while the velocity stays as it is (x += vx h, one rounding each), keeps the leading ones that lie in the first
+// one's broad-phase cell (all of them, almost always: a ball moves at most 0.07 r per substep), loads that cell and
+// walks its candidate list once, testing every candidate edge at all of those positions - independent dependency
+// chains instead of one per substep.  The substeps before the first one with a hit or a goal are committed as they
+// are; that substep then runs the sequential loop's collision response and goal test in the same order, and the
+// next chunk starts after it with the new velocity.  So every committed substep sees exactly the position, velocity,
+// edge set and goal bit the one-substep-at-a-time loop saw, and the result is the same bit for bit.
 template <bool kCull>
 __device__ __forceinline__ void pinball_step(const StepMap &m, float &x, float &y, float &vx, float &vy, int a,
                                              float &reward, int &flags) {
+    constexpr int C = kStepChunk;
     const float kImpulse = 0.2f;  // fp32(1)/fp32(5)
     if (a == 0) vx = fminf(fmaxf(__fadd_rn(vx, kImpulse), -1.f), 1.f);
     else if (a == 1) vy = fminf(fmaxf(__fadd_rn(vy, kImpulse), -1.f), 1.f);
@@ -96,38 +113,65 @@ __device__ __forceinline__ void pinball_step(const StepMap &m, float &x, float &
     int kind = 0, ids = 0;
     bool done = false;
 #pragma unroll 1
-    for (int i = 0; i < 20; ++i) {
-        x = __fadd_rn(x, __fmul_rn(vx, m.h));
-        y = __fadd_rn(y, __fmul_rn(vy, m.h));
-        int nhit = 0, first = -1;
-        // cell of (x, y): floor(x G) is exact (G is a power of two), and 0 <= x < 1 is 0 <= floor(x G) < G
-        const int ci = __float2int_rd(x * m.gf), cj = __float2int_rd(y * m.gf);
-        const bool in_grid = kCull && (unsigned)ci < (unsigned)m.G && (unsigned)cj < (unsigned)m.G;
-        bool goal_near = true;
-        if (in_grid) {
-            const uint32_t cell = m.cells[ci * m.G + cj];
-            goal_near = (cell >> 31) != 0u;      // set by scg_map_create where the goal test can succeed
-            const int cnt = cell & 0xFF, start = (cell >> 8) & 0x7FFFFF;
-#pragma unroll 1   // lists are short (0-4 edges): the unrolled-by-4 prologue cost more than it saved
-            for (int j = 0; j < cnt; ++j) {
-                int e = m.cand[start + j];
-                float4 ea = m.ea[e];
-                float inv = m.eb[e].x;
-                if (edge_hit(ea, inv, x, y, vx, vy, m.r2)) {
-                    if (first < 0) first = e;
-                    ++nhit;
-                }
-            }
-        } else {
-            for (int e = 0; e < m.n_edges; ++e) {
-                float4 ea = m.ea[e];
-                float inv = m.eb[e].x;
-                if (edge_hit(ea, inv, x, y, vx, vy, m.r2)) {
-                    if (first < 0) first = e;
-                    ++nhit;
-                }
-            }
+    for (int i = 0; i < 20;) {
+        const float hx = __fmul_rn(vx, m.h), hy = __fmul_rn(vy, m.h);
+        float px[C], py[C];
+        int key[C];   // cell of each position, -1 outside the grid (or without culling: every edge is tested)
+#pragma unroll
+        for (int k = 0; k < C; ++k) {
+            px[k] = __fadd_rn(k ? px[k - 1] : x, hx);
+            py[k] = __fadd_rn(k ? py[k - 1] : y, hy);
+            // floor(x G) is exact (G is a power of two), and 0 <= x < 1 is 0 <= floor(x G) < G
+            const int ci = __float2int_rd(px[k] * m.gf), cj = __float2int_rd(py[k] * m.gf);
+            key[k] = (kCull && (unsigned)ci < (unsigned)m.G && (unsigned)cj < (unsigned)m.G) ? ci * m.G + cj : -1;
         }
+        int n = 1;   // substeps of this chunk: the leading positions in position 0's cell, within the 20 substeps
+#pragma unroll
+        for (int k = 1; k < C; ++k) n += (n == k && i + k < 20 && key[k] == key[0]) ? 1 : 0;
+        const bool in_grid = key[0] >= 0;
+        bool goal_near = true;
+        int cnt = m.n_edges, start = 0;
+        if (in_grid) {
+            const uint32_t cell = m.cells[key[0]];
+            goal_near = (cell >> 31) != 0u;      // set by scg_map_create where the goal test can succeed
+            cnt = cell & 0xFF;
+            start = (cell >> 8) & 0x7FFFFF;
+        }
+        const unsigned live = (1u << n) - 1u;
+        // bit k of hit: substep k hits an edge; of multi: it hits two or more.  first: the first edge (lists ascend)
+        // that the earliest substep with a hit hits - the only substep whose hits are used.
+        unsigned hit = 0u, multi = 0u;
+        int first = -1;
+#pragma unroll 1   // lists are short (0-4 edges)
+        for (int j = 0; j < cnt; ++j) {
+            const int e = in_grid ? (int)m.cand[start + j] : j;
+            const float4 ea = m.ea[e];
+            const float inv = m.eb[e].x;
+            unsigned hm = 0u;
+#pragma unroll
+            for (int k = 0; k < C; ++k) hm |= edge_hit(ea, inv, px[k], py[k], vx, vy, m.r2) ? 1u << k : 0u;
+            hm &= live;
+            if (hm & ((hit & (0u - hit)) - 1u)) first = e;   // hits a substep before every earlier hit (or is the first)
+            multi |= hm & hit;
+            hit |= hm;
+        }
+        unsigned goal = 0u;
+        if (goal_near) {
+#pragma unroll
+            for (int k = 0; k < C; ++k) goal |= goal_hit(m, px[k], py[k]) ? 1u << k : 0u;
+            goal &= live;
+        }
+        // commit up to the first substep with an event, or the whole chunk
+        const unsigned ev = hit | goal;
+        const int j = ev ? __ffs(ev) - 1 : n - 1;
+#pragma unroll
+        for (int k = 0; k < C; ++k)
+            if (k == j) { x = px[k]; y = py[k]; }
+        const int sub = i + j;
+        i = sub + 1;
+        if (!ev) continue;
+        // substep `sub` as the sequential loop runs it: collision response, then the goal test on the new position
+        const int nhit = ((hit >> j) & 1u) ? (((multi >> j) & 1u) ? 2 : 1) : 0;
         if (nhit == 1) {
             float4 eb = m.eb[first];
             float k = __fmul_rn(2.0f, __fadd_rn(__fmul_rn(vx, eb.y), __fmul_rn(vy, eb.z)));
@@ -135,7 +179,7 @@ __device__ __forceinline__ void pinball_step(const StepMap &m, float &x, float &
             vy = __fsub_rn(vy, __fmul_rn(k, eb.z));
             kind = 1;
             ids = __float_as_int(eb.w);
-            if (i == 19) {
+            if (sub == 19) {
                 x = __fadd_rn(x, __fmul_rn(vx, m.h));
                 y = __fadd_rn(y, __fmul_rn(vy, m.h));
             }
@@ -145,12 +189,9 @@ __device__ __forceinline__ void pinball_step(const StepMap &m, float &x, float &
             kind = 2;
             ids = __float_as_int(m.eb[first].w);
         }
-        if (goal_near) {
-            float gx = __fsub_rn(x, m.tx), gy = __fsub_rn(y, m.ty);
-            if (__fadd_rn(__fmul_rn(gx, gx), __fmul_rn(gy, gy)) < m.tr2) {
-                done = true;
-                break;
-            }
+        if (goal_near && goal_hit(m, x, y)) {
+            done = true;
+            break;
         }
     }
     if (done) {
