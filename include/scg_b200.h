@@ -225,6 +225,23 @@ typedef struct scg_agent {
     float *ev_ep;                    /* [ev_cap][B][2] at an episode end: its return, its length (int32 bits) */
     uint32_t *ep_log;                /* [episode_capacity][4] the records */
     int64_t *ep_log_count;           /* [1] episodes ever logged; the next one goes to slot ep_log_count % episode_capacity */
+    /* option log (optional, same rules as the episode log: all NULL / 0 = off, and the kernels do exactly the work they do
+     * without it).  When on, the step kernel keeps, beside every termination's event byte, where the execution ended, how
+     * long it ran and why it stopped; the ring pass appends every termination to opt_log in (step, env) order:
+     *   record i (32 bytes) at slot i % option_capacity: uint32 step (agent step at which the option terminated),
+     *   uint32 env (global env id), uint32 option (bits 0-3) | outcome bits, int32 duration (t_opt at termination, >= 1),
+     *   float start x, y (where the execution began), float end x, y (the state the step reached, before any env reset).
+     *   Outcome bits (oracle/agent.py SkillChainAgent.step items 3 and 6), every one that holds is set:
+     *   0x100 hit (reached one of its targets), 0x200 label (the example label: hit and t_opt <= init_horizon),
+     *   0x400 env_done (the episode ended at the goal), 0x800 option_timeout (t_opt >= option_timeout),
+     *   0x1000 left (an active option whose initiation set does not hold at s'), 0x2000 episode_timeout.
+     * The last option_capacity records survive.  ev_opt, opt_log and opt_log_count are all NULL or all set, with
+     * option_capacity > 0. */
+    uint32_t option_capacity;        /* records in the option log ring (opt_log); 0 with ev_opt = opt_log = NULL: no log */
+    float *ev_opt;                   /* [ev_cap][B][4] at a termination: end x, end y, duration (int32 bits), word 2 of the
+                                        record (uint32 bits) */
+    uint32_t *opt_log;               /* [option_capacity][8] the records */
+    int64_t *opt_log_count;          /* [1] executions ever logged; the next one goes to slot opt_log_count % option_capacity */
 } scg_agent_t;
 
 /* One lock-step agent step.  Updates the struct: swaps (x..vy) with (x2..vy2) so that x..vy is the new
@@ -242,7 +259,8 @@ int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
  * exactly the oracle's sequence, whatever the launch geometry; when more than `example_capacity` examples of one option
  * arrive, the last `example_capacity` survive.  Called by flush and manage; call it before reading the rings.
  * With the episode log on it also brings the log up to date: the same pass appends the episode ends of those steps to
- * ep_log, in the same (step, env) order, and advances *ep_log_count.  Call it before reading the log. */
+ * ep_log, in the same (step, env) order, and advances *ep_log_count.  Call it before reading the log.  The option log
+ * likewise: every termination of those steps goes to opt_log in (step, env) order, and *opt_log_count advances. */
 int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* The option-creation controller (oracle/agent.py manage) as ONE kernel on `stream`, no host round trip: if the
  * gestating option g = ctl->n_active has at least gestation_successes successes (n_success[g]; across ranks:

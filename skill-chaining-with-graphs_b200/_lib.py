@@ -56,6 +56,7 @@ class AgentStruct(C.Structure):
         ("n_success_global", C.c_void_p),
         ("stats", C.c_void_p),
         ("ev_ep", C.c_void_p), ("ep_log", C.c_void_p), ("ep_log_count", C.c_void_p),
+        ("option_capacity", C.c_uint32), ("ev_opt", C.c_void_p), ("opt_log", C.c_void_p), ("opt_log_count", C.c_void_p),
     ]
 
 

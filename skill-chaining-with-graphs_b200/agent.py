@@ -52,6 +52,8 @@ class AgentConfig:
     event_history: int = 64       # steps of option-termination events kept on the device between example-ring passes
     episode_log: int = 0          # records in the device episode log ring (every finished episode: step, env, return,
                                   # length, goal; read with episodes()); 0: no log
+    option_log: int = 0           # records in the device option log ring (every option execution: step, env, option,
+                                  # duration, outcome, start and end; read with option_executions()); 0: no log
     init_horizon: int = 1 << 30   # an example is positive iff the option hit a target within this many steps of its start
     merge_overlap: float = 0.0    # graph mode: an older option's initiation set becomes a target of the next option iff at
                                   # least this fraction of the promoted option's positive examples lies inside it (0: all)
@@ -139,6 +141,17 @@ class SkillChainAgent:
             self._ep_log_count = torch.zeros(1, dtype=torch.int64, device=dev)
         else:
             self.ev_ep = self._ep_log = self._ep_log_count = None
+        # option log (optional): at every termination the step kernel keeps (end x, end y, duration, option | outcome)
+        # in ev_opt beside the event byte; the ring pass appends every termination to _opt_log ([capacity][8], the
+        # records of include/scg_b200.h) and counts them in _opt_log_count
+        if int(cfg.option_log) < 0:
+            raise ValueError("option_log must be >= 0")
+        if cfg.option_log:
+            self.ev_opt = torch.zeros((self.ev_cap, max(B, 1), 4), **f32)
+            self._opt_log = torch.zeros((int(cfg.option_log), 8), **i32)
+            self._opt_log_count = torch.zeros(1, dtype=torch.int64, device=dev)
+        else:
+            self.ev_opt = self._opt_log = self._opt_log_count = None
         # initial state, option and action (oracle/agent.py __init__)
         s = self._sbuf[0]
         if initial_states is not None:
@@ -286,23 +299,41 @@ class SkillChainAgent:
         the capacity arrived in between, the oldest are gone (total - since - len(step) of them).
         gather=True (several ranks): every rank's records, all-gathered over the process group and merged by (step, env);
         `since` is then one value per rank (or one for all), `total` the sum and `totals` the per-rank counts."""
-        torch = self.torch
         if not self.cfg.episode_log:
             raise _lib.ScgError("the episode log is off: build the agent with AgentConfig(episode_log=capacity)")
+        return self._read_log(self._ep_log, self._ep_log_count, decode_episode_records, since, gather)
+
+    def option_executions(self, since=0, gather=False):
+        """The option executions logged on the device (AgentConfig.option_log > 0), brought up to date first (ring pass):
+        one record per option termination.  Returns a dict of NumPy arrays in (step, env) order - step (uint32: the agent
+        step at which the option terminated), env (uint32: global env id), option (int32), duration (int32: steps the
+        execution ran), the outcome flags (bool; every one that holds is set) hit (reached one of its targets), label
+        (the example label: hit within init_horizon steps), env_done (the episode ended at the goal), option_timeout,
+        left (an active option whose initiation set does not hold at the state reached), episode_timeout, and start,
+        end (float32 (n, 2): where the execution began and the state it reached, before any env reset) - plus `total`.
+        `since` and `gather` work as for episodes()."""
+        if not self.cfg.option_log:
+            raise _lib.ScgError("the option log is off: build the agent with AgentConfig(option_log=capacity)")
+        return self._read_log(self._opt_log, self._opt_log_count, decode_option_records, since, gather)
+
+    def _read_log(self, ring, count, decode, since, gather):
+        """Records with index >= since still in a device log ring (record i at row i % capacity), decoded, plus `total`;
+        with gather=True across a process group, every rank's merged by (step, env)."""
+        torch = self.torch
         multi = gather and world_size(self.pg) > 1
         if multi:
             since = since[torch.distributed.get_rank(self.pg)] if np.ndim(since) else since
         self._ring()
-        total = int(self._ep_log_count.item())
-        cap = int(self.cfg.episode_log)
+        total = int(count.item())
+        cap = ring.shape[0]
         lo = max(int(since), total - cap, 0)
         n = max(total - lo, 0)
         s0 = lo % cap
         if s0 + n <= cap:
-            rows = self._ep_log[s0:s0 + n]
+            rows = ring[s0:s0 + n]
         else:                               # the range wraps around the end of the ring
-            rows = torch.cat([self._ep_log[s0:], self._ep_log[:s0 + n - cap]])
-        out = decode_episode_records(rows.cpu().numpy())
+            rows = torch.cat([ring[s0:], ring[:s0 + n - cap]])
+        out = decode(rows.cpu().numpy())
         out["total"] = total
         if not multi:
             return out
@@ -339,6 +370,10 @@ class SkillChainAgent:
         if cfg.episode_log:
             g.episode_capacity = int(cfg.episode_log)
             g.ev_ep, g.ep_log, g.ep_log_count = self.ev_ep.data_ptr(), self._ep_log.data_ptr(), self._ep_log_count.data_ptr()
+        if cfg.option_log:
+            g.option_capacity = int(cfg.option_log)
+            g.ev_opt, g.opt_log, g.opt_log_count = (self.ev_opt.data_ptr(), self._opt_log.data_ptr(),
+                                                    self._opt_log_count.data_ptr())
         g.trace, g.W, g.Wt, g.theta = o._trace.data_ptr(), o.W.data_ptr(), o.Wt.data_ptr(), o.theta.data_ptr()
         g.dW, g.cnt = o._dW.data_ptr(), o._cnt.data_ptr()
         return g
@@ -609,6 +644,12 @@ class SkillChainAgent:
                      "n_success", "n_fail", "n_success_global", "stats", "q_carry", "ep_count", "last_return", "start_vxy",
                      "opt_ret", "opt_disc")
 
+    def _logs(self):
+        """(checkpoint name, ring, count) of each device log that is on."""
+        return [(name, ring, count) for name, ring, count in (("ep_log", self._ep_log, self._ep_log_count),
+                                                              ("opt_log", self._opt_log, self._opt_log_count))
+                if ring is not None]
+
     def save(self, path):
         """Write everything needed to resume this rank (option weights, classifiers, option graph, per-env state and
         traces, counters) to `path` (.npz).  The open window is folded in first."""
@@ -617,8 +658,8 @@ class SkillChainAgent:
         o, g = self.options, self._struct
         c = self.controller_state(sync=True)
         arrs = {k.lstrip("_"): getattr(self, k).cpu().numpy() for k in self._CKPT_TENSORS}
-        if self.cfg.episode_log:
-            arrs.update(ep_log=self._ep_log.cpu().numpy(), ep_log_count=self._ep_log_count.cpu().numpy())
+        for name, ring, count in self._logs():
+            arrs.update({name: ring.cpu().numpy(), name + "_count": count.cpu().numpy()})
         arrs.update(W=o.W.cpu().numpy(), theta=o.theta.cpu().numpy(), trace=o._trace.cpu().numpy(),
                     dW=o._dW.cpu().numpy(), cnt=o._cnt.cpu().numpy(), state=self.s.cpu().numpy(),
                     parents=np.array(c["parents"], dtype=np.uint32),
@@ -643,15 +684,15 @@ class SkillChainAgent:
         o._cnt.copy_(torch.as_tensor(z["cnt"]))
         o.pack()
         self.s.copy_(torch.as_tensor(z["state"]))
-        if self.cfg.episode_log:     # (a checkpoint without a log resumes with an empty one)
-            log, total = np.zeros((int(self.cfg.episode_log), 4), dtype=np.int32), 0
-            if "ep_log" in z.files and "ep_log_count" in z.files:
-                old, total = z["ep_log"], int(z["ep_log_count"][0])
+        for name, ring, count in self._logs():     # (a checkpoint without a log resumes with an empty one)
+            log, total = np.zeros(tuple(ring.shape), dtype=np.int32), 0
+            if name in z.files and name + "_count" in z.files:
+                old, total = z[name], int(z[name + "_count"][0])
                 # the records that fit this agent's ring keep their index i, so they sit at slot i % capacity
                 idx = np.arange(max(0, total - min(len(log), len(old))), total, dtype=np.int64)
                 log[idx % len(log)] = old[idx % len(old)]
-            self._ep_log.copy_(torch.as_tensor(log))
-            self._ep_log_count.fill_(total)
+            ring.copy_(torch.as_tensor(log))
+            count.fill_(total)
         self.torch.cuda.current_stream().synchronize()
         self._poll()
         self.parents_host[:] = z["parents"]
@@ -711,10 +752,29 @@ def decode_episode_records(rec):
                 length=(u[:, 3] & 0x7FFFFFFF).astype(np.int32), goal=(u[:, 3] >> 31).astype(bool))
 
 
+# option-log outcome bits of record word 2 (include/scg_b200.h), in bit order from 0x100
+OPTION_OUTCOMES = ("hit", "label", "env_done", "option_timeout", "left", "episode_timeout")
+
+
+def decode_option_records(rec):
+    """[n][8] int32 option-log records (include/scg_b200.h: step, env, option | outcome bits, duration, start x, y,
+    end x, y) -> dict of NumPy arrays step, env (uint32), option, duration (int32), one bool array per outcome
+    (OPTION_OUTCOMES), start, end (float32 (n, 2))."""
+    rec = np.ascontiguousarray(rec, dtype=np.int32).reshape(-1, 8)
+    u = rec.view(np.uint32)
+    out = dict(step=u[:, 0].copy(), env=u[:, 1].copy(), option=(u[:, 2] & 0xF).astype(np.int32),
+               duration=rec[:, 3].copy())
+    for i, k in enumerate(OPTION_OUTCOMES):
+        out[k] = ((u[:, 2] >> (8 + i)) & 1).astype(bool)
+    out["start"] = rec[:, 4:6].copy().view(np.float32)
+    out["end"] = rec[:, 6:8].copy().view(np.float32)
+    return out
+
+
 def merge_episodes(parts):
-    """Merge the episodes() results of several ranks (a list in rank order) into one in (step, env) order; `total` is
-    the sum of their totals and `totals` the list of them."""
-    keys = ("step", "env", "ret", "length", "goal")
+    """Merge the episodes() or option_executions() results of several ranks (a list in rank order) into one in
+    (step, env) order; `total` is the sum of their totals and `totals` the list of them."""
+    keys = [k for k in parts[0] if k not in ("total", "totals")]
     cat = {k: np.concatenate([p[k] for p in parts]) for k in keys}
     order = np.lexsort((cat["env"], cat["step"]))
     out = {k: v[order] for k, v in cat.items()}

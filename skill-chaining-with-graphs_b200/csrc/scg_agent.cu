@@ -44,6 +44,7 @@ struct StepArgs {
     float2 *pos;  // this step's slab of option start positions: [B]
     float *top;   // this step's slab of the top-level update records: [B][8] (top_slots > 0)
     float2 *ep;   // this step's slab of episode ends (return, length as int bits): [B]; NULL: episode log off
+    float4 *opt;  // this step's slab of option terminations (end x, end y, duration bits, record word 2): [B]; NULL: option log off
 };
 
 // Q_slot(z, .) for the lanes of `mask` (a warp-uniform ballot), compacted: N1 lanes share one of those envs, one leading
@@ -213,6 +214,12 @@ __global__ void __launch_bounds__(NTH, 512 / NTH) k_agent_step(const __grid_cons
                 if (term) {
                     args.pos[(size_t)s * g.B + b] = make_float2(stx, sty);
                     atomicAdd((hit ? g.n_success : g.n_fail) + o, 1);
+                    if (args.opt != nullptr) {   // option log: where the execution ended (before the reset), how long, why
+                        const uint32_t why = (uint32_t)o | (hit ? SCG_OL_HIT : 0u) | ((hit && t_opt <= g.init_horizon) ? SCG_OL_LABEL : 0u) |
+                                             (env_done ? SCG_OL_ENV_DONE : 0u) | ((t_opt >= g.option_timeout) ? SCG_OL_OPTION_TIMEOUT : 0u) |
+                                             (left ? SCG_OL_LEFT : 0u) | (ep_timeout ? SCG_OL_EPISODE_TIMEOUT : 0u);
+                        args.opt[(size_t)s * g.B + b] = make_float4(nx, ny, __int_as_float(t_opt), __uint_as_float(why));
+                    }
                 }
                 // 7: env reset
                 if (reset) {
@@ -404,7 +411,7 @@ static int check_agent(const scg_map_t *map, const scg_ctx_t *ctx, const scg_age
     if (ag->ev_cap < 2 * ag->win_cap || ag->ev_len < ag->win_len || ag->ev_len > ag->ev_cap || ag->ring_len < 0 ||
         ag->ring_len > ag->ev_len)
         return SCG_EINVAL;
-    if (!scg_episode_log_ok(ag)) return SCG_EINVAL;
+    if (!scg_episode_log_ok(ag) || !scg_option_log_ok(ag)) return SCG_EINVAL;
     if (map->hdr.blob_bytes > 160 * 1024) return SCG_ELIMIT;
     return 0;
 }
@@ -449,6 +456,7 @@ static int agent_steps(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, in
     args.pos = reinterpret_cast<float2 *>(ag->ev_pos) + (size_t)ag->ev_len * ag->B;
     args.top = ag->win_top ? ag->win_top + (size_t)ag->win_len * ag->B * 8 : nullptr;
     args.ep = ag->ev_ep ? reinterpret_cast<float2 *>(ag->ev_ep) + (size_t)ag->ev_len * ag->B : nullptr;
+    args.opt = ag->ev_opt ? reinterpret_cast<float4 *>(ag->ev_opt) + (size_t)ag->ev_len * ag->B : nullptr;
     args.n_steps = n;
     args.b_begin = b_begin;
     args.b_end = b_end;

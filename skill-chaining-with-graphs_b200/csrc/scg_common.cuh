@@ -22,6 +22,13 @@
 // in the ev_ep plane; GOAL: it ended at the goal, else it timed out
 #define SCG_EV_EPEND 0x20u
 #define SCG_EV_GOAL 0x10u
+// option log on (scg_agent_t::ev_opt set): outcome bits of word 2 of a record (option id in bits 0-3), include/scg_b200.h
+#define SCG_OL_HIT 0x100u
+#define SCG_OL_LABEL 0x200u
+#define SCG_OL_ENV_DONE 0x400u
+#define SCG_OL_OPTION_TIMEOUT 0x800u
+#define SCG_OL_LEFT 0x1000u
+#define SCG_OL_EPISODE_TIMEOUT 0x2000u
 
 extern uint64_t g_scg_launches;  // host-side launch counter (scg_api.cu)
 
@@ -605,4 +612,10 @@ __device__ __forceinline__ bool scg_last_block(unsigned int *ticket, unsigned in
 static inline bool scg_episode_log_ok(const scg_agent_t *ag) {
     if (!ag->ev_ep && !ag->ep_log) return true;
     return ag->ev_ep && ag->ep_log && ag->ep_log_count && ag->episode_capacity > 0;
+}
+
+// the option log's fields: all off (NULL / 0), or the event plane, the log ring, its count and a capacity all set
+static inline bool scg_option_log_ok(const scg_agent_t *ag) {
+    if (!ag->ev_opt && !ag->opt_log && !ag->opt_log_count && ag->option_capacity == 0) return true;
+    return ag->ev_opt && ag->opt_log && ag->opt_log_count && ag->option_capacity > 0;
 }

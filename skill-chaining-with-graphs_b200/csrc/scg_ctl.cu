@@ -14,7 +14,8 @@
 //          are written (no two writers per slot).  With the episode log on, episode ends are one more bucket after the 16
 //          options: counted, ranked (by a 17th warp) and placed by the same two kernels into the log ring, in the same
 //          order and with the same one-writer-per-slot rule.  A byte that is both an example and an episode end is
-//          ranked in both buckets.
+//          ranked in both buckets.  With the option log on, every termination is a record: its rank is its position in
+//          the pass's (step, env) order, which the tile's event list already holds, so it needs no count of its own.
 // k_manage One CTA.  Reads the gestating option's success count, and if it qualifies fits its logistic initiation
 //          classifier on its ring by batch gradient descent from theta = 0, flips the option to active and wires the
 //          next gestating slot's parents - all in device memory, so the agent loop never waits for the host.  Across
@@ -114,12 +115,16 @@ __global__ void __launch_bounds__(RING_NT) k_ring_count(int n, const uint8_t *__
     if (ep_on && tid == SCG_MAX_OPTIONS) scratch[RING_EP + blockIdx.x] = cnt_s[tid];
 }
 
-// where k_ring_place writes the episode log (ep_log NULL: off)
-struct RingEpisodeLog {
-    uint4 *ep_log;              // [cap] records (step, env, return bits, length | goal << 31)
+// where k_ring_place writes the episode log and the option log (ep_log / opt_log NULL: that log is off)
+struct RingLogs {
+    uint4 *ep_log;              // [ep_cap] records (step, env, return bits, length | goal << 31)
     long long *ep_log_count;
-    uint32_t cap;
+    uint32_t ep_cap;
     const float2 *ev_ep;        // (return, length bits) at the pass's first byte, flat [step][env] like the bytes
+    uint4 *opt_log;             // [opt_cap][2] records (step, env, option | outcome, duration), (start x, y, end x, y)
+    long long *opt_log_count;
+    uint32_t opt_cap;
+    const float4 *ev_opt;       // (end x, end y, duration bits, option | outcome) at the pass's first byte, like ev_ep
     uint32_t step0;             // agent step of the pass's first step
     int B;
     uint32_t env_offset;
@@ -128,7 +133,7 @@ struct RingEpisodeLog {
 // pass B, on the counts of every CTA that k_ring_count (same grid) left in scratch
 __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint8_t *__restrict__ ev, const float2 *__restrict__ pos,
                                                         float *ex_xy, uint8_t *ex_label, long long *ex_count, uint32_t cap,
-                                                        unsigned int *scratch, int tiles_per_cta, const RingEpisodeLog lg) {
+                                                        unsigned int *scratch, int tiles_per_cta, const RingLogs lg) {
     __shared__ uint32_t lst[RING_TILE];                 // this tile's events in flat order: option | RING_L_* | byte index << 8
     __shared__ uint32_t rk[RING_TILE];                  // their rank among the CTA's events of the same option
     __shared__ uint16_t rke[RING_TILE];                 // episode ends: their rank among this tile's episode ends
@@ -143,7 +148,10 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
     const long long nv = (long long)n + mis;
     const long long cta_lo = (long long)blockIdx.x * tiles_per_cta * RING_TILE;
     if (tid < SCG_MAX_OPTIONS) { run_s[tid] = 0; slot0_s[tid] = tid < K ? (uint32_t)((unsigned long long)ex_count[tid] % cap) : 0u; }
-    if (ep_on && tid == SCG_MAX_OPTIONS) { run_s[tid] = 0; slot0_s[tid] = (uint32_t)((unsigned long long)*lg.ep_log_count % lg.cap); }
+    if (ep_on && tid == SCG_MAX_OPTIONS) { run_s[tid] = 0; slot0_s[tid] = (uint32_t)((unsigned long long)*lg.ep_log_count % lg.ep_cap); }
+    // option log: its slot of rank 0 (read before this CTA's ticket, like the other counts)
+    const bool ol_on = lg.opt_log != nullptr;
+    const uint32_t oslot0 = ol_on ? (uint32_t)((unsigned long long)*lg.opt_log_count % lg.opt_cap) : 0u;
     // every CTA's per-option totals: threads (c, o) load them with independent loads, 16 threads form this CTA's bases
     // (and with the log on, thread 16 those of the episode ends, loaded behind them)
     const int n_opt_words = (int)gridDim.x * SCG_MAX_OPTIONS;
@@ -162,6 +170,11 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
         tot_s[tid] = tt;
     }
     __syncthreads();
+    // option log: a termination's rank is the terminations of every option in earlier CTAs (obase), then those of this
+    // CTA's earlier tiles (orun), then its index in the tile's list; the pass appends otot of them
+    uint32_t obase = 0, otot = 0, orun = 0;
+    if (ol_on)
+        for (int o = 0; o < SCG_MAX_OPTIONS; ++o) { obase += base_s[o]; otot += tot_s[o]; }
     // per tile, the ordered event list (block scan), per-option ranks (warp o walks the list with ballots), then one
     // thread per event places it.  rank = position among this pass's events of the option in (step, env) order; only
     // the last `cap` of them are written, so every slot has exactly one writer.
@@ -216,28 +229,41 @@ __global__ void __launch_bounds__(RING_NT) k_ring_place(int n, int K, const uint
             }
             if (ep_on && (e & RING_L_EPEND)) {
                 const uint32_t erank = base_s[SCG_MAX_OPTIONS] + ep0_s + rke[i];
-                if ((unsigned long long)erank + lg.cap >= tot_s[SCG_MAX_OPTIONS]) {
-                    const uint32_t slot = (uint32_t)(((unsigned long long)slot0_s[SCG_MAX_OPTIONS] + erank) % lg.cap);
+                if ((unsigned long long)erank + lg.ep_cap >= tot_s[SCG_MAX_OPTIONS]) {
+                    const uint32_t slot = (uint32_t)(((unsigned long long)slot0_s[SCG_MAX_OPTIONS] + erank) % lg.ep_cap);
                     const long long f = cta_lo + (long long)t * RING_TILE + (e >> 8) - mis;
                     const float2 rl = __ldg(lg.ev_ep + f);
                     lg.ep_log[slot] = make_uint4(lg.step0 + (uint32_t)(f / lg.B), lg.env_offset + (uint32_t)(f % lg.B),
                                                  __float_as_uint(rl.x), __float_as_uint(rl.y) | ((e & RING_L_GOAL) ? 0x80000000u : 0u));
                 }
             }
+            const uint32_t orank = obase + orun + i;
+            if (ol_on && (unsigned long long)orank + lg.opt_cap >= otot) {
+                const uint32_t slot = (uint32_t)(((unsigned long long)oslot0 + orank) % lg.opt_cap);
+                const long long f = cta_lo + (long long)t * RING_TILE + (e >> 8) - mis;
+                const float4 q = __ldg(lg.ev_opt + f);
+                const float2 p0 = __ldg(pos + f);
+                lg.opt_log[2 * (size_t)slot] = make_uint4(lg.step0 + (uint32_t)(f / lg.B), lg.env_offset + (uint32_t)(f % lg.B),
+                                                          __float_as_uint(q.w), __float_as_uint(q.z));
+                lg.opt_log[2 * (size_t)slot + 1] = make_uint4(__float_as_uint(p0.x), __float_as_uint(p0.y), __float_as_uint(q.x),
+                                                              __float_as_uint(q.y));
+            }
         }
+        orun += total;
         __syncthreads();
     }
     // the last CTA to finish advances the counts (every CTA has read them by then)
     if (scg_last_block(scratch + RING_DONE, gridDim.x)) {
         if (tid < K) ex_count[tid] += (long long)tot_s[tid];
         if (ep_on && tid == SCG_MAX_OPTIONS) *lg.ep_log_count += (long long)tot_s[tid];
+        if (ol_on && tid == 0) *lg.opt_log_count += (long long)otot;
     }
 }
 
 extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
     if (!ctx || !ag) return SCG_EINVAL;
     if (ag->ring_len < 0 || ag->ring_len > ag->ev_len || ag->ev_len > ag->ev_cap) return SCG_EINVAL;
-    if (!scg_episode_log_ok(ag)) return SCG_EINVAL;
+    if (!scg_episode_log_ok(ag) || !scg_option_log_ok(ag)) return SCG_EINVAL;
     const int T = ag->ev_len - ag->ring_len;
     cudaStream_t st = (cudaStream_t)stream;
     if (T > 0 && ag->B > 0) {
@@ -255,16 +281,22 @@ extern "C" int scg_agent_ring(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
         const size_t off = (size_t)ag->ring_len * ag->B;
         int rcp;
         if ((rcp = scg_prof_push(ctx, 4, st, false))) return rcp;
-        RingEpisodeLog lg = {};
+        RingLogs lg = {};
         if (ag->ep_log) {
             lg.ep_log = reinterpret_cast<uint4 *>(ag->ep_log);
             lg.ep_log_count = reinterpret_cast<long long *>(ag->ep_log_count);
-            lg.cap = ag->episode_capacity;
+            lg.ep_cap = ag->episode_capacity;
             lg.ev_ep = reinterpret_cast<const float2 *>(ag->ev_ep) + off;
-            lg.step0 = ag->step - (uint32_t)ag->ev_len + (uint32_t)ag->ring_len;   // step of history slab ring_len
-            lg.B = ag->B;
-            lg.env_offset = ag->env_offset;
         }
+        if (ag->opt_log) {
+            lg.opt_log = reinterpret_cast<uint4 *>(ag->opt_log);
+            lg.opt_log_count = reinterpret_cast<long long *>(ag->opt_log_count);
+            lg.opt_cap = ag->option_capacity;
+            lg.ev_opt = reinterpret_cast<const float4 *>(ag->ev_opt) + off;
+        }
+        lg.step0 = ag->step - (uint32_t)ag->ev_len + (uint32_t)ag->ring_len;   // step of history slab ring_len
+        lg.B = ag->B;
+        lg.env_offset = ag->env_offset;
         k_ring_count<<<grid, RING_NT, 0, st>>>((int)n, ag->ev_hist + off, ctx->d_ring, tiles_per_cta, lg.ep_log != nullptr);
         SCG_LAUNCH_CHECK();
         k_ring_place<<<grid, RING_NT, 0, st>>>((int)n, ag->K, ag->ev_hist + off, reinterpret_cast<const float2 *>(ag->ev_pos) + off,

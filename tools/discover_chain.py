@@ -16,6 +16,14 @@ first classifier already covered the start):
 The controller runs on the device (one kernel per manage() call); the host only polls the mirror to time-stamp promotions.
 After discovery a fresh batch of envs, all at the map's own start, runs the chain greedily (epsilon = 0) for one episode
 each: the success rate and the steps to the goal are reported, next to the same numbers for the untrained agent.
+With --option-log CAP every option execution of the run is logged on the device (AgentConfig.option_log) and polled after
+each chunk; the final JSON then carries per-option totals for the whole run ("options": executions, hit and label rates,
+mean duration, the count of each outcome flag, the share of env-steps spent in the option) - how each link of the chain
+was used, and why its executions stopped.  A poll waits for the device and copies the new records to the host, so the
+run's clocks (--budget, --train-seconds, wall_s and the promotion times) leave the polls out: a logged run takes the same
+steps in the same clock time as an unlogged one, up to the overlap of host and device work that each poll's wait gives
+up and the example-ring pass that each poll runs in place of the next manage().  The time the polls took is reported
+as option_poll_s.
 """
 import argparse
 import json
@@ -26,6 +34,8 @@ import time
 import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
+from learning_curve import OptionTally  # noqa: E402
 
 
 def evaluate(scg, torch, base_map, src, args, n_env=4096, trained=True):
@@ -67,6 +77,8 @@ def main():
     ap.add_argument("--starts", type=int, default=255)
     ap.add_argument("--chunk", type=int, default=64)
     ap.add_argument("--min-chain", type=int, default=3)
+    ap.add_argument("--option-log", type=int, default=0, metavar="CAP",
+                    help="log every option execution (ring of CAP records, polled every chunk) and report per-option totals")
     args = ap.parse_args()
     import torch
     import skill_chaining_with_graphs_b200 as scg
@@ -81,54 +93,80 @@ def main():
                           max_episode_steps=args.max_episode_steps, gestation_successes=args.gestation,
                           example_capacity=8192, clf_steps=300, clf_lr=2.0, graph=args.graph, option_bonus=1000.0,
                           top_level=not args.no_top_level, alpha_top=args.alpha_top, epsilon_top=0.1,
-                          init_horizon=args.horizon)
+                          init_horizon=args.horizon, option_log=args.option_log)
     ag = scg.SkillChainAgent(cfg, train_map)
+    tally = OptionTally([0, 1 << 32], args.options) if args.option_log else None
+    opt = dict(seen=0, lost=0, s=0.0)
+
+    def poll_options():
+        if tally is not None:
+            torch.cuda.synchronize()             # the steps queued so far run on the clock, the poll does not
+            p0 = time.perf_counter()
+            ex = ag.option_executions(since=opt["seen"])
+            opt["lost"] += ex["total"] - opt["seen"] - len(ex["step"])
+            opt["seen"] = ex["total"]
+            tally.add(ex)
+            opt["s"] += time.perf_counter() - p0
+
+    def clock():                                 # wall clock less the time spent in polls of the option log
+        return time.perf_counter() - opt["s"]
     before = evaluate(scg, torch, base, ag, args, trained=False)
     start = torch.tensor([[float(base.starts[0][0]), float(base.starts[0][1]), 0.0, 0.0]], device="cuda")
     torch.cuda.synchronize()
-    t0 = time.perf_counter()
+    t0 = clock()
     log, steps, seen, done = [], 0, 0, False
 
     def start_covered(n_active):
         return bool(ag.options.initiation(start)[0, :n_active].any()) if n_active else False
 
     # skill chaining stops creating options once an initiation set covers the start state (or the slots run out)
-    while time.perf_counter() - t0 < args.budget and not done:
+    while clock() - t0 < args.budget and not done:
         ag.run(args.chunk)
         ag.manage()                                   # one kernel on the stream; nothing waits for it
         steps += args.chunk
+        poll_options()
         c = ag.controller_state(sync=False)           # the host mirror: promotions show up here a moment later
         if c["n_promotions"] > seen:
             seen = c["n_promotions"]
             covered = start_covered(c["n_active"])
-            log.append(dict(t=round(time.perf_counter() - t0, 3), steps=steps, n_active=c["n_active"],
+            log.append(dict(t=round(clock() - t0, 3), steps=steps, n_active=c["n_active"],
                             promoted_at_step=c["last_promotion_step"], start_covered=covered))
             print(json.dumps(log[-1]), flush=True)
             done = (covered and c["n_active"] >= args.min_chain) or c["n_active"] >= args.options - 1
     torch.cuda.synchronize()
-    wall = time.perf_counter() - t0
+    wall = clock() - t0
     # the chain is in place: keep learning the option policies and the top-level values for a while
-    t1 = time.perf_counter()
+    t1 = clock()
     train_steps = 0
-    while time.perf_counter() - t1 < args.train_seconds:
-        ag.run(16 * args.chunk)
+    while clock() - t1 < args.train_seconds:
+        if tally is None:
+            ag.run(16 * args.chunk)
+        else:                                         # the same steps, with a poll of the option log after each chunk
+            for _ in range(16):
+                ag.run(args.chunk)
+                poll_options()
         ag.manage()
         train_steps += 16 * args.chunk
         torch.cuda.synchronize()
-    train_wall = time.perf_counter() - t1
+    train_wall = clock() - t1
     c = ag.controller_state(sync=True)
     cnt = ag.counters()
     # how much of the free space each initiation set covers, and whether it contains the map's start
     probe = torch.as_tensor(base.sample_free_states(np.random.default_rng(1), 20000)).cuda()
     inside = ag.options.initiation(probe)[:, :c["n_active"]].float().mean(dim=0).cpu().numpy().tolist() if c["n_active"] else []
     after = evaluate(scg, torch, base, ag, args, trained=True)
+    options = {}
+    if tally is not None:
+        poll_options()
+        options = dict(options=tally.rows(0, (steps + train_steps) * args.batch), option_executions=opt["seen"],
+                       option_executions_lost=opt["lost"], option_poll_s=round(opt["s"], 3))
     print(json.dumps(dict(map=args.map, batch=args.batch, graph=args.graph, top_level=not args.no_top_level,
                           wall_s=round(wall, 3), train_after_s=round(train_wall, 2), train_after_steps=train_steps, steps=steps, env_steps=steps * args.batch, n_active=c["n_active"],
                           chain_complete=done, start_covered=start_covered(c["n_active"]), parents=c["parents"],
                           initiation_set_fraction_of_free_space=[round(v, 3) for v in inside],
                           goals=cnt["goals"], episodes=cnt["episodes"], mean_return=cnt["mean_return"],
                           n_success=cnt["n_success"].tolist(), promotions=log,
-                          greedy_from_start_untrained=before, greedy_from_start_after_discovery=after)))
+                          greedy_from_start_untrained=before, greedy_from_start_after_discovery=after, **options)))
 
 
 if __name__ == "__main__":

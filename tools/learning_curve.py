@@ -12,6 +12,11 @@ produces fewer than --capacity of them (the number lost, if any, is reported).  
   curve_episodes.jsonl    one line per bin of consecutive episodes in (step, env) order: the same fields, with
                           episodes_end (episodes finished by the bin's end) in place of env_steps
   summary.json            configuration, device, totals, the controller's promotions and the wall time
+With --option-log CAP the device option log (AgentConfig.option_log) is polled after each chunk as well, and
+  options_env_steps.jsonl one line per (bin of agent steps, option): executions that ended in the bin, hit_rate,
+                          label_rate, mean_duration, the count of each outcome flag, and env_step_share - the summed
+                          durations of those executions over the bin's env-steps (the share of the batch's time spent in
+                          the option, credited to the bin in which each execution ended)
 """
 import argparse
 import json
@@ -53,6 +58,43 @@ def bin_rows(idx_end, ret, length, goal, edges):
     return rows
 
 
+class OptionTally:
+    """Running sums over option-log records (SkillChainAgent.option_executions) per (bin of agent steps, option):
+    executions, summed duration and the count of each outcome flag.  Records are added as they are polled, so a long run
+    needs no more host memory than its bins."""
+
+    def __init__(self, edges, n_options):
+        from skill_chaining_with_graphs_b200.agent import OPTION_OUTCOMES
+        self.outcomes = OPTION_OUTCOMES
+        self.edges = np.asarray(edges, dtype=np.int64)
+        shape = (len(self.edges) - 1, n_options)
+        self.n, self.dur = np.zeros(shape, np.int64), np.zeros(shape, np.int64)
+        self.flags = {k: np.zeros(shape, np.int64) for k in OPTION_OUTCOMES}
+
+    def add(self, log):
+        b = np.searchsorted(self.edges, log["step"].astype(np.int64), side="right") - 1
+        keep = (b >= 0) & (b < self.n.shape[0])
+        at = (b[keep], log["option"][keep])
+        np.add.at(self.n, at, 1)
+        np.add.at(self.dur, at, log["duration"][keep].astype(np.int64))
+        for k in self.outcomes:
+            np.add.at(self.flags[k], at, log[k][keep].astype(np.int64))
+
+    def rows(self, i, env_steps):
+        """One dict per option for bin i, whose agent steps amount to `env_steps` env-steps."""
+        out = []
+        for o in range(self.n.shape[1]):
+            n = int(self.n[i, o])
+            row = dict(option=o, executions=n,
+                       hit_rate=self.flags["hit"][i, o] / n if n else None,
+                       label_rate=self.flags["label"][i, o] / n if n else None,
+                       mean_duration=self.dur[i, o] / n if n else None)
+            row.update({k: int(self.flags[k][i, o]) for k in self.outcomes})
+            row["env_step_share"] = float(self.dur[i, o]) / env_steps if env_steps else None
+            out.append({k: float(v) if isinstance(v, np.floating) else v for k, v in row.items()})
+        return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--map", default="easy")
@@ -71,6 +113,8 @@ def main():
     ap.add_argument("--sync-interval", type=int, default=8)
     ap.add_argument("--bins", type=int, default=50)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--option-log", type=int, default=0, metavar="CAP",
+                    help="also log every option execution (option log ring of CAP records) and write options_env_steps.jsonl")
     ap.add_argument("--out", required=True)
     args = ap.parse_args()
 
@@ -82,9 +126,13 @@ def main():
                           alpha=args.alpha, epsilon=args.epsilon, sync_interval=args.sync_interval, seed=args.seed,
                           option_timeout=args.option_timeout, max_episode_steps=args.max_episode_steps,
                           gestation_successes=args.gestation_successes, top_level=not args.no_top_level,
-                          episode_log=args.capacity)
+                          episode_log=args.capacity, option_log=args.option_log)
     ag = scg.SkillChainAgent(cfg)
     parts, seen, lost = [], 0, 0
+    # against env-steps: bins of agent steps; an episode that ended at agent step t belongs to env-step (t + 1) * batch
+    edges = np.linspace(0, args.steps, args.bins + 1).round().astype(np.int64)
+    tally = OptionTally(edges, args.options) if args.option_log else None
+    opt_seen = opt_lost = 0
     t0 = time.time()
     done = 0
     while done < args.steps:
@@ -96,6 +144,11 @@ def main():
         lost += new["total"] - seen - len(new["step"])
         seen = new["total"]
         parts.append(new)
+        if tally is not None:
+            ex = ag.option_executions(since=opt_seen)
+            opt_lost += ex["total"] - opt_seen - len(ex["step"])
+            opt_seen = ex["total"]
+            tally.add(ex)
     torch.cuda.synchronize()
     wall = time.time() - t0
     log = {k: np.concatenate([p[k] for p in parts]) for k in ("step", "env", "ret", "length", "goal")}
@@ -103,8 +156,6 @@ def main():
 
     os.makedirs(args.out, exist_ok=True)
     step = log["step"].astype(np.int64)
-    # against env-steps: bins of agent steps; an episode that ended at agent step t belongs to env-step (t + 1) * batch
-    edges = np.linspace(0, args.steps, args.bins + 1).round().astype(np.int64)
     with open(os.path.join(args.out, "curve_env_steps.jsonl"), "w") as f:
         for e, row in zip(edges[1:], bin_rows(step, log["ret"], log["length"], log["goal"], edges)):
             f.write(json.dumps(dict(env_steps=int(e) * args.batch, **row)) + "\n")
@@ -118,6 +169,12 @@ def main():
                    agent_steps=done, env_steps=done * args.batch, episodes=int(seen), episodes_lost=int(lost),
                    goals=int(log["goal"].sum()), mean_return=float(log["ret"].astype(np.float64).mean()) if n_ep else None,
                    n_active_end=ctl["n_active"], promotions=ctl["n_promotions"], wall_s=wall)
+    if tally is not None:
+        with open(os.path.join(args.out, "options_env_steps.jsonl"), "w") as f:
+            for i, e in enumerate(edges[1:]):
+                for row in tally.rows(i, int(edges[i + 1] - edges[i]) * args.batch):
+                    f.write(json.dumps(dict(env_steps=int(e) * args.batch, **row)) + "\n")
+        summary.update(option_executions=int(opt_seen), option_executions_lost=int(opt_lost))
     with open(os.path.join(args.out, "summary.json"), "w") as f:
         json.dump(summary, f, indent=1)
     print(json.dumps(summary))
