@@ -13,8 +13,10 @@
  *     DEVICE pointers unless the function name ends in `_host`
  *   - every launch is asynchronous on `stream` (a cudaStream_t passed as void*; NULL = default)
  *   - no function synchronises the device except the `_host` variants, scg_map_create, scg_xchg_create and
- *     the scratch (re)allocations inside the context (first sweep) and the map (first scg_step_host)
- *   - one host thread drives one context; entry points are re-entrant, not internally locked
+ *     the scratch (re)allocations inside the context (first sweep, first apply) and the map (first scg_step_host)
+ *   - one host thread drives one context; entry points are re-entrant, not internally locked.  The weight applies on one
+ *     context (scg_apply, scg_agent_sync, scg_agent_run) must be stream-ordered: like W and dW, they share the
+ *     context's "blocks done" counter
  *   - actions: 0 +x, 1 +y, 2 -x, 3 -y, 4 none;  A = 5;  F = (order+1)^4;  orders 1..5
  *   - state is structure-of-arrays: x[B], y[B], vx[B], vy[B] (fp32)
  */
@@ -89,7 +91,7 @@ int scg_step_host(scg_map_t *map, int B, float *state_soa /* HOST [4][B] in/out 
 /* ---- K2: Fourier features, Q evaluation, action selection, TD error ------------------------
  * mirrors oracle/fourier.py FourierBasis.features, oracle/option.py OptionSet.q / act / td_error.
  * W is [K][A][F]; Wt is the packed copy the kernels read, made by scg_pack_weights (and kept current by scg_apply /
- * scg_xchg_sync): [K][scg_packed_slot_floats(order)] fp32, a slot holding its features in pairs of 12 floats
+ * scg_xchg_sync / scg_agent_sync): [K][scg_packed_slot_floats(order)] fp32, a slot holding its features in pairs of 12 floats
  * (w0a w1a w2a w3a | w0b w1b w2b w3b | w4a w4b 0 0) - the operands of the two-wide FMAs, 1.5 16-byte loads per
  * feature - padded so that consecutive slots start 16 bytes apart modulo 128 (shared-memory banks). */
 int scg_packed_slot_floats(int order);
@@ -123,12 +125,12 @@ int scg_sarsa_update(scg_ctx_t *ctx, int B, const float *x, const float *y, cons
                      const float *vy, const int *a, const int *option, const float *delta,
                      const uint8_t *done, const uint8_t *mask /* may be NULL */, float gamma_lambda,
                      float *trace, float *dW, int *cnt, void *stream);
-int scg_apply(int order, int K, float *W, float *Wt, float *dW, int *cnt, float alpha,
+/* W += alpha * alpha_scale_f * dW * (window_steps / cnt[k]) for every slot k with cnt[k] > 0, Wt refreshed, dW and cnt
+ * zeroed, over all of the context's K slots at its order.  Slots K_opt .. K-1 hold the top-level learner
+ * (oracle/option.py OptionSet(top_slots=...)): they are stepped with alpha_top and the mean over the window's events
+ * (cnt[k] = event count) instead; K_opt == K: no top-level slots. */
+int scg_apply(scg_ctx_t *ctx, int K_opt, float *W, float *Wt, float *dW, int *cnt, float alpha, float alpha_top,
               int window_steps, void *stream);
-/* same with the top-level learner's slots (oracle/option.py OptionSet(top_slots=...)): slots K_opt .. K-1 are stepped
- * with alpha_top and the mean over the window's events (cnt[k] = event count) instead of alpha * steps / cnt[k] */
-int scg_apply_top(int order, int K, int K_opt, float *W, float *Wt, float *dW, int *cnt, float alpha,
-                  float alpha_top, int window_steps, void *stream);
 
 /* ---- K4: initiation classifiers --------------------------------------------------------------
  * mirrors oracle/option.py OptionSet.initiation_prob / clf_grad / fit_initiation. */
@@ -247,7 +249,7 @@ typedef struct scg_agent {
 /* One lock-step agent step.  Updates the struct: swaps (x..vy) with (x2..vy2) so that x..vy is the new
  * current state, step += 1, window_steps += 1, win_len += 1, carry_valid = 1; flushes the window when
  * win_len reaches win_cap.  Clear carry_valid whenever state, action, option or weights are changed
- * from outside (scg_apply changes the weights: callers clear it after every apply). */
+ * from outside (scg_apply changes the weights: callers clear it after every apply; scg_agent_sync does). */
 int scg_agent_step(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* Fold the open window into dW and the traces (no-op when win_len == 0).  Accepts any K <= SCG_MAX_OPTIONS (16, the
  * top-level slots included) at every order and batch size. */
@@ -278,11 +280,14 @@ int scg_agent_manage(scg_ctx_t *ctx, scg_agent_t *ag, scg_xchg_t *xchg, void *st
 int scg_agent_poll(scg_ctx_t *ctx, scg_ctl_t *out /* HOST */);
 /* Overwrite the controller state from the host (tests, checkpoints): device copy on `stream` + the mirror. */
 int scg_agent_set_ctl(scg_ctx_t *ctx, scg_agent_t *ag, const scg_ctl_t *in /* HOST */, void *stream);
-/* n_steps steps in one call; when sync_interval > 0 also flush + apply every sync_interval steps:
- * scg_apply for a single rank (xchg == NULL), scg_xchg_sync across ranks otherwise.  With
- * sync_interval == 0 the caller flushes, sums dW / cnt over ranks and applies. */
+/* n_steps steps in one call; when sync_interval > 0 also scg_agent_sync every sync_interval steps.  With
+ * sync_interval == 0 the caller syncs: scg_agent_sync, or flush, sum dW / cnt over ranks itself and scg_apply. */
 int scg_agent_run(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, int n_steps, int sync_interval,
                   scg_xchg_t *xchg, void *stream);
+/* The weight sync of the agent: flush the open window, then scg_apply for a single rank (xchg == NULL) or scg_xchg_sync
+ * across ranks (dW, cnt and the success counters summed over ranks), with the agent's alpha, alpha_top and window_steps
+ * (the top-level slots are K .. K+top_slots-1); then window_steps = 0 and carry_valid = 0.  Profiled as kind 3. */
+int scg_agent_sync(scg_ctx_t *ctx, scg_agent_t *ag, scg_xchg_t *xchg, void *stream);
 
 /* ---- S5: cross-GPU weight-delta exchange over NVLink peer memory ---------------------------------
  * mirrors the multi-rank half of oracle/option.py OptionSet.apply (sum dW and cnt over ranks, then the
@@ -299,20 +304,17 @@ int scg_xchg_connect(scg_xchg_t *x, const void *all_handles /* HOST [world][hand
 int scg_xchg_local_ptr(scg_xchg_t *x, void **ptr_out);
 int scg_xchg_connect_ptrs(scg_xchg_t *x, void *const *peer_ptrs /* HOST [world] device pointers */);
 /* *timed_out != 0: some exchange gave up waiting for a peer.  The flag is sticky and lives in host-mapped memory (no
- * device synchronisation to read it); from then on scg_xchg_sync and scg_agent_run return SCG_EPEER. */
+ * device synchronisation to read it); from then on scg_xchg_sync, scg_agent_sync and scg_agent_run return SCG_EPEER. */
 int scg_xchg_status(scg_xchg_t *x, int *timed_out);
 /* how long an exchange waits for its peers before giving up (default 30 s) */
 int scg_xchg_set_timeout(scg_xchg_t *x, double seconds);
-/* dW (reduced over this rank's envs) and cnt -> summed over ranks -> W, Wt updated; dW and cnt zeroed.
+/* dW (reduced over this rank's envs) and cnt -> summed over ranks -> W, Wt updated as scg_apply does (order and K of
+ * the context the handle was created from, top-level slots K_opt .. K-1); dW and cnt zeroed.
  * nsucc_local [K] (optional): this rank's option success counters; nsucc_global [K] (optional) receives their sum
  * over ranks, identical on every rank, so the controller needs no collective of its own.
  * Every rank must call it the same number of times. */
-int scg_xchg_sync(scg_xchg_t *x, int order, int K, float *W, float *Wt, float *dW, int *cnt, float alpha,
+int scg_xchg_sync(scg_xchg_t *x, int K_opt, float *W, float *Wt, float *dW, int *cnt, float alpha, float alpha_top,
                   int window_steps, const int *nsucc_local, int *nsucc_global, void *stream);
-/* same with top-level learner slots K_opt .. K-1 (see scg_apply_top) */
-int scg_xchg_sync_top(scg_xchg_t *x, int order, int K, int K_opt, float *W, float *Wt, float *dW, int *cnt,
-                      float alpha, float alpha_top, int window_steps, const int *nsucc_local, int *nsucc_global,
-                      void *stream);
 
 /* HOST-buffer variant of scg_agent_step: the call a user makes who keeps state and actions in
  * host (NumPy) arrays, as with the oracle's SkillChainAgent.  Copies state [4][B] and action [B]

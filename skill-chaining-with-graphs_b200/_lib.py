@@ -85,8 +85,7 @@ _SIGS = {
     "scg_ctx_destroy": (C.c_int, [_P]),
     "scg_ctx_set_deterministic": (C.c_int, [_P, C.c_int]),
     "scg_sarsa_update": (C.c_int, [_P, C.c_int] + [_P] * 9 + [C.c_float, _P, _P, _P, _P]),
-    "scg_apply": (C.c_int, [C.c_int, C.c_int, _P, _P, _P, _P, C.c_float, C.c_int, _P]),
-    "scg_apply_top": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, C.c_float, C.c_float, C.c_int, _P]),
+    "scg_apply": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, C.c_float, C.c_float, C.c_int, _P]),
     "scg_clf_eval": (C.c_int, [C.c_int, _P, _P, _P, C.c_int, _P, _P]),
     "scg_clf_decide": (C.c_int, [C.c_int, _P, _P, _P, C.c_int, _P, _P]),
     "scg_clf_grad": (C.c_int, [C.c_int, _P, _P, _P, _P, _P]),
@@ -98,6 +97,7 @@ _SIGS = {
     "scg_agent_poll": (C.c_int, [_P, C.POINTER(CtlStruct)]),
     "scg_agent_set_ctl": (C.c_int, [_P, C.POINTER(AgentStruct), C.POINTER(CtlStruct), _P]),
     "scg_agent_run": (C.c_int, [_P, _P, C.POINTER(AgentStruct), C.c_int, C.c_int, _P, _P]),
+    "scg_agent_sync": (C.c_int, [_P, C.POINTER(AgentStruct), _P, _P]),
     "scg_xchg_create": (C.c_int, [_P, C.c_int, C.c_int, C.POINTER(_P)]),
     "scg_xchg_destroy": (C.c_int, [_P]),
     "scg_xchg_handle_bytes": (C.c_int, []),
@@ -107,8 +107,7 @@ _SIGS = {
     "scg_xchg_connect_ptrs": (C.c_int, [_P, _P]),
     "scg_xchg_status": (C.c_int, [_P, C.POINTER(C.c_int)]),
     "scg_xchg_set_timeout": (C.c_int, [_P, C.c_double]),
-    "scg_xchg_sync": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P, _P, C.c_float, C.c_int, _P, _P, _P]),
-    "scg_xchg_sync_top": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, C.c_float, C.c_float, C.c_int, _P, _P, _P]),
+    "scg_xchg_sync": (C.c_int, [_P, C.c_int, _P, _P, _P, _P, C.c_float, C.c_float, C.c_int, _P, _P, _P]),
     "scg_agent_step_host": (C.c_int, [_P, _P, C.POINTER(AgentStruct)] + [_P] * 8),
     "scg_agent_run_host": (C.c_int, [_P, _P, C.POINTER(AgentStruct), _P, _P, C.c_int, C.c_int, _P] + [_P] * 6),
     "scg_profile_begin": (C.c_int, [_P, C.c_int, C.c_int]),

@@ -542,20 +542,17 @@ class SkillChainAgent:
         return [float(v) for v in ms], [int(v) for v in n]
 
     def sync(self):
-        """Flush the window, sum its dW / cnt over ranks (if any) and apply."""
+        """Flush the window, sum its dW / cnt over ranks (if any) and apply: one library call (scg_agent_sync) on one
+        rank or over peer memory; with the NCCL backend the all-reduce runs between the flush and the apply."""
         o, g = self.options, self._struct
-        self.flush()
-        if self._xchg is not None:
-            check(self.lib.scg_xchg_sync_top(self._xchg, o.order, o.K_all, o.K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o._cnt),
-                                             self.cfg.alpha, self.cfg.alpha_top, max(int(g.window_steps), 1),
-                                             ptr(self.n_success), ptr(self.n_success_global), _lib.current_stream()))
+        if world_size(self.pg) == 1 or self._xchg is not None:
+            check(self.lib.scg_agent_sync(o.ctx, C.byref(g), self._xchg, _lib.current_stream()))
             o.window_steps = 0
-        else:
-            allreduce_deltas(o._dW, o._cnt, self.pg)
-            o.window_steps = int(g.window_steps)
-            o.apply()
-        g.window_steps = 0
-        g.carry_valid = 0
+            return
+        self.flush()
+        allreduce_deltas(o._dW, o._cnt, self.pg)
+        o.window_steps = int(g.window_steps)
+        o.apply()
 
     def peer_sync_timed_out(self):
         """True if a peer failed to show up at some sync (the exchange kernel gives up after ~2 s)."""

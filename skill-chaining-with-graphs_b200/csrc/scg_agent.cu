@@ -502,18 +502,23 @@ extern "C" int scg_agent_run(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *
         if (sync_interval > 0) n = std::min(n, std::max(1, sync_interval - ag->window_steps));
         if ((rc = agent_steps(map, ctx, ag, n, stream))) return rc;
         done += n;
-        if (sync_interval > 0 && ag->window_steps >= sync_interval) {
-            if ((rc = scg_agent_flush(ctx, ag, stream))) return rc;
-            if ((rc = scg_prof_push(ctx, 3, (cudaStream_t)stream, false))) return rc;
-            const int Kall = ag->K + ag->top_slots;
-            if (xchg) rc = scg_xchg_sync_top(xchg, ag->order, Kall, ag->K, ag->W, ag->Wt, ag->dW, ag->cnt, ag->alpha, ag->alpha_top, ag->window_steps, ag->n_success, ag->n_success_global, stream);
-            else rc = scg_apply_top(ag->order, Kall, ag->K, ag->W, ag->Wt, ag->dW, ag->cnt, ag->alpha, ag->alpha_top, ag->window_steps, stream);
-            if (rc) return rc;
-            if ((rc = scg_prof_push(ctx, 3, (cudaStream_t)stream, true))) return rc;
-            ag->window_steps = 0;
-            ag->carry_valid = 0;
-        }
+        if (sync_interval > 0 && ag->window_steps >= sync_interval && (rc = scg_agent_sync(ctx, ag, xchg, stream)))
+            return rc;
     }
+    return 0;
+}
+
+extern "C" int scg_agent_sync(scg_ctx_t *ctx, scg_agent_t *ag, scg_xchg_t *xchg, void *stream) {
+    if (!ctx || !ag || ag->K + ag->top_slots != ctx->K) return SCG_EINVAL;   // the apply covers the context's K slots
+    int rc;
+    if ((rc = scg_agent_flush(ctx, ag, stream))) return rc;
+    if ((rc = scg_prof_push(ctx, 3, (cudaStream_t)stream, false))) return rc;
+    if (xchg) rc = scg_xchg_sync(xchg, ag->K, ag->W, ag->Wt, ag->dW, ag->cnt, ag->alpha, ag->alpha_top, ag->window_steps, ag->n_success, ag->n_success_global, stream);
+    else rc = scg_apply(ctx, ag->K, ag->W, ag->Wt, ag->dW, ag->cnt, ag->alpha, ag->alpha_top, ag->window_steps, stream);
+    if (rc) return rc;
+    if ((rc = scg_prof_push(ctx, 3, (cudaStream_t)stream, true))) return rc;
+    ag->window_steps = 0;
+    ag->carry_valid = 0;
     return 0;
 }
 

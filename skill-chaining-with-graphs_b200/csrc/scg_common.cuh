@@ -135,6 +135,7 @@ struct scg_ctx {
     float *d_red;        // [SCG_RED_SLICES][K][A*F] second-stage scratch of the slab reduction
     unsigned int *d_tickets;   // one "blocks done" counter per 256-element column of the reduction
     int deterministic;         // 1: fixed-order slab reduction (scg_ctx_set_deterministic)
+    unsigned int *d_apply_ticket;   // "blocks done" counter of k_apply, allocated by the first apply
     float *d_rec;        // records for the standalone scg_sarsa_update, grown on demand
     int rec_capacity;
     cudaEvent_t host_ev; // "results copied" marker of scg_agent_step_host

@@ -771,6 +771,7 @@ extern "C" int scg_ctx_destroy(scg_ctx_t *c) {
     if (c->d_rec) cudaFree(c->d_rec);
     if (c->d_red) cudaFree(c->d_red);
     if (c->d_tickets) cudaFree(c->d_tickets);
+    if (c->d_apply_ticket) cudaFree(c->d_apply_ticket);
     if (c->host_ev) cudaEventDestroy(c->host_ev);
     for (int i = 0; i < 2; ++i) if (c->host_st[i]) cudaStreamDestroy(c->host_st[i]);
     for (int i = 0; i < 2 * SCG_HOST_PARTS_MAX + 1; ++i) if (c->host_evs[i]) cudaEventDestroy(c->host_evs[i]);
@@ -806,40 +807,19 @@ extern "C" int scg_sarsa_update(scg_ctx_t *ctx, int B, const float *x, const flo
     return scg_reduce_window(ctx, n, ctx->K, dW, st);
 }
 
-extern "C" int scg_apply(int order, int K, float *W, float *Wt, float *dW, int *cnt, float alpha, int window_steps,
-                         void *stream) {
-    return scg_apply_top(order, K, K, W, Wt, dW, cnt, alpha, 0.f, window_steps, stream);
-}
-
-extern "C" int scg_apply_top(int order, int K, int K_opt, float *W, float *Wt, float *dW, int *cnt, float alpha,
-                             float alpha_top, int window_steps, void *stream) {
-    if (K < 1 || K > SCG_MAX_OPTIONS) return SCG_ELIMIT;
-    if (!W || !Wt || !dW || !cnt || K_opt < 0 || K_opt > K) return SCG_EINVAL;
+extern "C" int scg_apply(scg_ctx_t *ctx, int K_opt, float *W, float *Wt, float *dW, int *cnt, float alpha,
+                         float alpha_top, int window_steps, void *stream) {
+    if (!ctx || !W || !Wt || !dW || !cnt || K_opt < 0 || K_opt > ctx->K) return SCG_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
     float steps = (float)std::max(window_steps, 1);
-    int F = scg_pow4(order + 1);
-    int grid = scg_grid(K * SCG_A * F, 256, 8);
-    // one "blocks done" counter per (device, stream): launches on one stream are ordered, so the counter (which atomicInc
-    // wraps back to 0) is reusable launch after launch; applies running concurrently on other streams have their own
-    struct Slot { int dev; cudaStream_t st; unsigned int *ticket; };
-    static Slot slots[64];
-    static int n_slots = 0;
-    int dev = 0;
-    SCG_CUDA_OK(cudaGetDevice(&dev));
-    unsigned int *ticket = nullptr;
-    for (int i = 0; i < n_slots; ++i)
-        if (slots[i].dev == dev && slots[i].st == st) ticket = slots[i].ticket;
-    if (!ticket) {
-        if (n_slots >= 64) {           // many short-lived streams: wait for everything, start the table over
-            SCG_CUDA_OK(cudaDeviceSynchronize());
-            for (int i = 0; i < n_slots; ++i) cudaFree(slots[i].ticket);
-            n_slots = 0;
-        }
-        SCG_CUDA_OK(cudaMalloc((void **)&ticket, sizeof(unsigned int)));
-        SCG_CUDA_OK(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), st));
-        slots[n_slots++] = Slot{dev, st, ticket};
+    int grid = scg_grid(ctx->K * SCG_A * ctx->F, 256, 8);
+    // the "blocks done" counter: atomicInc wraps it back to 0, so it serves every (stream-ordered) apply on this context
+    if (!ctx->d_apply_ticket) {
+        SCG_CUDA_OK(cudaMalloc((void **)&ctx->d_apply_ticket, sizeof(unsigned int)));
+        SCG_CUDA_OK(cudaMemsetAsync(ctx->d_apply_ticket, 0, sizeof(unsigned int), st));
     }
-    DISPATCH_ORDER(order, k_apply<N1><<<grid, 256, 0, st>>>(K, K_opt, W, Wt, dW, cnt, alpha, alpha_top, steps, ticket));
+    DISPATCH_ORDER(ctx->order, k_apply<N1><<<grid, 256, 0, st>>>(ctx->K, K_opt, W, Wt, dW, cnt, alpha, alpha_top, steps,
+                                                                 ctx->d_apply_ticket));
     SCG_LAUNCH_CHECK();
     return 0;
 }

@@ -116,12 +116,21 @@ __global__ void __launch_bounds__(XCHG_SLICE, 8) k_sync(const __grid_constant__ 
 }
 
 // ---- host side ------------------------------------------------------------------------------------------
+// the peer wait limit in SM clock cycles of the current device
+static cudaError_t set_timeout_cycles(scg_xchg *x, double seconds) {
+    int dev = 0, khz = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, dev);
+    x->timeout_cycles = (long long)(seconds * 1000.0 * (double)(khz > 0 ? khz : 2000000));
+    return e;
+}
+
 extern "C" int scg_xchg_create(scg_ctx_t *ctx, int rank, int world, scg_xchg_t **out) {
     if (!ctx || !out || world < 1 || world > XCHG_MAX_WORLD || rank < 0 || rank >= world) return SCG_EINVAL;
     if (ctx->K > 16) return SCG_ELIMIT;
     scg_xchg *x = (scg_xchg *)calloc(1, sizeof(scg_xchg));
     if (!x) return SCG_ENOMEM;
-    x->rank = rank; x->world = world; x->K = ctx->K;
+    x->rank = rank; x->world = world; x->order = ctx->order; x->K = ctx->K;
     x->n = ctx->K * SCG_A * ctx->F;
     x->slices = (x->n + XCHG_SLICE - 1) / XCHG_SLICE;
     x->flag_bytes = (((size_t)world * x->slices + 16) * sizeof(uint32_t) + 255) & ~(size_t)255;
@@ -136,10 +145,7 @@ extern "C" int scg_xchg_create(scg_ctx_t *ctx, int rank, int world, scg_xchg_t *
         *x->h_status = 0u;
         e = cudaHostGetDevicePointer((void **)&x->d_status, (void *)x->h_status, 0);
     }
-    int dev = 0, khz = 0;
-    if (e == cudaSuccess) e = cudaGetDevice(&dev);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, dev);
-    x->timeout_cycles = 30ll * 1000ll * (long long)(khz > 0 ? khz : 2000000);
+    if (e == cudaSuccess) e = set_timeout_cycles(x, 30.0);
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         if (x->d_local) cudaFree(x->d_local);
@@ -166,10 +172,7 @@ extern "C" int scg_xchg_destroy(scg_xchg_t *x) {
 
 extern "C" int scg_xchg_set_timeout(scg_xchg_t *x, double seconds) {
     if (!x || !(seconds > 0.0)) return SCG_EINVAL;
-    int dev = 0, khz = 0;
-    SCG_CUDA_OK(cudaGetDevice(&dev));
-    SCG_CUDA_OK(cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, dev));
-    x->timeout_cycles = (long long)(seconds * 1000.0 * (double)(khz > 0 ? khz : 2000000));
+    SCG_CUDA_OK(set_timeout_cycles(x, seconds));
     return 0;
 }
 
@@ -221,21 +224,14 @@ extern "C" int scg_xchg_status(scg_xchg_t *x, int *timed_out) {
 }
 
 // dW (already reduced over this rank's slabs) and cnt -> summed over ranks -> applied; dW and cnt zeroed
-extern "C" int scg_xchg_sync(scg_xchg_t *x, int order, int K, float *W, float *Wt, float *dW, int *cnt, float alpha,
-                             int window_steps, const int *nsucc_local, int *nsucc_global, void *stream) {
-    return scg_xchg_sync_top(x, order, K, K, W, Wt, dW, cnt, alpha, 0.f, window_steps, nsucc_local, nsucc_global, stream);
-}
-
-extern "C" int scg_xchg_sync_top(scg_xchg_t *x, int order, int K, int K_opt, float *W, float *Wt, float *dW, int *cnt,
-                                 float alpha, float alpha_top, int window_steps, const int *nsucc_local,
-                                 int *nsucc_global, void *stream) {
-    if (!x || !W || !Wt || !dW || !cnt || K_opt < 0 || K_opt > K) return SCG_EINVAL;
-    if (K != x->K || K * SCG_A * scg_pow4(order + 1) != x->n) return SCG_EINVAL;
+extern "C" int scg_xchg_sync(scg_xchg_t *x, int K_opt, float *W, float *Wt, float *dW, int *cnt, float alpha,
+                             float alpha_top, int window_steps, const int *nsucc_local, int *nsucc_global, void *stream) {
+    if (!x || !W || !Wt || !dW || !cnt || K_opt < 0 || K_opt > x->K) return SCG_EINVAL;
     for (int r = 0; r < x->world; ++r)
         if (!x->d_peer[r]) return SCG_EINVAL;   // not connected
     if (*x->h_status) return SCG_EPEER;         // an earlier exchange timed out: the replicas are no longer in step
     SyncArgs a;
-    a.n = x->n; a.K = K; a.K_opt = K_opt; a.alpha_top = alpha_top; a.slices = x->slices; a.rank = x->rank; a.world = x->world;
+    a.n = x->n; a.K = x->K; a.K_opt = K_opt; a.alpha_top = alpha_top; a.slices = x->slices; a.rank = x->rank; a.world = x->world;
     a.seq = ++x->seq;
     a.alpha = alpha; a.steps = (float)std::max(window_steps, 1);
     a.W = W; a.Wt = Wt; a.dW = dW; a.cnt = cnt; a.ticket = x->d_ticket;
@@ -244,7 +240,7 @@ extern "C" int scg_xchg_sync_top(scg_xchg_t *x, int order, int K, int K_opt, flo
     a.flag_bytes = x->flag_bytes;
     for (int r = 0; r < XCHG_MAX_WORLD; ++r) a.peer[r] = r < x->world ? x->d_peer[r] : nullptr;
     cudaStream_t st = (cudaStream_t)stream;
-    DISPATCH_ORDER(order, k_sync<N1><<<x->slices, XCHG_SLICE, 0, st>>>(a));
+    DISPATCH_ORDER(x->order, k_sync<N1><<<x->slices, XCHG_SLICE, 0, st>>>(a));
     SCG_LAUNCH_CHECK();
     return 0;
 }

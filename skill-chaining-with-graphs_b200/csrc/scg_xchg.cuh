@@ -8,7 +8,7 @@
 #define XCHG_MAX_WORLD 16
 
 struct scg_xchg {
-    int rank, world, n, K, slices;
+    int rank, world, order, n, K, slices;
     uint32_t seq;
     size_t bytes, flag_bytes;
     // [flags: world*slices u32 | 16 spare u32 | xbuf: 2*slices*XCHG_ROW f32 | controller region, see XCHG_M_*]

@@ -215,9 +215,8 @@ class OptionSet:
         """Fold the window's dW into W (call after any cross-rank allreduce of dW / cnt)."""
         if self._pre_read is not None:
             self._pre_read()
-        check(self.lib.scg_apply_top(self.order, self.K_all, self.K, ptr(self.W), ptr(self.Wt), ptr(self._dW),
-                                     ptr(self._cnt), self.alpha, self.alpha_top, max(self.window_steps, 1),
-                                     _lib.current_stream()))
+        check(self.lib.scg_apply(self._ctx, self.K, ptr(self.W), ptr(self.Wt), ptr(self._dW), ptr(self._cnt), self.alpha,
+                                 self.alpha_top, max(self.window_steps, 1), _lib.current_stream()))
         self.window_steps = 0
         if self._on_weights_changed is not None:
             self._on_weights_changed(applied=True)

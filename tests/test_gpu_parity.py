@@ -1178,7 +1178,7 @@ def test_xchg_single_rank_equals_apply(scg, torch):
     lib = scg.load_library()
     x = C.c_void_p()
     check(lib.scg_xchg_create(b.ctx, 0, 1, C.byref(x)))
-    check(lib.scg_xchg_sync(x, order, K, ptr(b.W), ptr(b.Wt), ptr(b._dW), ptr(b.cnt), 0.07, 4, None, None, current_stream()))
+    check(lib.scg_xchg_sync(x, K, ptr(b.W), ptr(b.Wt), ptr(b._dW), ptr(b.cnt), 0.07, 0.0, 4, None, None, current_stream()))
     torch.cuda.synchronize()
     assert torch.equal(a.W, b.W) and torch.equal(a.Wt, b.Wt)
     assert float(b._dW.abs().max()) == 0.0 and int(b.cnt.sum()) == 0
@@ -1226,7 +1226,7 @@ def test_xchg_two_devices_sum_and_identical_replicas(scg, torch):
         for r in range(2):
             with torch.cuda.device(r):
                 o = sets[r]
-                check(lib.scg_xchg_sync(xs[r], order, K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 8,
+                check(lib.scg_xchg_sync(xs[r], K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 0.0, 8,
                                         ptr(nloc[r]), ptr(nglob[r]), C.c_void_p(torch.cuda.current_stream().cuda_stream)))
         for r in range(2):
             torch.cuda.synchronize(r)
@@ -1297,7 +1297,7 @@ def test_xchg_ranks_on_one_device_sum_and_identical_replicas(scg, torch, world, 
         for it in range(3):                                  # three syncs: double buffering and sequence flags
             for r in range(world):
                 o = sets[r]
-                check(lib.scg_xchg_sync(xs[r], order, K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 8,
+                check(lib.scg_xchg_sync(xs[r], K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 0.0, 8,
                                         ptr(nloc[r]), ptr(nglob[r]), C.c_void_p(streams[r].cuda_stream)))
             torch.cuda.synchronize()
             for r in range(1, world):
@@ -1345,14 +1345,14 @@ def test_xchg_missing_peer_is_fatal_not_silent(scg, torch):
     try:
         check(lib.scg_xchg_set_timeout(xs[0], 0.05))
         o = sets[0]
-        check(lib.scg_xchg_sync(xs[0], order, K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 8, None, None,
+        check(lib.scg_xchg_sync(xs[0], K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 0.0, 8, None, None,
                                 current_stream()))          # rank 1 never calls
         torch.cuda.synchronize()
         t = C.c_int(0)
         check(lib.scg_xchg_status(xs[0], C.byref(t)))
         assert t.value == 1
         assert float((o.W - 0.25).abs().max()) == 0.0 and float((o._dW - 1.0).abs().max()) == 0.0   # nothing applied
-        rc = lib.scg_xchg_sync(xs[0], order, K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 8, None, None,
+        rc = lib.scg_xchg_sync(xs[0], K, ptr(o.W), ptr(o.Wt), ptr(o._dW), ptr(o.cnt), 0.05, 0.0, 8, None, None,
                                current_stream())
         assert rc == -4 and b"peer" in lib.scg_error_string(rc)
     finally:
