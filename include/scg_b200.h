@@ -244,6 +244,25 @@ typedef struct scg_agent {
                                         record (uint32 bits) */
     uint32_t *opt_log;               /* [option_capacity][8] the records */
     int64_t *opt_log_count;          /* [1] executions ever logged; the next one goes to slot opt_log_count % option_capacity */
+    /* trajectory log (optional, same rules: all NULL / 0 = off).  When on, every step of traj_n chosen envs is recorded:
+     * scg_agent_traj gathers the open window's step records (win_rec) and event bytes of those envs into traj_log, at
+     * every flush and whenever the log is read.  The step kernel's only part is to mark episode ends in the event byte
+     * (as with the episode log on).  Records in (step, env) order, traj_n per step, tracked envs in ascending order:
+     *   record i (32 bytes) at slot i % traj_capacity: uint32 step (agent step t: the record is the state at which step
+     *   t began and what happened in it), uint32 env (global env id; 0xFFFFFFFF with a zero payload for a traj_env entry
+     *   outside [0, B)), float x, y, vx, vy (s_t, bit-identical to the agent's state), uint32 action (bits 0-2) |
+     *   option << 8 | 0x10000 term (the option terminated at this step) | 0x20000 label (the example label: hit and
+     *   t_opt <= init_horizon) | 0x40000 episode end | 0x80000 goal (the episode ended at the goal), float delta (this
+     *   step's TD error).
+     * The last traj_capacity records survive.  traj_env, traj_log and traj_log_count are all NULL with traj_n =
+     * traj_capacity = 0, or all set with 1 <= traj_n <= B and traj_capacity > 0. */
+    uint32_t traj_n;                 /* tracked envs; 0: no log */
+    const int32_t *traj_env;         /* [traj_n] local env indices, ascending and distinct, each < B (device) */
+    uint32_t traj_capacity;          /* records in the trajectory log ring (traj_log) */
+    uint32_t *traj_log;              /* [traj_capacity][8] the records */
+    int64_t *traj_log_count;         /* [1] records ever logged; record i sits at slot i % traj_capacity */
+    int32_t traj_len;                /* steps of the open window already gathered (0 .. win_len; host bookkeeping, like
+                                        ring_len: scg_agent_traj sets it to win_len, the flush resets it with win_len) */
 } scg_agent_t;
 
 /* One lock-step agent step.  Updates the struct: swaps (x..vy) with (x2..vy2) so that x..vy is the new
@@ -252,8 +271,14 @@ typedef struct scg_agent {
  * from outside (scg_apply changes the weights: callers clear it after every apply; scg_agent_sync does). */
 int scg_agent_step(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* Fold the open window into dW and the traces (no-op when win_len == 0).  Accepts any K <= SCG_MAX_OPTIONS (16, the
- * top-level slots included) at every order and batch size. */
+ * top-level slots included) at every order and batch size.  With the trajectory log on it first gathers the window's
+ * remaining steps into the log (scg_agent_traj); win_len and traj_len then return to 0. */
 int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
+/* Bring the trajectory log up to date: append the records of the tracked envs for the open window's steps
+ * [traj_len, win_len) to traj_log (one small kernel on `stream`), advance *traj_log_count by traj_n per step, and set
+ * traj_len = win_len.  It does not flush, so calling it between steps leaves every learning result bit for bit as it
+ * would be without the call.  No-op with the log off.  Call it before reading the log. */
+int scg_agent_traj(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* Append the option-termination examples of the recorded, not yet processed steps to the example rings
  * (oracle/agent.py step, item 6).  The step kernel only leaves an event byte and a start position per termination; the
  * rings are brought up to date here - by scg_agent_manage, when the event history is full, or on request - so the pass

@@ -54,6 +54,9 @@ class AgentConfig:
                                   # length, goal; read with episodes()); 0: no log
     option_log: int = 0           # records in the device option log ring (every option execution: step, env, option,
                                   # duration, outcome, start and end; read with option_executions()); 0: no log
+    trajectory_envs: tuple = ()   # local indices of the envs whose every step is logged on the device (state, action,
+                                  # option, TD error, outcome; read with trajectories()); () with trajectory_log = 0: no log
+    trajectory_log: int = 0       # records in the device trajectory log ring (32 bytes each, len(trajectory_envs) per step)
     init_horizon: int = 1 << 30   # an example is positive iff the option hit a target within this many steps of its start
     merge_overlap: float = 0.0    # graph mode: an older option's initiation set becomes a target of the next option iff at
                                   # least this fraction of the promoted option's positive examples lies inside it (0: all)
@@ -152,6 +155,23 @@ class SkillChainAgent:
             self._opt_log_count = torch.zeros(1, dtype=torch.int64, device=dev)
         else:
             self.ev_opt = self._opt_log = self._opt_log_count = None
+        # trajectory log (optional): scg_agent_traj gathers the tracked envs' step records and event bytes of the open
+        # window into _traj_log ([capacity][8], the records of include/scg_b200.h) at every flush and every read
+        envs = sorted(int(b) for b in cfg.trajectory_envs)
+        if int(cfg.trajectory_log) < 0:
+            raise ValueError("trajectory_log must be >= 0")
+        if bool(envs) != bool(cfg.trajectory_log):
+            raise ValueError("trajectory_envs and trajectory_log are set together (both or neither)")
+        if len(set(envs)) != len(envs):
+            raise ValueError("trajectory_envs has duplicates")
+        if envs and not (0 <= envs[0] and envs[-1] < B):
+            raise ValueError(f"trajectory_envs must lie in [0, {B})")
+        if envs:
+            self._traj_env = torch.tensor(envs, **i32)
+            self._traj_log = torch.zeros((int(cfg.trajectory_log), 8), **i32)
+            self._traj_log_count = torch.zeros(1, dtype=torch.int64, device=dev)
+        else:
+            self._traj_env = self._traj_log = self._traj_log_count = None
         # initial state, option and action (oracle/agent.py __init__)
         s = self._sbuf[0]
         if initial_states is not None:
@@ -316,6 +336,21 @@ class SkillChainAgent:
             raise _lib.ScgError("the option log is off: build the agent with AgentConfig(option_log=capacity)")
         return self._read_log(self._opt_log, self._opt_log_count, decode_option_records, since, gather)
 
+    def trajectories(self, since=0, gather=False):
+        """The steps of the tracked envs logged on the device (AgentConfig.trajectory_envs / trajectory_log), brought up
+        to date first (scg_agent_traj gathers the open window's steps without flushing it, so reading does not change
+        what the agent learns): one record per (step, tracked env).  Returns a dict of NumPy arrays in (step, env) order -
+        step (uint32: agent step t; the record is the state at which step t began and what happened in it), env (uint32:
+        global env id), state (float32 (n, 4): s_t, bit-identical to the agent's state), action, option (int32: what
+        was taken at s_t), delta (float32: the step's TD error), term (the option terminated at this step), label (the
+        example label: hit within init_horizon steps), episode_end, goal (the episode ended here, at the goal) (bool) -
+        plus `total`.  `since` and `gather` work as for episodes()."""
+        if self._traj_log is None:
+            raise _lib.ScgError("the trajectory log is off: build the agent with AgentConfig(trajectory_envs=..., "
+                                "trajectory_log=capacity)")
+        check(self.lib.scg_agent_traj(self.options.ctx, C.byref(self._struct), _lib.current_stream()))
+        return self._read_log(self._traj_log, self._traj_log_count, decode_trajectory_records, since, gather)
+
     def _read_log(self, ring, count, decode, since, gather):
         """Records with index >= since still in a device log ring (record i at row i % capacity), decoded, plus `total`;
         with gather=True across a process group, every rank's merged by (step, env)."""
@@ -374,6 +409,10 @@ class SkillChainAgent:
             g.option_capacity = int(cfg.option_log)
             g.ev_opt, g.opt_log, g.opt_log_count = (self.ev_opt.data_ptr(), self._opt_log.data_ptr(),
                                                     self._opt_log_count.data_ptr())
+        if self._traj_log is not None:
+            g.traj_n, g.traj_capacity = len(self._traj_env), int(cfg.trajectory_log)
+            g.traj_env, g.traj_log, g.traj_log_count = (self._traj_env.data_ptr(), self._traj_log.data_ptr(),
+                                                        self._traj_log_count.data_ptr())
         g.trace, g.W, g.Wt, g.theta = o._trace.data_ptr(), o.W.data_ptr(), o.Wt.data_ptr(), o.theta.data_ptr()
         g.dW, g.cnt = o._dW.data_ptr(), o._cnt.data_ptr()
         return g
@@ -644,7 +683,8 @@ class SkillChainAgent:
     def _logs(self):
         """(checkpoint name, ring, count) of each device log that is on."""
         return [(name, ring, count) for name, ring, count in (("ep_log", self._ep_log, self._ep_log_count),
-                                                              ("opt_log", self._opt_log, self._opt_log_count))
+                                                              ("opt_log", self._opt_log, self._opt_log_count),
+                                                              ("traj_log", self._traj_log, self._traj_log_count))
                 if ring is not None]
 
     def save(self, path):
@@ -698,6 +738,7 @@ class SkillChainAgent:
             self._ctl.n_promotions, self._ctl.last_promotion_step = int(z["meta"][4]), int(z["meta"][5])
         self._push_ctl()
         g.step, g.window_steps, g.win_len, g.ring_len, g.ev_len = int(z["meta"][2]), int(z["meta"][3]), 0, 0, 0
+        g.traj_len = 0
         o.window_steps = int(z["meta"][3])
         g.carry_valid = 0
 
@@ -768,8 +809,27 @@ def decode_option_records(rec):
     return out
 
 
+# trajectory-log flag bits of record word 6 (include/scg_b200.h), in bit order from 0x10000
+TRAJECTORY_FLAGS = ("term", "label", "episode_end", "goal")
+
+
+def decode_trajectory_records(rec):
+    """[n][8] int32 trajectory-log records (include/scg_b200.h: step, env, x, y, vx, vy, action | option << 8 | flag
+    bits, delta) -> dict of NumPy arrays step, env (uint32), state (float32 (n, 4)), action, option (int32), delta
+    (float32), term, label, episode_end, goal (bool)."""
+    rec = np.ascontiguousarray(rec, dtype=np.int32).reshape(-1, 8)
+    u = rec.view(np.uint32)
+    w = u[:, 6]
+    out = dict(step=u[:, 0].copy(), env=u[:, 1].copy(), state=rec[:, 2:6].copy().view(np.float32),
+               action=(w & 0x7).astype(np.int32), option=((w >> 8) & 0xFF).astype(np.int32),
+               delta=rec[:, 7].copy().view(np.float32))
+    for i, k in enumerate(TRAJECTORY_FLAGS):
+        out[k] = ((w >> (16 + i)) & 1).astype(bool)
+    return out
+
+
 def merge_episodes(parts):
-    """Merge the episodes() or option_executions() results of several ranks (a list in rank order) into one in
+    """Merge the episodes(), option_executions() or trajectories() results of several ranks (a list in rank order) into one in
     (step, env) order; `total` is the sum of their totals and `totals` the list of them."""
     keys = [k for k in parts[0] if k not in ("total", "totals")]
     cat = {k: np.concatenate([p[k] for p in parts]) for k in keys}

@@ -45,6 +45,7 @@ struct StepArgs {
     float *top;   // this step's slab of the top-level update records: [B][8] (top_slots > 0)
     float2 *ep;   // this step's slab of episode ends (return, length as int bits): [B]; NULL: episode log off
     float4 *opt;  // this step's slab of option terminations (end x, end y, duration bits, record word 2): [B]; NULL: option log off
+    int traj;     // trajectory log on: episode ends are marked in the event byte (SCG_EV_EPEND | SCG_EV_GOAL) as with the episode log
 };
 
 // Q_slot(z, .) for the lanes of `mask` (a warp-uniform ballot), compacted: N1 lanes share one of those envs, one leading
@@ -223,10 +224,10 @@ __global__ void __launch_bounds__(NTH, 512 / NTH) k_agent_step(const __grid_cons
                 }
                 // 7: env reset
                 if (reset) {
-                    if (args.ep != nullptr) {   // episode log: the end (always also a termination) goes into the event
-                        const size_t i = (size_t)s * g.B + b;   // byte, its return and length beside it
+                    if (args.ep != nullptr || args.traj) {   // episode / trajectory log: the end (always also a termination) goes into the
+                        const size_t i = (size_t)s * g.B + b;   // event byte, with the episode log its return and length beside it
                         args.ev[i] |= (uint8_t)(SCG_EV_EPEND | (env_done ? SCG_EV_GOAL : 0u));
-                        args.ep[i] = make_float2(ret, __int_as_float(ep));
+                        if (args.ep != nullptr) args.ep[i] = make_float2(ret, __int_as_float(ep));
                     }
                     const uint4 rr = scg_draw(g.seed, env, step, SCG_STREAM_RESET);
                     const int ns = mh->n_starts;
@@ -411,24 +412,85 @@ static int check_agent(const scg_map_t *map, const scg_ctx_t *ctx, const scg_age
     if (ag->ev_cap < 2 * ag->win_cap || ag->ev_len < ag->win_len || ag->ev_len > ag->ev_cap || ag->ring_len < 0 ||
         ag->ring_len > ag->ev_len)
         return SCG_EINVAL;
-    if (!scg_episode_log_ok(ag) || !scg_option_log_ok(ag)) return SCG_EINVAL;
+    if (!scg_episode_log_ok(ag) || !scg_option_log_ok(ag) || !scg_traj_log_ok(ag)) return SCG_EINVAL;
     if (map->hdr.blob_bytes > 160 * 1024) return SCG_ELIMIT;
+    return 0;
+}
+
+// ---- trajectory log --------------------------------------------------------------------------------
+// k_traj_gather: the tracked envs' records of window steps [s0, s0 + n_steps), copied out of the step records (win_rec)
+// and the event bytes the step kernel left; record r = (step, tracked env) in (step, env) order.  One CTA: it reads the
+// count, every thread writes its records (only the last `cap` of this pass, so every slot has one writer), then one
+// thread advances the count.  It is launched without programmatic serialization and never triggers its dependents, so
+// the next step kernel's griddepcontrol.wait covers all of it before win_rec is rewritten.
+#define TRAJ_NT 1024
+
+__global__ void __launch_bounds__(TRAJ_NT) k_traj_gather(const float4 *__restrict__ rec, const uint8_t *__restrict__ ev,
+                                                         const int32_t *__restrict__ env, int traj_n, int n_steps, int B,
+                                                         uint32_t env_offset, uint32_t step0, uint4 *log,
+                                                         long long *count, uint32_t cap) {
+    const unsigned long long c0 = (unsigned long long)*count;
+    const uint32_t n = (uint32_t)traj_n * (uint32_t)n_steps;
+    const uint32_t first = n > cap ? n - cap : 0u;     // records of this pass that the ring keeps
+#pragma unroll 4
+    for (uint32_t r = first + threadIdx.x; r < n; r += TRAJ_NT) {
+        const uint32_t s = r / (uint32_t)traj_n, j = r - s * (uint32_t)traj_n;
+        const int b = __ldg(env + j);
+        uint4 w0 = make_uint4(step0 + s, 0xFFFFFFFFu, 0u, 0u), w1 = make_uint4(0u, 0u, 0u, 0u);
+        if (b >= 0 && b < B) {
+            const size_t i = (size_t)s * B + b;
+            const float4 st = __ldg(rec + 2 * i), dm = __ldg(rec + 2 * i + 1);
+            const uint32_t meta = __float_as_uint(dm.y), e = __ldg(ev + i);
+            const uint32_t word = (meta & 7u) | (((meta >> 8) & 0xFFu) << 8) | ((meta & SCG_META_ZERO_AFTER) ? SCG_TL_TERM : 0u) |
+                                  ((e & SCG_EV_HIT) ? SCG_TL_LABEL : 0u) | ((e & SCG_EV_EPEND) ? SCG_TL_EPEND : 0u) |
+                                  ((e & SCG_EV_GOAL) ? SCG_TL_GOAL : 0u);
+            w0 = make_uint4(step0 + s, env_offset + (uint32_t)b, __float_as_uint(st.x), __float_as_uint(st.y));
+            w1 = make_uint4(__float_as_uint(st.z), __float_as_uint(st.w), word, __float_as_uint(dm.x));
+        }
+        const size_t slot = (size_t)((c0 + r) % cap);
+        log[2 * slot] = w0;
+        log[2 * slot + 1] = w1;
+    }
+    __syncthreads();                                    // every thread has read the count
+    if (threadIdx.x == 0) *count = (long long)(c0 + n);
+}
+
+extern "C" int scg_agent_traj(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
+    if (!ctx || !ag || !scg_traj_log_ok(ag)) return SCG_EINVAL;
+    if (!ag->traj_log) return 0;
+    if (ag->win_len > ag->win_cap || ag->ev_len < ag->win_len || ag->ev_len > ag->ev_cap || !ag->win_rec || !ag->ev_hist)
+        return SCG_EINVAL;
+    const int n = ag->win_len - ag->traj_len;
+    if (n > 0) {
+        // window step s is history row ev_len - win_len + s (as k_top reads it); the ring pass only recycles rows
+        // between windows
+        const size_t s0 = (size_t)ag->traj_len;
+        const size_t row = (size_t)(ag->ev_len - ag->win_len) + s0;
+        k_traj_gather<<<1, TRAJ_NT, 0, (cudaStream_t)stream>>>(
+            reinterpret_cast<const float4 *>(ag->win_rec) + s0 * ag->B * 2, ag->ev_hist + row * ag->B, ag->traj_env,
+            (int)ag->traj_n, n, ag->B, ag->env_offset, ag->step - (uint32_t)ag->win_len + (uint32_t)ag->traj_len,
+            reinterpret_cast<uint4 *>(ag->traj_log), reinterpret_cast<long long *>(ag->traj_log_count), ag->traj_capacity);
+        SCG_LAUNCH_CHECK();
+    }
+    ag->traj_len = ag->win_len;
     return 0;
 }
 
 extern "C" int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
     if (!ctx || !ag) return SCG_EINVAL;
-    if (ag->win_len <= 0 || ag->B <= 0) { ag->win_len = 0; return 0; }
+    int rc;
+    // the trajectory log takes the window's last steps before anything else reads or recycles the window
+    if ((rc = scg_agent_traj(ctx, ag, stream))) return rc;
+    if (ag->win_len <= 0 || ag->B <= 0) { ag->win_len = ag->traj_len = 0; return 0; }
     // option ids in the records are 0 .. n_active (the gestating slot); n_active is the host's lower bound of the
     // device's value: records of an option promoted since then are folded through the sweep's global-memory path
     const int k_used = std::min(ag->K, std::max(ag->n_active, 0) + 1);
-    int rc;
     if ((rc = scg_launch_top(ctx, ag, (cudaStream_t)stream))) return rc;     // the top-level learner's SMDP updates
     const int n_slabs = scg_launch_window(ctx, ag->B, ag->win_len, k_used, ag->win_rec, ag->trace, ag->gamma * ag->lambda,
                                           ag->dW, (cudaStream_t)stream);
     if (n_slabs <= 0) return n_slabs == 0 ? SCG_EINVAL : n_slabs;
     if ((rc = scg_reduce_window(ctx, n_slabs, k_used, ag->dW, (cudaStream_t)stream))) return rc;
-    ag->win_len = 0;
+    ag->win_len = ag->traj_len = 0;
     // the event history must have room for the next full window: when it has not, bring the rings up to date now
     if (ag->ev_len + ag->win_cap > ag->ev_cap && (rc = scg_agent_ring(ctx, ag, stream))) return rc;
     return 0;
@@ -457,6 +519,7 @@ static int agent_steps(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, in
     args.top = ag->win_top ? ag->win_top + (size_t)ag->win_len * ag->B * 8 : nullptr;
     args.ep = ag->ev_ep ? reinterpret_cast<float2 *>(ag->ev_ep) + (size_t)ag->ev_len * ag->B : nullptr;
     args.opt = ag->ev_opt ? reinterpret_cast<float4 *>(ag->ev_opt) + (size_t)ag->ev_len * ag->B : nullptr;
+    args.traj = ag->traj_log != nullptr;
     args.n_steps = n;
     args.b_begin = b_begin;
     args.b_end = b_end;

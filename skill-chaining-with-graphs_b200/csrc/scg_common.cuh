@@ -18,8 +18,8 @@
 #define SCG_EV_TERM 0x80u   // the option terminated at this step
 #define SCG_EV_HIT 0x40u    // ... by reaching one of its targets (label 1), else label 0
 #define SCG_EV_OPT 0x0Fu    // option id
-// episode log on (scg_agent_t::ev_ep set): an episode ended at this step (always also TERM), with its return and length
-// in the ev_ep plane; GOAL: it ended at the goal, else it timed out
+// episode or trajectory log on (scg_agent_t::ev_ep or traj_log set): an episode ended at this step (always also TERM);
+// GOAL: it ended at the goal, else it timed out.  With the episode log on its return and length are in the ev_ep plane
 #define SCG_EV_EPEND 0x20u
 #define SCG_EV_GOAL 0x10u
 // option log on (scg_agent_t::ev_opt set): outcome bits of word 2 of a record (option id in bits 0-3), include/scg_b200.h
@@ -29,6 +29,11 @@
 #define SCG_OL_OPTION_TIMEOUT 0x800u
 #define SCG_OL_LEFT 0x1000u
 #define SCG_OL_EPISODE_TIMEOUT 0x2000u
+// trajectory log on (scg_agent_t::traj_log set): flag bits of word 6 of a record (action in bits 0-2, option << 8)
+#define SCG_TL_TERM 0x10000u
+#define SCG_TL_LABEL 0x20000u
+#define SCG_TL_EPEND 0x40000u
+#define SCG_TL_GOAL 0x80000u
 
 extern uint64_t g_scg_launches;  // host-side launch counter (scg_api.cu)
 
@@ -619,4 +624,13 @@ static inline bool scg_episode_log_ok(const scg_agent_t *ag) {
 static inline bool scg_option_log_ok(const scg_agent_t *ag) {
     if (!ag->ev_opt && !ag->opt_log && !ag->opt_log_count && ag->option_capacity == 0) return true;
     return ag->ev_opt && ag->opt_log && ag->opt_log_count && ag->option_capacity > 0;
+}
+
+// the trajectory log's fields: all off (NULL / 0), or the tracked envs (1 .. B of them), the log ring, its count and a
+// capacity all set; traj_len counts gathered steps of the open window
+static inline bool scg_traj_log_ok(const scg_agent_t *ag) {
+    if (!ag->traj_env && !ag->traj_log && !ag->traj_log_count && ag->traj_n == 0 && ag->traj_capacity == 0)
+        return ag->traj_len == 0;
+    return ag->traj_env && ag->traj_log && ag->traj_log_count && ag->traj_n >= 1 && ag->traj_n <= (uint32_t)ag->B &&
+           ag->B > 0 && ag->traj_capacity > 0 && ag->traj_len >= 0 && ag->traj_len <= ag->win_len;
 }

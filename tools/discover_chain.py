@@ -24,6 +24,10 @@ run's clocks (--budget, --train-seconds, wall_s and the promotion times) leave t
 steps in the same clock time as an unlogged one, up to the overlap of host and device work that each poll's wait gives
 up and the example-ring pass that each poll runs in place of the next manage().  The time the polls took is reported
 as option_poll_s.
+With --draw PATH the greedy evaluation after discovery also logs the trajectories of its first --draw-envs envs
+(AgentConfig.trajectory_envs) and the script writes PATH, an SVG of the map, each active option's initiation set (64 x 64
+positions at zero velocity) and those greedy paths coloured by the running option (tools/chain_svg.py); the final JSON
+names it as "drawing".
 """
 import argparse
 import json
@@ -38,12 +42,15 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from learning_curve import OptionTally  # noqa: E402
 
 
-def evaluate(scg, torch, base_map, src, args, n_env=4096, trained=True):
-    """Greedy episodes from the map's own start with (a copy of) the agent's weights, classifiers and option graph."""
+def evaluate(scg, torch, base_map, src, args, n_env=4096, trained=True, draw=None):
+    """Greedy episodes from the map's own start with (a copy of) the agent's weights, classifiers and option graph.
+    draw: SVG path - the first args.draw_envs envs' trajectories and the initiation sets are drawn there."""
+    traj = dict(trajectory_envs=tuple(range(min(args.draw_envs, n_env))),
+                trajectory_log=min(args.draw_envs, n_env) * (args.max_episode_steps + 64)) if draw else {}
     cfg = scg.AgentConfig(map=args.map, batch=n_env, order=args.order, max_options=args.options, gamma=0.99, lam=0.9,
                           alpha=0.0, epsilon=0.0, sync_interval=8, option_timeout=args.option_timeout,
                           max_episode_steps=args.max_episode_steps, gestation_successes=1 << 30, graph=args.graph,
-                          top_level=not args.no_top_level, alpha_top=0.0, epsilon_top=0.0, seed=123)
+                          top_level=not args.no_top_level, alpha_top=0.0, epsilon_top=0.0, seed=123, **traj)
     ev = scg.SkillChainAgent(cfg, base_map)
     if trained:
         ev.options.set_weights(src.options.W)
@@ -54,6 +61,13 @@ def evaluate(scg, torch, base_map, src, args, n_env=4096, trained=True):
         ev._push_ctl()
     st = ev.run_episode(max_steps=args.max_episode_steps, manage_every=64)
     goals = int(ev.stats[1])
+    if draw:
+        from chain_svg import initiation_grid, render
+        c = ev.controller_state(sync=True)
+        grid = initiation_grid(ev.options, c["active_mask"])
+        with open(draw, "w") as f:
+            f.write(render(base_map, ev.trajectories(), init_grid=grid,
+                           title=f"{args.map} map: {c['n_active']} active options, greedy paths of {args.draw_envs} envs"))
     return dict(success_rate=goals / n_env, finished=st["finished"], mean_return=st["mean_return"], steps=st["steps"])
 
 
@@ -79,6 +93,8 @@ def main():
     ap.add_argument("--min-chain", type=int, default=3)
     ap.add_argument("--option-log", type=int, default=0, metavar="CAP",
                     help="log every option execution (ring of CAP records, polled every chunk) and report per-option totals")
+    ap.add_argument("--draw", default=None, metavar="PATH", help="write an SVG of the chain and the greedy paths here")
+    ap.add_argument("--draw-envs", type=int, default=32, help="greedy envs whose paths are drawn")
     args = ap.parse_args()
     import torch
     import skill_chaining_with_graphs_b200 as scg
@@ -154,7 +170,7 @@ def main():
     # how much of the free space each initiation set covers, and whether it contains the map's start
     probe = torch.as_tensor(base.sample_free_states(np.random.default_rng(1), 20000)).cuda()
     inside = ag.options.initiation(probe)[:, :c["n_active"]].float().mean(dim=0).cpu().numpy().tolist() if c["n_active"] else []
-    after = evaluate(scg, torch, base, ag, args, trained=True)
+    after = evaluate(scg, torch, base, ag, args, trained=True, draw=args.draw)
     options = {}
     if tally is not None:
         poll_options()
@@ -166,7 +182,8 @@ def main():
                           initiation_set_fraction_of_free_space=[round(v, 3) for v in inside],
                           goals=cnt["goals"], episodes=cnt["episodes"], mean_return=cnt["mean_return"],
                           n_success=cnt["n_success"].tolist(), promotions=log,
-                          greedy_from_start_untrained=before, greedy_from_start_after_discovery=after, **options)))
+                          greedy_from_start_untrained=before, greedy_from_start_after_discovery=after, **options,
+                          **(dict(drawing=args.draw) if args.draw else {}))))
 
 
 if __name__ == "__main__":
