@@ -1022,7 +1022,7 @@ def test_windowed_sweep_equals_oracle_dense_traces(scg, torch, order, K, window,
     gag.win_rec = torch.zeros((window, B, 8), dtype=torch.float32, device="cuda")
     gag._struct.win_rec = gag.win_rec.data_ptr()
     gag._struct.win_cap = window
-    n_steps = min(window, 12)
+    n_steps = window
     for t in range(n_steps):
         out = oag.step()
         gag.step()
