@@ -263,6 +263,20 @@ typedef struct scg_agent {
     int64_t *traj_log_count;         /* [1] records ever logged; record i sits at slot i % traj_capacity */
     int32_t traj_len;                /* steps of the open window already gathered (0 .. win_len; host bookkeeping, like
                                         ring_len: scg_agent_traj sets it to win_len, the flush resets it with win_len) */
+    /* occupancy grid (optional: occ_grid = 0 and occ_counts = NULL = off, and the kernels do exactly the work they do
+     * without it).  When on, every env-step of every env is counted by the option running during it and the map cell
+     * of the state at which it began: scg_agent_occupancy adds the open window's step records (win_rec) to occ_counts,
+     * at every flush and whenever the grid is read.  The step kernel has no part in it.  Step t of env b adds 1 to
+     *   occ_counts[o][iy][ix], o = the record's option (slots 0 .. K-1, the gestating one included; the top-level
+     *   learner's weight slots have no cell), ix = min(max((int)(x * occ_grid), 0), occ_grid - 1) with x the fp32 x of
+     *   s_t and the conversion truncating toward zero, iy likewise from y.
+     * occ_grid is a power of two in 1 .. 128, so x * occ_grid is exact in fp32.  Counts are cumulative (subtract two
+     * reads for an interval), and integer adds make them the same whatever the order of the adds.  occ_counts is NULL
+     * iff occ_grid == 0. */
+    uint32_t occ_grid;               /* cells per side of the unit square; 0: no grid */
+    uint64_t *occ_counts;            /* [K][occ_grid][occ_grid] env-steps per (option, cell) (device) */
+    int32_t occ_len;                 /* steps of the open window already counted (0 .. win_len; host bookkeeping, like
+                                        traj_len: scg_agent_occupancy sets it to win_len, the flush resets it with win_len) */
 } scg_agent_t;
 
 /* One lock-step agent step.  Updates the struct: swaps (x..vy) with (x2..vy2) so that x..vy is the new
@@ -272,13 +286,19 @@ typedef struct scg_agent {
 int scg_agent_step(const scg_map_t *map, scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* Fold the open window into dW and the traces (no-op when win_len == 0).  Accepts any K <= SCG_MAX_OPTIONS (16, the
  * top-level slots included) at every order and batch size.  With the trajectory log on it first gathers the window's
- * remaining steps into the log (scg_agent_traj); win_len and traj_len then return to 0. */
+ * remaining steps into the log (scg_agent_traj), and with the occupancy grid on counts them (scg_agent_occupancy);
+ * win_len, traj_len and occ_len then return to 0. */
 int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* Bring the trajectory log up to date: append the records of the tracked envs for the open window's steps
  * [traj_len, win_len) to traj_log (one small kernel on `stream`), advance *traj_log_count by traj_n per step, and set
  * traj_len = win_len.  It does not flush, so calling it between steps leaves every learning result bit for bit as it
  * would be without the call.  No-op with the log off.  Call it before reading the log. */
 int scg_agent_traj(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
+/* Bring the occupancy grid up to date: add the open window's steps [occ_len, win_len) of all B envs to occ_counts (one
+ * kernel on `stream`: per-CTA shared-memory bins, then integer adds to occ_counts) and set occ_len = win_len.  It does not flush, so calling it
+ * between steps leaves every learning result bit for bit as it would be without the call.  No-op with the grid off.
+ * Call it before reading the grid. */
+int scg_agent_occupancy(scg_ctx_t *ctx, scg_agent_t *ag, void *stream);
 /* Append the option-termination examples of the recorded, not yet processed steps to the example rings
  * (oracle/agent.py step, item 6).  The step kernel only leaves an event byte and a start position per termination; the
  * rings are brought up to date here - by scg_agent_manage, when the event history is full, or on request - so the pass

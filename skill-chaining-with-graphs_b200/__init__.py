@@ -15,7 +15,8 @@ operator raises if libscg_b200.so or a CUDA device is missing.
 from ._lib import LIB_PATH, EXPORTS, ScgError, load as load_library
 from .pinball import PinballMap, PinballEnv, unpack_flags
 from .option import FourierBasis, OptionSet, Option
-from .agent import SkillChainAgent, AgentConfig, merge_episodes
+from .agent import SkillChainAgent, AgentConfig, merge_episodes, merge_occupancy
 
 __all__ = ["LIB_PATH", "EXPORTS", "ScgError", "load_library", "PinballMap", "PinballEnv", "unpack_flags",
-           "FourierBasis", "OptionSet", "Option", "SkillChainAgent", "AgentConfig", "merge_episodes"]
+           "FourierBasis", "OptionSet", "Option", "SkillChainAgent", "AgentConfig", "merge_episodes",
+           "merge_occupancy"]

@@ -59,6 +59,7 @@ class AgentStruct(C.Structure):
         ("option_capacity", C.c_uint32), ("ev_opt", C.c_void_p), ("opt_log", C.c_void_p), ("opt_log_count", C.c_void_p),
         ("traj_n", C.c_uint32), ("traj_env", C.c_void_p), ("traj_capacity", C.c_uint32), ("traj_log", C.c_void_p),
         ("traj_log_count", C.c_void_p), ("traj_len", C.c_int32),
+        ("occ_grid", C.c_uint32), ("occ_counts", C.c_void_p), ("occ_len", C.c_int32),
     ]
 
 
@@ -96,6 +97,7 @@ _SIGS = {
     "scg_agent_flush": (C.c_int, [_P, C.POINTER(AgentStruct), _P]),
     "scg_agent_ring": (C.c_int, [_P, C.POINTER(AgentStruct), _P]),
     "scg_agent_traj": (C.c_int, [_P, C.POINTER(AgentStruct), _P]),
+    "scg_agent_occupancy": (C.c_int, [_P, C.POINTER(AgentStruct), _P]),
     "scg_agent_manage": (C.c_int, [_P, C.POINTER(AgentStruct), _P, _P]),
     "scg_agent_poll": (C.c_int, [_P, C.POINTER(CtlStruct)]),
     "scg_agent_set_ctl": (C.c_int, [_P, C.POINTER(AgentStruct), C.POINTER(CtlStruct), _P]),

@@ -57,6 +57,8 @@ class AgentConfig:
     trajectory_envs: tuple = ()   # local indices of the envs whose every step is logged on the device (state, action,
                                   # option, TD error, outcome; read with trajectories()); () with trajectory_log = 0: no log
     trajectory_log: int = 0       # records in the device trajectory log ring (32 bytes each, len(trajectory_envs) per step)
+    occupancy_grid: int = 0       # G: every env-step counted on the device by (option, cell of a G x G grid over the map);
+                                  # read with occupancy().  A power of two in 1..128; 0: no grid
     init_horizon: int = 1 << 30   # an example is positive iff the option hit a target within this many steps of its start
     merge_overlap: float = 0.0    # graph mode: an older option's initiation set becomes a target of the next option iff at
                                   # least this fraction of the promoted option's positive examples lies inside it (0: all)
@@ -69,6 +71,19 @@ class AgentConfig:
     alpha_top: float = 1e-3
     epsilon_top: float = 0.05
     sync_timeout_s: float = 30.0   # how long a peer-memory exchange waits for the other ranks before failing (ScgError)
+
+    def __post_init__(self):
+        occupancy_grid_size(self.occupancy_grid)
+
+
+OCCUPANCY_GRID_MAX = 128
+
+
+def occupancy_grid_size(g):
+    """AgentConfig.occupancy_grid as an int: 0 (off) or a power of two in 1..OCCUPANCY_GRID_MAX; else ValueError."""
+    if isinstance(g, bool) or int(g) != g or not (g == 0 or (1 <= g <= OCCUPANCY_GRID_MAX and int(g) & (int(g) - 1) == 0)):
+        raise ValueError(f"occupancy_grid must be 0 (off) or a power of two in 1..{OCCUPANCY_GRID_MAX}, not {g!r}")
+    return int(g)
 
 
 class SkillChainAgent:
@@ -172,6 +187,10 @@ class SkillChainAgent:
             self._traj_log_count = torch.zeros(1, dtype=torch.int64, device=dev)
         else:
             self._traj_env = self._traj_log = self._traj_log_count = None
+        # occupancy grid (optional): scg_agent_occupancy adds every env-step of the open window to _occ ([K][G][G]
+        # uint64 counts held as int64, indexed [option, iy, ix]) at every flush and every read
+        G = occupancy_grid_size(cfg.occupancy_grid)
+        self._occ = torch.zeros((K, G, G), dtype=torch.int64, device=dev) if G else None
         # initial state, option and action (oracle/agent.py __init__)
         s = self._sbuf[0]
         if initial_states is not None:
@@ -351,6 +370,26 @@ class SkillChainAgent:
         check(self.lib.scg_agent_traj(self.options.ctx, C.byref(self._struct), _lib.current_stream()))
         return self._read_log(self._traj_log, self._traj_log_count, decode_trajectory_records, since, gather)
 
+    def occupancy(self, gather=False):
+        """The occupancy grid (AgentConfig.occupancy_grid = G), brought up to date first (scg_agent_occupancy counts the
+        open window's steps without flushing it, so reading does not change what the agent learns).  Every env-step
+        since the agent was built adds 1 to the cell of the option running during it and of the state at which it began:
+        cell i = min(max(int(x * G), 0), G - 1) along x, likewise along y.  Returns dict(counts=uint64 (K, G, G) indexed
+        [option, iy, ix], grid=G, env_steps=counts.sum()).  Counts are cumulative: subtract two reads for an interval.
+        gather=True (several ranks): the counts summed over the process group, plus per_rank, each rank's env_steps."""
+        if self._occ is None:
+            raise _lib.ScgError("the occupancy grid is off: build the agent with AgentConfig(occupancy_grid=G)")
+        check(self.lib.scg_agent_occupancy(self.options.ctx, C.byref(self._struct), _lib.current_stream()))
+        counts = self._occ.cpu().numpy().view(np.uint64)
+        out = dict(counts=counts, grid=int(counts.shape[1]), env_steps=int(counts.sum()))
+        if not gather:
+            return out
+        parts = [out]
+        if world_size(self.pg) > 1:
+            parts = [None] * world_size(self.pg)
+            self.torch.distributed.all_gather_object(parts, out, group=self.pg)
+        return merge_occupancy(parts)
+
     def _read_log(self, ring, count, decode, since, gather):
         """Records with index >= since still in a device log ring (record i at row i % capacity), decoded, plus `total`;
         with gather=True across a process group, every rank's merged by (step, env)."""
@@ -413,6 +452,8 @@ class SkillChainAgent:
             g.traj_n, g.traj_capacity = len(self._traj_env), int(cfg.trajectory_log)
             g.traj_env, g.traj_log, g.traj_log_count = (self._traj_env.data_ptr(), self._traj_log.data_ptr(),
                                                         self._traj_log_count.data_ptr())
+        if self._occ is not None:
+            g.occ_grid, g.occ_counts = int(self._occ.shape[1]), self._occ.data_ptr()
         g.trace, g.W, g.Wt, g.theta = o._trace.data_ptr(), o.W.data_ptr(), o.Wt.data_ptr(), o.theta.data_ptr()
         g.dW, g.cnt = o._dW.data_ptr(), o._cnt.data_ptr()
         return g
@@ -697,6 +738,8 @@ class SkillChainAgent:
         arrs = {k.lstrip("_"): getattr(self, k).cpu().numpy() for k in self._CKPT_TENSORS}
         for name, ring, count in self._logs():
             arrs.update({name: ring.cpu().numpy(), name + "_count": count.cpu().numpy()})
+        if self._occ is not None:
+            arrs["occ_counts"] = self._occ.cpu().numpy()
         arrs.update(W=o.W.cpu().numpy(), theta=o.theta.cpu().numpy(), trace=o._trace.cpu().numpy(),
                     dW=o._dW.cpu().numpy(), cnt=o._cnt.cpu().numpy(), state=self.s.cpu().numpy(),
                     parents=np.array(c["parents"], dtype=np.uint32),
@@ -711,6 +754,9 @@ class SkillChainAgent:
         o, g = self.options, self._struct
         if tuple(z["W"].shape) != tuple(o.W.shape) or z["state"].shape != tuple(self.s.shape):
             raise ValueError("checkpoint does not match this agent's configuration")
+        if self._occ is not None and "occ_counts" in z.files and z["occ_counts"].shape != tuple(self._occ.shape):
+            raise ValueError(f"checkpoint occupancy grid {z['occ_counts'].shape} does not match this agent's "
+                             f"{tuple(self._occ.shape)}")
         self.flush()
         for k in self._CKPT_TENSORS:
             getattr(self, k).copy_(torch.as_tensor(z[k.lstrip("_")]))
@@ -730,6 +776,11 @@ class SkillChainAgent:
                 log[idx % len(log)] = old[idx % len(old)]
             ring.copy_(torch.as_tensor(log))
             count.fill_(total)
+        if self._occ is not None:                  # (a checkpoint without a grid resumes with zeros)
+            if "occ_counts" in z.files:
+                self._occ.copy_(torch.as_tensor(z["occ_counts"]))
+            else:
+                self._occ.zero_()
         self.torch.cuda.current_stream().synchronize()
         self._poll()
         self.parents_host[:] = z["parents"]
@@ -738,7 +789,7 @@ class SkillChainAgent:
             self._ctl.n_promotions, self._ctl.last_promotion_step = int(z["meta"][4]), int(z["meta"][5])
         self._push_ctl()
         g.step, g.window_steps, g.win_len, g.ring_len, g.ev_len = int(z["meta"][2]), int(z["meta"][3]), 0, 0, 0
-        g.traj_len = 0
+        g.traj_len = g.occ_len = 0
         o.window_steps = int(z["meta"][3])
         g.carry_valid = 0
 
@@ -838,3 +889,11 @@ def merge_episodes(parts):
     out["totals"] = [int(p["total"]) for p in parts]
     out["total"] = sum(out["totals"])
     return out
+
+
+def merge_occupancy(parts):
+    """Merge the occupancy() results of several ranks (a list in rank order): the counts summed, env_steps their total
+    and per_rank each rank's env_steps."""
+    counts = np.sum([p["counts"] for p in parts], axis=0, dtype=np.uint64)
+    return dict(counts=counts, grid=int(parts[0]["grid"]), env_steps=int(counts.sum()),
+                per_rank=[int(p["env_steps"]) for p in parts])

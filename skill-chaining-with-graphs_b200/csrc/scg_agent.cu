@@ -412,7 +412,8 @@ static int check_agent(const scg_map_t *map, const scg_ctx_t *ctx, const scg_age
     if (ag->ev_cap < 2 * ag->win_cap || ag->ev_len < ag->win_len || ag->ev_len > ag->ev_cap || ag->ring_len < 0 ||
         ag->ring_len > ag->ev_len)
         return SCG_EINVAL;
-    if (!scg_episode_log_ok(ag) || !scg_option_log_ok(ag) || !scg_traj_log_ok(ag)) return SCG_EINVAL;
+    if (!scg_episode_log_ok(ag) || !scg_option_log_ok(ag) || !scg_traj_log_ok(ag) || !scg_occupancy_ok(ag))
+        return SCG_EINVAL;
     if (map->hdr.blob_bytes > 160 * 1024) return SCG_ELIMIT;
     return 0;
 }
@@ -476,12 +477,75 @@ extern "C" int scg_agent_traj(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
     return 0;
 }
 
+// ---- occupancy grid --------------------------------------------------------------------------------
+// k_occupancy: the step records of window steps [s0, s0 + n_steps) of all B envs, n = n_steps * B of them back to back
+// in win_rec.  A record's option (meta word) and the cell of its (x, y) give its bin, key = (option * grid + iy) * grid
+// + ix.  Many envs share a few cells (around the start positions, along walls), so one global atomic per record
+// serialises on those addresses: each CTA counts its OCC_REC_PER_CTA records in 32-bit shared-memory bins, then adds
+// its non-zero bins to the global counts (red.global.add.u64), at most one add per bin and CTA.  Bins beyond the shared
+// memory of one CTA are split into chunks along blockIdx.y; a CTA counts the records whose key falls into its chunk.
+// Integer adds make the counts independent of the order of the adds.  Launched like k_traj_gather: no programmatic
+// serialization and no trigger, so the next step kernel's griddepcontrol.wait covers all of it before win_rec is
+// rewritten.
+#define OCC_NT 512
+#define OCC_REC_PER_CTA 4096            // records per CTA: < 2^32, so the shared counters cannot overflow
+#define OCC_SMEM_BINS 16384             // 64 KiB of shared counters per CTA
+
+__global__ void __launch_bounds__(OCC_NT) k_occupancy(const float4 *__restrict__ rec, size_t n, int K, int grid,
+                                                       int chunk_bins, unsigned long long *counts) {
+    extern __shared__ uint32_t bins[];
+    const int n_bins = K * grid * grid, lo = (int)blockIdx.y * chunk_bins;
+    const int hi = min(lo + chunk_bins, n_bins);
+    for (int j = threadIdx.x; j < hi - lo; j += OCC_NT) bins[j] = 0u;
+    __syncthreads();
+    const size_t end = min(n, (size_t)(blockIdx.x + 1) * OCC_REC_PER_CTA);
+    for (size_t i = (size_t)blockIdx.x * OCC_REC_PER_CTA + threadIdx.x; i < end; i += OCC_NT) {
+        const float2 xy = __ldg(reinterpret_cast<const float2 *>(rec + 2 * i));
+        const uint32_t o = (__float_as_uint(__ldg(reinterpret_cast<const float *>(rec + 2 * i + 1) + 1)) >> 8) & 0xFFu;
+        if (o >= (uint32_t)K) continue;
+        // grid is a power of two: x * grid is exact, and the conversion truncates toward zero (include/scg_b200.h)
+        const int ix = min(max(__float2int_rz(__fmul_rn(xy.x, (float)grid)), 0), grid - 1);
+        const int iy = min(max(__float2int_rz(__fmul_rn(xy.y, (float)grid)), 0), grid - 1);
+        const int key = ((int)o * grid + iy) * grid + ix;
+        if (key >= lo && key < hi) atomicAdd(bins + (key - lo), 1u);
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < hi - lo; j += OCC_NT) {
+        const uint32_t v = bins[j];
+        if (v) atomicAdd(counts + lo + j, (unsigned long long)v);
+    }
+}
+
+extern "C" int scg_agent_occupancy(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
+    if (!ctx || !ag || !scg_occupancy_ok(ag)) return SCG_EINVAL;
+    if (!ag->occ_counts) return 0;
+    if (ag->win_len > ag->win_cap || ag->B < 0 || ag->K < 1 || ag->K > SCG_MAX_OPTIONS || !ag->win_rec) return SCG_EINVAL;
+    const int n = ag->win_len - ag->occ_len;
+    if (n > 0 && ag->B > 0) {
+        static ScgKernelCfg cfgc = {};
+        int per_sm, rc;
+        if ((rc = scg_configure(cfgc, k_occupancy, OCC_NT, OCC_SMEM_BINS * sizeof(uint32_t), &per_sm))) return rc;
+        const int grid = (int)ag->occ_grid, n_bins = ag->K * grid * grid;
+        const int chunk_bins = std::min(n_bins, OCC_SMEM_BINS);
+        const size_t s0 = (size_t)ag->occ_len, m = (size_t)n * ag->B;
+        const dim3 blocks((unsigned)((m + OCC_REC_PER_CTA - 1) / OCC_REC_PER_CTA), (unsigned)((n_bins + chunk_bins - 1) / chunk_bins));
+        k_occupancy<<<blocks, OCC_NT, chunk_bins * sizeof(uint32_t), (cudaStream_t)stream>>>(
+            reinterpret_cast<const float4 *>(ag->win_rec) + s0 * ag->B * 2, m, ag->K, grid, chunk_bins,
+            reinterpret_cast<unsigned long long *>(ag->occ_counts));
+        SCG_LAUNCH_CHECK();
+    }
+    ag->occ_len = ag->win_len;
+    return 0;
+}
+
 extern "C" int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
     if (!ctx || !ag) return SCG_EINVAL;
     int rc;
-    // the trajectory log takes the window's last steps before anything else reads or recycles the window
+    // the trajectory log and the occupancy grid take the window's last steps before anything else reads or recycles
+    // the window
     if ((rc = scg_agent_traj(ctx, ag, stream))) return rc;
-    if (ag->win_len <= 0 || ag->B <= 0) { ag->win_len = ag->traj_len = 0; return 0; }
+    if ((rc = scg_agent_occupancy(ctx, ag, stream))) return rc;
+    if (ag->win_len <= 0 || ag->B <= 0) { ag->win_len = ag->traj_len = ag->occ_len = 0; return 0; }
     // option ids in the records are 0 .. n_active (the gestating slot); n_active is the host's lower bound of the
     // device's value: records of an option promoted since then are folded through the sweep's global-memory path
     const int k_used = std::min(ag->K, std::max(ag->n_active, 0) + 1);
@@ -490,7 +554,7 @@ extern "C" int scg_agent_flush(scg_ctx_t *ctx, scg_agent_t *ag, void *stream) {
                                           ag->dW, (cudaStream_t)stream);
     if (n_slabs <= 0) return n_slabs == 0 ? SCG_EINVAL : n_slabs;
     if ((rc = scg_reduce_window(ctx, n_slabs, k_used, ag->dW, (cudaStream_t)stream))) return rc;
-    ag->win_len = ag->traj_len = 0;
+    ag->win_len = ag->traj_len = ag->occ_len = 0;
     // the event history must have room for the next full window: when it has not, bring the rings up to date now
     if (ag->ev_len + ag->win_cap > ag->ev_cap && (rc = scg_agent_ring(ctx, ag, stream))) return rc;
     return 0;

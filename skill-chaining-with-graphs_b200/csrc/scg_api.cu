@@ -21,6 +21,6 @@ extern "C" const char *scg_error_string(int code) {
     return "scg: unknown error";
 }
 
-extern "C" int scg_version(void) { return 221; }
+extern "C" int scg_version(void) { return 222; }
 
 extern "C" uint64_t scg_launch_count(void) { return g_scg_launches; }

@@ -634,3 +634,12 @@ static inline bool scg_traj_log_ok(const scg_agent_t *ag) {
     return ag->traj_env && ag->traj_log && ag->traj_log_count && ag->traj_n >= 1 && ag->traj_n <= (uint32_t)ag->B &&
            ag->B > 0 && ag->traj_capacity > 0 && ag->traj_len >= 0 && ag->traj_len <= ag->win_len;
 }
+
+// the occupancy grid's fields: off (occ_grid = 0, occ_counts NULL), or a power of two <= SCG_OCC_GRID_MAX cells per
+// side with the counts set; occ_len counts the open window's steps already added
+#define SCG_OCC_GRID_MAX 128u
+static inline bool scg_occupancy_ok(const scg_agent_t *ag) {
+    if (ag->occ_grid == 0) return !ag->occ_counts && ag->occ_len == 0;
+    return ag->occ_counts && ag->occ_grid <= SCG_OCC_GRID_MAX && (ag->occ_grid & (ag->occ_grid - 1)) == 0 &&
+           ag->occ_len >= 0 && ag->occ_len <= ag->win_len;
+}

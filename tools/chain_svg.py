@@ -8,7 +8,10 @@ trajectories of tracked envs coloured by the running option (the standard skill-
 square; both PinballMap classes have them.  `trajectories` is what SkillChainAgent.trajectories() returns (step, env,
 state, option, term, episode_end; any order).  `init_grid` is an optional bool array (n_options, G, G): cell
 [o, i, j] is True when option o's initiation set holds at x = (j + 0.5) / G, y = (i + 0.5) / G, zero velocity
-(initiation_grid() builds it).  The picture has y pointing up.
+(initiation_grid() builds it).  `occupancy` is an optional count array (n_options, G, G) indexed [option, iy, ix], what
+SkillChainAgent.occupancy() returns as "counts": each option with any count gets a shaded layer of its visited cells,
+darker on a log scale of the count, under the initiation sets, which are then drawn as outlines.  The picture has y
+pointing up.
 """
 from xml.sax.saxutils import escape
 
@@ -18,6 +21,7 @@ import numpy as np
 OPTION_COLORS = ("#1f77b4", "#ff7f0e", "#2ca02c", "#d62728", "#9467bd", "#8c564b", "#e377c2", "#17becf",
                  "#bcbd22", "#7f7f7f", "#393b79", "#637939", "#8c6d31", "#843c39", "#7b4173", "#3182bd")
 SIZE = 640
+OCCUPANCY_LEVELS = 8        # shades of an occupancy layer (log scale of the count)
 
 
 def initiation_grid(options, active_mask, grid=64, device="cuda"):
@@ -75,20 +79,57 @@ def _paths(tr):
     return lines, marks
 
 
-def render(pmap, trajectories, init_grid=None, option_colors=OPTION_COLORS, title=None):
-    """-> the SVG document (str).  Layers, bottom to top: initiation sets (translucent cells, horizontal runs merged into
-    one rect), obstacles, target disc, start positions, trajectories (one polyline per run of one option), termination
-    markers."""
+def _outline(g, cw, ch):
+    """SVG path data of the boundary of the True cells of a bool grid (row i from the bottom): one segment per cell edge
+    between a True and a False cell."""
+    p = np.pad(np.asarray(g, dtype=bool), 1)
+    d = [f"M{j * cw:.2f},{SIZE - (i + 1) * ch:.2f}v{ch:.2f}" for i, j in zip(*np.nonzero(p[1:-1, 1:] != p[1:-1, :-1]))]
+    d += [f"M{j * cw:.2f},{SIZE - i * ch:.2f}h{cw:.2f}" for i, j in zip(*np.nonzero(p[1:, 1:-1] != p[:-1, 1:-1]))]
+    return "".join(d)
+
+
+def _occupancy_layers(counts, color):
+    """One <g class="occupancy"> per option with any count: its visited cells, shade level = ceil(L * log(1 + c) /
+    log(1 + max c)) with the max over all options, so the layers compare; one <path> per level, a subpath per horizontal
+    run of cells of that level."""
+    c = np.asarray(counts, dtype=np.float64)
+    out, top = [], np.log1p(c.max()) if c.size else 0.0
+    cw, ch = SIZE / c.shape[2], SIZE / c.shape[1]
+    for o in range(c.shape[0]):
+        if not c[o].any():
+            continue
+        level = np.ceil(np.log1p(c[o]) / top * OCCUPANCY_LEVELS).astype(np.int64)
+        out.append(f'<g class="occupancy" data-option="{o}" data-env-steps="{int(c[o].sum())}" fill="{color(o)}" '
+                   'stroke="none">')
+        for lv in range(1, OCCUPANCY_LEVELS + 1):
+            d = [f"M{j0 * cw:g} {SIZE - (i + 1) * ch:g}h{n * cw:g}v{ch:g}h{-n * cw:g}z"
+                 for i in range(c.shape[1]) for j0, n in _runs(level[i] == lv)]
+            if d:
+                out.append(f'<path data-level="{lv}" fill-opacity="{0.7 * lv / OCCUPANCY_LEVELS:.3f}" d="{"".join(d)}"/>')
+        out.append('</g>')
+    return out
+
+
+def render(pmap, trajectories, init_grid=None, option_colors=OPTION_COLORS, title=None, occupancy=None):
+    """-> the SVG document (str).  Layers, bottom to top: occupancy (one shaded layer per option, when given),
+    initiation sets (translucent cells, horizontal runs merged into one rect; outlines over an occupancy layer),
+    obstacles, target disc, start positions, trajectories (one polyline per run of one option), termination markers."""
     color = lambda o: option_colors[int(o) % len(option_colors)]
     out = [f'<svg xmlns="http://www.w3.org/2000/svg" width="{SIZE}" height="{SIZE}" viewBox="0 0 {SIZE} {SIZE}">',
            f'<rect x="0" y="0" width="{SIZE}" height="{SIZE}" fill="white" stroke="black"/>']
     if title:
         out.append(f'<title>{escape(str(title))}</title>')
+    if occupancy is not None:
+        out += _occupancy_layers(occupancy, color)
     if init_grid is not None:
         g = np.asarray(init_grid, dtype=bool)
         cell = SIZE / g.shape[2]
         for o in range(g.shape[0]):
             if not g[o].any():
+                continue
+            if occupancy is not None:
+                out.append(f'<g class="initiation" data-option="{o}" fill="none" stroke="{color(o)}" stroke-width="1.5">'
+                           f'<path d="{_outline(g[o], cell, SIZE / g.shape[1])}"/></g>')
                 continue
             out.append(f'<g class="initiation" data-option="{o}" fill="{color(o)}" fill-opacity="0.18" stroke="none">')
             for i in range(g.shape[1]):

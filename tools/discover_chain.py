@@ -28,6 +28,10 @@ With --draw PATH the greedy evaluation after discovery also logs the trajectorie
 (AgentConfig.trajectory_envs) and the script writes PATH, an SVG of the map, each active option's initiation set (64 x 64
 positions at zero velocity) and those greedy paths coloured by the running option (tools/chain_svg.py); the final JSON
 names it as "drawing".
+With --occupancy G the training agent counts every env-step by option and cell of a G x G grid (AgentConfig.occupancy_grid);
+the final JSON then carries, per option, its share of all env-steps and the fraction of the free-space cells (cells that
+hold a position sampled uniformly from free space) that it visited, and --draw shades each option's visited cells under
+its initiation set's outline.
 """
 import argparse
 import json
@@ -42,9 +46,10 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 from learning_curve import OptionTally  # noqa: E402
 
 
-def evaluate(scg, torch, base_map, src, args, n_env=4096, trained=True, draw=None):
+def evaluate(scg, torch, base_map, src, args, n_env=4096, trained=True, draw=None, occupancy=None):
     """Greedy episodes from the map's own start with (a copy of) the agent's weights, classifiers and option graph.
-    draw: SVG path - the first args.draw_envs envs' trajectories and the initiation sets are drawn there."""
+    draw: SVG path - the first args.draw_envs envs' trajectories and the initiation sets are drawn there, over the
+    training run's occupancy counts when given."""
     traj = dict(trajectory_envs=tuple(range(min(args.draw_envs, n_env))),
                 trajectory_log=min(args.draw_envs, n_env) * (args.max_episode_steps + 64)) if draw else {}
     cfg = scg.AgentConfig(map=args.map, batch=n_env, order=args.order, max_options=args.options, gamma=0.99, lam=0.9,
@@ -66,8 +71,9 @@ def evaluate(scg, torch, base_map, src, args, n_env=4096, trained=True, draw=Non
         c = ev.controller_state(sync=True)
         grid = initiation_grid(ev.options, c["active_mask"])
         with open(draw, "w") as f:
-            f.write(render(base_map, ev.trajectories(), init_grid=grid,
-                           title=f"{args.map} map: {c['n_active']} active options, greedy paths of {args.draw_envs} envs"))
+            f.write(render(base_map, ev.trajectories(), init_grid=grid, occupancy=occupancy,
+                           title=f"{args.map} map: {c['n_active']} active options, greedy paths of {args.draw_envs} envs"
+                                 + (", shaded where each option ran in training" if occupancy is not None else "")))
     return dict(success_rate=goals / n_env, finished=st["finished"], mean_return=st["mean_return"], steps=st["steps"])
 
 
@@ -95,6 +101,8 @@ def main():
                     help="log every option execution (ring of CAP records, polled every chunk) and report per-option totals")
     ap.add_argument("--draw", default=None, metavar="PATH", help="write an SVG of the chain and the greedy paths here")
     ap.add_argument("--draw-envs", type=int, default=32, help="greedy envs whose paths are drawn")
+    ap.add_argument("--occupancy", type=int, default=0, metavar="G",
+                    help="count every training env-step by option and cell of a G x G grid and report where each option ran")
     args = ap.parse_args()
     import torch
     import skill_chaining_with_graphs_b200 as scg
@@ -109,7 +117,7 @@ def main():
                           max_episode_steps=args.max_episode_steps, gestation_successes=args.gestation,
                           example_capacity=8192, clf_steps=300, clf_lr=2.0, graph=args.graph, option_bonus=1000.0,
                           top_level=not args.no_top_level, alpha_top=args.alpha_top, epsilon_top=0.1,
-                          init_horizon=args.horizon, option_log=args.option_log)
+                          init_horizon=args.horizon, option_log=args.option_log, occupancy_grid=args.occupancy)
     ag = scg.SkillChainAgent(cfg, train_map)
     tally = OptionTally([0, 1 << 32], args.options) if args.option_log else None
     opt = dict(seen=0, lost=0, s=0.0)
@@ -170,11 +178,24 @@ def main():
     # how much of the free space each initiation set covers, and whether it contains the map's start
     probe = torch.as_tensor(base.sample_free_states(np.random.default_rng(1), 20000)).cuda()
     inside = ag.options.initiation(probe)[:, :c["n_active"]].float().mean(dim=0).cpu().numpy().tolist() if c["n_active"] else []
-    after = evaluate(scg, torch, base, ag, args, trained=True, draw=args.draw)
+    occ = ag.occupancy() if args.occupancy else None
+    after = evaluate(scg, torch, base, ag, args, trained=True, draw=args.draw,
+                     occupancy=occ["counts"] if occ is not None else None)
     options = {}
+    if occ is not None:
+        G = occ["grid"]
+        free_xy = base.sample_free_states(np.random.default_rng(2), 200000)[:, :2]
+        free = np.zeros((G, G), dtype=bool)
+        free[np.clip((free_xy[:, 1] * np.float32(G)).astype(np.int64), 0, G - 1),
+             np.clip((free_xy[:, 0] * np.float32(G)).astype(np.int64), 0, G - 1)] = True
+        counts = occ["counts"]
+        options["occupancy"] = dict(
+            grid=G, env_steps=occ["env_steps"], free_cells=int(free.sum()),
+            share_of_env_steps=[round(int(counts[o].sum()) / max(occ["env_steps"], 1), 4) for o in range(len(counts))],
+            free_cells_visited=[round(float(((counts[o] > 0) & free).sum()) / free.sum(), 3) for o in range(len(counts))])
     if tally is not None:
         poll_options()
-        options = dict(options=tally.rows(0, (steps + train_steps) * args.batch), option_executions=opt["seen"],
+        options.update(options=tally.rows(0, (steps + train_steps) * args.batch), option_executions=opt["seen"],
                        option_executions_lost=opt["lost"], option_poll_s=round(opt["s"], 3))
     print(json.dumps(dict(map=args.map, batch=args.batch, graph=args.graph, top_level=not args.no_top_level,
                           wall_s=round(wall, 3), train_after_s=round(train_wall, 2), train_after_steps=train_steps, steps=steps, env_steps=steps * args.batch, n_active=c["n_active"],
